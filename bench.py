@@ -4,6 +4,8 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   (one rank per GPU, NCCL)
   python bench.py --impl reference ...   the reference's own CPU implementation of the same step on the host cores (the
                                           unmodified reference classes from baseline/_ref; the oracle port if that is absent)
+  python bench.py ... --dump-outputs DIR  also writes what the last timed step computed as DIR/*.npy (same arguments, same
+                                          inputs: two builds can be compared output for output)
 
 Default workload: the polyvore-shaped multi-slot step (BASELINE.json configs[3]: 10 x Linear(4096, 4096), B = 8192 per GPU,
 bf16 tensor-core engine) -- the largest single-GPU training configuration and the one the tensor-pipe bar is written for.
@@ -190,8 +192,9 @@ def workload_config(name, w, dims, world):
 
 
 # ----------------------------------------------------------------------------------------------------------------
-def train_block(name, dtype, K, Wm, args, env, e2e=True):
-    """One training workload on this rank's GPU: device-timed `value`, end-to-end `e2e`, per-kernel rooflines."""
+def train_block(name, dtype, K, Wm, args, env, e2e=True, dump_dir=None):
+    """One training workload on this rank's GPU: device-timed `value`, end-to-end `e2e`, per-kernel rooflines; with dump_dir,
+    what the last timed step computed (dump_outputs)."""
     import torch.distributed as dist
     from codae import _C
     from codae.dataset import ConcatenatedEmbeddingDataset
@@ -240,6 +243,10 @@ def train_block(name, dtype, K, Wm, args, env, e2e=True):
     clocks = sampler.stop() if sampler else None
     launches = K * fs.kernel_launches
     loss_last = fs.last_loss(B)
+    if dump_dir:
+        fs.flush()                # data-parallel peer mode gathers the master-weight shards: every rank takes part
+        if rank == 0:
+            dump_outputs(dump_dir, fs, B, loss_last)
     out = {"metric": "train samples/s", "value": world * B * K / (ms / 1e3), "unit": "samples/s", "n_gpus": world, "steps": K,
            "warmup": Wm, "ms_per_step": ms / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
            "dtype": "bf16" if fs_dtype(dtype, model) == "bf16" else "f32", "data": "synthetic",
@@ -329,6 +336,39 @@ def train_block(name, dtype, K, Wm, args, env, e2e=True):
     del fs, model, cor, data, ds, batches
     torch.cuda.empty_cache()
     return out, w
+
+
+DUMP_MAX_ELEMS = 1 << 22      # per array (16 MB of float32): a dump stays under 64 MB
+DUMP_SEED = 20240917
+
+
+def dump_outputs(out_dir, fs, B, loss):
+    """What a caller of FusedStep.step holds after the last timed step, as out_dir/<name>.npy: the loss, the monitor sums, the
+    reconstruction of the last batch, the model's parameters and their gradients (weights then bias of every layer, in
+    model.dims order).  An array of more than DUMP_MAX_ELEMS elements is replaced by a fixed, seeded sample (rows of the
+    reconstruction; positions of the parameter vector, the same for parameters and gradients): the same positions every run,
+    so that two builds compare output for output."""
+    model = fs.model
+    g = torch.Generator().manual_seed(DUMP_SEED)
+
+    y = fs._bufs[B]["acts"][-1][:, :fs.io]
+    if y.numel() > DUMP_MAX_ELEMS:
+        y = y[torch.randperm(B, generator=g)[:DUMP_MAX_ELEMS // fs.io].sort().values.to(y.device)]
+    P = model.nb_parameters()
+    pos = None if P <= DUMP_MAX_ELEMS else torch.randint(0, P, (DUMP_MAX_ELEMS,), generator=g).sort().values.to(fs.dev)
+
+    def params(flat):
+        v = torch.cat([torch.cat([model.weight_view(flat, l).reshape(-1), model.bias_view(flat, l)]) for l in range(len(model.dims))])
+        return (v if pos is None else v[pos]).cpu().numpy()
+
+    arrays = {"loss": np.array([loss], dtype=np.float64),
+              "monitors": fs.acc.cpu().numpy(),                    # sums of the full / partial loss, rows, last step's sum
+              "reconstruction": y.cpu().numpy(),
+              "parameters": params(model.flat),
+              "gradients": params(fs.gflat)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def scoring_block(args, env, E, seed, model_for_swaps=None):
@@ -452,6 +492,9 @@ def main():
     ap.add_argument("--dp-mode", type=str, default=None, choices=["peer", "nccl"],
                     help="data parallel: fused peer-memory reduce-scatter + sharded Adam + all-gather kernel (default) or NCCL all-reduce")
     ap.add_argument("--catalog", type=int, default=10_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, monitors, reconstruction, parameters and "
+                         "gradients; larger arrays as a fixed, seeded sample) as DIR/<name>.npy")
     args = ap.parse_args()
     w0 = dict(WORKLOADS[args.workload])
     big = args.workload == "polyvore"
@@ -497,7 +540,7 @@ def main():
         _C.set_option(dev, _C.OPT_TMA_STORE_PERSISTENT, 0)
     env = dict(rank=rank, world=world, dev=dev, local=local)
 
-    out, w = train_block(args.workload, dtype, K, Wm, args, env, e2e=True)
+    out, w = train_block(args.workload, dtype, K, Wm, args, env, e2e=True, dump_dir=args.dump_outputs)
     # ---- the shipped small-batch configs, each at its stated precision and in the other mode (same run, same box) -------
     if not args.no_secondary and args.workload == "polyvore" and args.dtype is None:
         sec = {}

@@ -2,6 +2,7 @@
 header's arity, and the product fails loudly (never falls back) without a GPU."""
 import os
 import re
+import shutil
 import subprocess
 
 import pytest
@@ -57,7 +58,10 @@ def test_library_exports_every_symbol():
 def test_sass_is_blackwell_native():
     """tcgen05.mma / tcgen05.ld / TMA show up as UTCHMMA / LDTM / UTMALDG in the sm_100a SASS."""
     from codae import _C
-    r = subprocess.run(["cuobjdump", "-sass", _C.LIB_PATH], capture_output=True, text=True)
+    # the Makefile calls nvcc by its full path, so the toolkit's bin directory need not be on PATH
+    from torch.utils.cpp_extension import CUDA_HOME
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(CUDA_HOME or "/usr/local/cuda", "bin", "cuobjdump")
+    r = subprocess.run([cuobjdump, "-sass", _C.LIB_PATH], capture_output=True, text=True)
     if r.returncode != 0:
         pytest.skip("cuobjdump unavailable")
     assert "sm_100a" in r.stdout

@@ -1,10 +1,11 @@
 """CPU: bench.py's reference arm runs without a GPU and prints the contract's JSON line; the product arm refuses to run
-without a B200 instead of falling back."""
+without a B200 instead of falling back.  GPU: --dump-outputs writes what the last timed step computed."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -60,6 +61,25 @@ def test_reference_arm_other_ranks_exit_silently():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "2", "--warmup", "1"],
                        capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(tmp_path):
+    """--dump-outputs writes float32 / float64 arrays, under 64 MB in all, of the last timed step: its loss is the JSON line's
+    loss_last_step, and the rows monitor counts exactly the warm-up and --steps steps."""
+    out = tmp_path / "dump"
+    r = run_bench("--workload", "embedding", "--steps", "5", "--warmup", "3", "--no-secondary", "--no-scoring", "--no-cpu",
+                  "--dump-outputs", str(out), timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])
+    a = {f[:-4]: np.load(out / f) for f in os.listdir(out)}
+    assert sorted(a) == ["gradients", "loss", "monitors", "parameters", "reconstruction"]
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert float(a["loss"][0]) == d["loss_last_step"] and d["steps"] == 5
+    assert a["monitors"][2] == 128 * (3 + 5)
+    assert a["reconstruction"].shape == (128, 1536) and np.isfinite(a["reconstruction"]).all()
+    assert a["parameters"].shape == a["gradients"].shape == (1 << 22,) and np.abs(a["gradients"]).max() > 0
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")
