@@ -314,6 +314,26 @@ size_t codae_score_topk_workspace_bytes(const codae_ctx* ctx, int Q, int k);
 int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
                      int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
                      float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes, void* stream);
+/* Batched top-k on tensor cores: the same results as codae_score_topk -- the same scores bit for bit, the same indices, ties
+ * by (score, index) -- for many queries in about one pass over the catalog.  A tcgen05 contraction of the queries (as hi / mid
+ * bf16 planes) against the catalog PROPOSES k' = min(2k + 32, 128) candidates per query, ranked by a bound on the sweep's
+ * fp32 score; the proposals are re-scored with the sweep's own arithmetic and the query is CERTIFIED when the exact k-th score
+ * is strictly better than the bound of every row left out (or when the shard has at most k' rows).
+ *   Arguments, layouts and E / ld / alignment rules: as codae_score_topk.  1 <= k <= CODAE_TOPK_BATCHED_MAX_K.
+ *   n_uncertified: device int, set to the number of queries that could not be certified; uncertified: device int [Q], its
+ *   first *n_uncertified entries are those query numbers (in no particular order).  Their out_score / out_idx rows are
+ *   unspecified: compute them with codae_score_topk (codae.tool.ComplementarityScorer.topk_local_batched does).
+ *   workspace >= codae_score_topk_batched_workspace_bytes(ctx, cat_dtype, n_rows, E, Q, k), 256-byte aligned; after the call
+ *   it begins with the merged proposals: float key[Q][k'] then, at offset round_up(4 Q k', 256), int64 idx[Q][k'] (best
+ *   first; key = the bound, never better than the row's exact score; idx -1 = empty).  fp32 catalogs are split into planes
+ *   chunk by chunk in the workspace (at most 512 MB of it).
+ *   Anything outside these limits returns CODAE_EINVAL; the call never switches to another algorithm by itself. */
+#define CODAE_TOPK_BATCHED_MAX_K 64
+size_t codae_score_topk_batched_workspace_bytes(const codae_ctx* ctx, int cat_dtype, int64_t n_rows, int E, int Q, int k);
+int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                             int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
+                             float* out_score, int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace,
+                             size_t ws_bytes, void* stream);
 /* Deterministic merge of G per-shard lists [G, Q, k] (e.g. after an all-gather) into [Q, k]. */
 int codae_topk_merge(codae_ctx* ctx, const float* scores, const int64_t* idx, int G, int Q, int k, int metric,
                      float* out_score, int64_t* out_idx, void* stream);

@@ -65,6 +65,9 @@ SIGNATURES = {
     "codae_dp_adam_step": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i64, _d, _d, _d, _d, _d, _i, _d, _vp, _vp, _sz, _d, _vp, _vp]),
     "codae_score_topk_workspace_bytes": (_sz, [_vp, _i, _i]),
     "codae_score_topk": (_i, [_vp, _vp, _i, _i64, _i64, _i, _i64, _vp, _i, _f, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "codae_score_topk_batched_workspace_bytes": (_sz, [_vp, _i, _i64, _i, _i, _i]),
+    "codae_score_topk_batched": (_i, [_vp, _vp, _i, _i64, _i64, _i, _i64, _vp, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz,
+                                      _vp]),
     "codae_topk_merge": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "codae_score_rank": (_i, [_vp, _vp, _i, _i64, _i64, _i, _vp, _i, _f, _i, _vp, _vp, _i64, _vp, _vp]),
     "codae_row_sqnorm": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp]),
@@ -457,6 +460,25 @@ def score_topk(catalog, E, row_offset, query, inv_scale, metric, k, out_score, o
     check(lib().codae_score_topk(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset, p(query),
                                  query.shape[0], inv_scale, metric, k, p(out_score), p(out_idx), p(ws), ws.numel(),
                                  stream()), c)
+
+
+TOPK_BATCHED_MAX_K = 64      # include/codae_b200.h: CODAE_TOPK_BATCHED_MAX_K
+
+
+def score_topk_batched_workspace(catalog, E, Q, k):
+    c = ctx(catalog.device)
+    n = int(lib().codae_score_topk_batched_workspace_bytes(c, dt(catalog), catalog.shape[0], E, Q, k))
+    return torch.empty(n, dtype=torch.uint8, device=catalog.device)
+
+
+def score_topk_batched(catalog, E, row_offset, query, inv_scale, metric, k, out_score, out_idx, n_uncertified, uncertified, ws):
+    """Tensor-core proposals + certification (codae_score_topk_batched).  n_uncertified: int32 [1], uncertified: int32 [Q]."""
+    _dev_check(catalog, query, out_score, out_idx, n_uncertified, uncertified, ws)
+    assert n_uncertified.dtype == torch.int32 and uncertified.dtype == torch.int32 and uncertified.numel() >= query.shape[0]
+    c = ctx(catalog.device)
+    check(lib().codae_score_topk_batched(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset, p(query),
+                                         query.shape[0], inv_scale, metric, k, p(out_score), p(out_idx), p(n_uncertified),
+                                         p(uncertified), p(ws), ws.numel(), stream()), c)
 
 
 def topk_merge(scores, idx, metric, out_score, out_idx):

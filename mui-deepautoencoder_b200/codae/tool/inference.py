@@ -25,6 +25,9 @@ def shard_rows(n_rows, world_size, rank):
 
 
 class ComplementarityScorer:
+    # Query batches of at least this many go through the tensor-core path (topk_batched) in the stage-IV script:
+    # the measured crossover against the row sweep on a 10 M x 512 catalog (DESIGN.md section 6).
+    TC_MIN_Q = 64
 
     def __init__(self, catalog, embedding_size, metric="sqerr", k=10, inv_scale=1.0, row_offset=0, process_group=None):
         """catalog: [n_local, E] fp32 or bf16 CUDA tensor -- this rank's shard (rows row_offset.. of the global
@@ -42,6 +45,8 @@ class ComplementarityScorer:
         self.row_offset = int(row_offset)
         self.pg = process_group
         self._ws = {}
+        self._ws_batched = {}
+        self.last_fallbacks = 0     # queries of the last batched call that were answered by the row sweep
 
     def _workspace(self, Q):
         ws = self._ws.get(Q)
@@ -59,9 +64,47 @@ class ComplementarityScorer:
         _C.score_topk(self.catalog, self.E, self.row_offset, q, self.inv_scale, self.metric, self.k, s, i, ws)
         return s, i
 
+    def _workspace_batched(self, Q):
+        ws = self._ws_batched.get(Q)
+        if ws is None:
+            dev = self.catalog.device
+            ws = (_C.score_topk_batched_workspace(self.catalog, self.E, Q, self.k),
+                  torch.empty((Q, self.k), dtype=torch.float32, device=dev), torch.empty((Q, self.k), dtype=torch.int64, device=dev),
+                  torch.zeros(1, dtype=torch.int32, device=dev), torch.empty(Q, dtype=torch.int32, device=dev))
+            self._ws_batched[Q] = ws
+        return ws
+
+    def topk_local_batched(self, query):
+        """Same inputs and results as topk_local -- the same scores bit for bit and the same indices -- for many queries in
+        about one pass over the shard: the tensor cores propose candidates, they are re-scored with the sweep's arithmetic,
+        and the queries whose result cannot be certified (last_fallbacks of them) are answered by the sweep.  Synchronises
+        once (one 4-byte device-to-host read of that count); reuses its buffers.  k > 64 is the sweep alone."""
+        q = query.to(torch.float32).contiguous()
+        Q = q.shape[0]
+        if self.k > _C.TOPK_BATCHED_MAX_K:
+            self.last_fallbacks = Q
+            return self.topk_local(q)
+        ws, s, i, n_unc, unc = self._workspace_batched(Q)
+        _C.score_topk_batched(self.catalog, self.E, self.row_offset, q, self.inv_scale, self.metric, self.k, s, i, n_unc, unc, ws)
+        nf = int(n_unc.item())
+        self.last_fallbacks = nf
+        if nf:
+            rows = unc[:nf].long()
+            fs, fi = self.topk_local(q.index_select(0, rows))
+            s.index_copy_(0, rows, fs)
+            i.index_copy_(0, rows, fi)
+        return s, i
+
+    def topk_batched(self, query):
+        """Global top-k of a query batch: topk_local_batched on this rank's shard (certification and fallback are per rank),
+        then the same all-gather + merge as topk -- every rank reaches it exactly once, whatever its fallback count."""
+        return self._gather_merge(*self.topk_local_batched(query))
+
     def topk(self, query):
         """Global top-k: local sweep, all-gather of k x 12 bytes per query, deterministic merge."""
-        s, i = self.topk_local(query)
+        return self._gather_merge(*self.topk_local(query))
+
+    def _gather_merge(self, s, i):
         import torch.distributed as dist
         if self.pg is None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
             return s, i

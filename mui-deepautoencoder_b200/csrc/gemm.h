@@ -1,5 +1,7 @@
 // Internal (non-ABI) entry points of the two GEMM engines; linear.cu dispatches between them.
 #pragma once
+#include <cuda.h>
+
 #include "common.cuh"
 
 int codae_simt_linear_fwd(codae_ctx* ctx, const float* X, int64_t ldx, const float* W, int64_t ldw, const float* bias,
@@ -33,3 +35,25 @@ bool codae_tc05_supported(const codae_ctx* ctx, const Tc05Gemm& g);
 int codae_tc05_gemm(codae_ctx* ctx, const Tc05Gemm& g, cudaStream_t s);
 // CTAs codae_tc05_gemm launches for this shape under the context's current options (0: shape not supported).
 int codae_tc05_gemm_ctas(const codae_ctx* ctx, const Tc05Gemm& g);
+// bf16 tensor map over a row-major [rows, cols] matrix with pitch ld (elements), box {box_cols, box_rows}, 128-byte swizzle,
+// out-of-range elements read as zero; planes > 1: a 3-D map {cols, rows, plane} over matrices plane_stride elements apart.
+int codae_tc05_make_map(codae_ctx* ctx, CUtensorMap* map, const void* base, long long rows, long long cols, long long ld,
+                        int box_cols, int box_rows, int planes, long long plane_stride);
+
+// Candidate pass of the batched top-k (score_tc.cu): one launch = one catalog chunk against query blocks qb0 .. qb0 + G - 1,
+// W CTAs per query block.  Every (CTA worker w, query q) keeps a sorted list of kp (bound key, global index) pairs in
+// ls / li [W][Q][kp] that persists across launches.  See the header comment of score_tc.cu for the keys.
+struct ScoreTcPass {
+    int metric;
+    const void* cat; int cat_planes;          // 1: the bf16 catalog rows in place; 2: hi / mid bf16 planes of an fp32 chunk
+    int64_t cat_ld, cat_plane_stride;
+    int64_t n_rows, row0;                     // rows of this chunk, global index of its row 0
+    const __nv_bfloat16* q_planes;            // hi / mid planes of the queries [2][Q][q_ld]
+    int64_t q_ld, q_plane_stride;
+    int Q, E, qb0, G, W, kp;
+    const float* cc;                          // [n_rows] row norms of the chunk
+    const float* qq;                          // [Q] query norms
+    float inv_scale, c_rel;                   // c_rel: relative error bound (score_tc.cu)
+    float* ls; int64_t* li;
+};
+int codae_score_tc_pass(codae_ctx* ctx, const ScoreTcPass& p, cudaStream_t s);

@@ -1258,6 +1258,11 @@ extern "C" int codae_debug_set_trace_cta(int linear_cta) {
     return 0;
 }
 
+int codae_tc05_make_map(codae_ctx* ctx, CUtensorMap* map, const void* base, long long rows, long long cols, long long ld,
+                        int box_cols, int box_rows, int planes, long long plane_stride) {
+    return make_map(ctx, map, base, rows, cols, ld, box_cols, box_rows, planes, plane_stride);
+}
+
 bool codae_tc05_supported(const codae_ctx* ctx, const Tc05Gemm& g) {
     if (!ctx || !ctx->encode_tiled) return false;
     if (g.M < 1 || g.N < 1 || g.K < 1) return false;

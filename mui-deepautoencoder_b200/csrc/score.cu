@@ -6,6 +6,7 @@
 #include <float.h>
 
 #include "common.cuh"
+#include "gemm.h"
 
 namespace {
 
@@ -315,13 +316,15 @@ __global__ void __launch_bounds__(kThreads) score_rank_kernel(const void* __rest
 //   rank_count_kernel  out_rank[q] = #{ j < n : cos(q, true_q) > cos(q, c_j) } with cos = dot / max(sqrt(|c|^2 |q|^2), 1e-8),
 //                      dot(q, true_q) = scores[q, n + q] (the true rows are appended to the catalog operand so that a true item
 //                      that is itself in the subset gets bit-identical scores on both sides of the strict comparison)
-__global__ void __launch_bounds__(kThreads) row_sqnorm_kernel(const float* __restrict__ X, int64_t ld, int64_t rows, int E,
+//                      (T = __nv_bfloat16: the row norms of a bf16 catalog for the batched top-k)
+template <typename T>
+__global__ void __launch_bounds__(kThreads) row_sqnorm_kernel(const T* __restrict__ X, int64_t ld, int64_t rows, int E,
                                                               float* __restrict__ out) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int64_t r = (int64_t)blockIdx.x * kWarps + warp; r < rows; r += (int64_t)gridDim.x * kWarps) {
-        const float* row = X + r * ld;
+        const T* row = X + r * ld;
         float s = 0.f;
-        for (int c = lane; c < E; c += 32) { const float v = row[c]; s = fmaf(v, v, s); }
+        for (int c = lane; c < E; c += 32) { const float v = (float)row[c]; s = fmaf(v, v, s); }
         s = warp_sum(s);
         if (lane == 0) out[r] = s;
     }
@@ -348,6 +351,134 @@ __global__ void __launch_bounds__(kThreads) rank_count_kernel(const float* __res
         for (int w = 0; w < kWarps; ++w) t += part[w];
         if (t) atomicAdd(&out_rank[q], (unsigned long long)t);      // integer counts: order-independent
     }
+}
+
+// ---- batched top-k: tensor-core proposals (score_tc.cu), certified here with the sweep's own arithmetic -------------------
+// hi / mid bf16 planes of fp32 rows (pitch `pitch`, columns E .. pitch - 1 zero): the A operand (queries) and, chunk by chunk, the
+// B operand of an fp32 catalog.  A padded pitch (multiple of 8 elements) keeps every plane row a whole number of 16-byte units,
+// which the tensor maps need; codae_split_x3 writes unpadded rows.
+__global__ void __launch_bounds__(kThreads) split_hm_kernel(const float* __restrict__ src, int64_t ld, int64_t rows, int E,
+                                                            __nv_bfloat16* __restrict__ dst, int64_t pitch, int64_t plane) {
+    const int64_t total = rows * pitch;
+    for (int64_t e = (int64_t)blockIdx.x * kThreads + threadIdx.x; e < total; e += (int64_t)gridDim.x * kThreads) {
+        const int64_t r = e / pitch;
+        const int c = (int)(e - r * pitch);
+        float h = 0.f, m = 0.f, l;
+        if (c < E) split3(src[r * ld + c], h, m, l);
+        dst[e] = __float2bfloat16_rn(h);
+        dst[plane + e] = __float2bfloat16_rn(m);
+    }
+}
+
+template <int METRIC>
+__global__ void __launch_bounds__(kThreads) list_init_kernel(float* __restrict__ ls, int64_t* __restrict__ li, int64_t n) {
+    for (int64_t e = (int64_t)blockIdx.x * kThreads + threadIdx.x; e < n; e += (int64_t)gridDim.x * kThreads) {
+        ls[e] = worst_score<METRIC>();
+        li[e] = kEmptyIdx;
+    }
+}
+
+// One CTA per query.  The merged proposal list of query q holds the kp best (bound key, index) pairs of the whole shard; every
+// row outside it has key >= the worst key b_w (SQERR; <= for COSINE) and, by the bound, an exact score no better than its key.
+// Re-score the kp rows exactly as score_topk_kernel does (query in shared memory, rows_partial, warp_sum tree, the same qq,
+// finish_score, NaN never ranks), keep the best k under (score, index), and CERTIFY the query when the exact k-th score is
+// strictly better than b_w -- then no outside row can enter -- or when the list holds every row of the shard.  Uncertified
+// queries are appended to uncert[] (count in *n_uncert); their outputs are written but unspecified.
+template <int METRIC, bool kBf16>
+__global__ void __launch_bounds__(kThreads) score_certify_kernel(const void* __restrict__ catalog, int64_t n_rows, int64_t ld, int E,
+                                                                 int64_t row_offset, const float* __restrict__ query, float inv_scale,
+                                                                 int k, int kp, const float* __restrict__ m_key,
+                                                                 const int64_t* __restrict__ m_idx, float* __restrict__ out_score,
+                                                                 int64_t* __restrict__ out_idx, int* __restrict__ n_uncert,
+                                                                 int* __restrict__ uncert) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    int64_t* ex_i = reinterpret_cast<int64_t*>(smem_raw);          // [kp] exact scores of the proposals
+    int64_t* li = ex_i + kp;                                        // [k]  best k
+    float* qs = reinterpret_cast<float*>(li + k);                   // [E]
+    float* ex_s = qs + E;                                           // [kp]
+    float* ls = ex_s + kp;                                          // [k]
+    float* qq = ls + k;                                             // [1]
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, q = blockIdx.x;
+    for (int e = threadIdx.x; e < E; e += kThreads) qs[e] = query[(int64_t)q * E + e];
+    for (int e = threadIdx.x; e < k; e += kThreads) { ls[e] = worst_score<METRIC>(); li[e] = kEmptyIdx; }
+    __syncthreads();
+    if (warp == 0) {
+        float s = 0.f;
+        for (int c = lane; c < E; c += 32) s = fmaf(qs[c], qs[c], s);
+        s = warp_sum(s);
+        if (lane == 0) qq[0] = s;
+    }
+    __syncthreads();
+    const size_t esz = kBf16 ? 2 : 4;
+    for (int e = warp; e < kp; e += kWarps) {
+        const int64_t gi = m_idx[(int64_t)q * kp + e];
+        float s = 0.f;
+        if (gi >= 0) {
+            float acc[1], cc;
+            row_partial<METRIC, 1, kBf16>(reinterpret_cast<const unsigned char*>(catalog) + (size_t)(gi - row_offset) * ld * esz, E, qs,
+                                          inv_scale, lane, acc, cc);
+            if (METRIC == CODAE_METRIC_COSINE) cc = warp_sum(cc);
+            s = finish_score<METRIC>(warp_sum(acc[0]), cc, qq[0]);
+        }
+        if (lane == 0) { ex_s[e] = s; ex_i[e] = (gi >= 0 && s == s) ? gi : kEmptyIdx; }    // NaN never ranks
+    }
+    __syncthreads();
+    if (warp != 0) return;
+    for (int e = 0; e < kp; ++e)
+        if (ex_i[e] != kEmptyIdx) list_insert<METRIC>(ls, li, k, ex_s[e], ex_i[e], lane);
+    const float bw = m_key[(int64_t)q * kp + kp - 1];
+    const int64_t iw = m_idx[(int64_t)q * kp + kp - 1];
+    bool cert = n_rows <= kp || iw < 0;             // the list holds every row of the shard
+    if (!cert) cert = li[k - 1] != kEmptyIdx && (METRIC == CODAE_METRIC_SQERR ? ls[k - 1] < bw : ls[k - 1] > bw);
+    for (int e = lane; e < k; e += 32) {
+        out_score[(int64_t)q * k + e] = ls[e];
+        out_idx[(int64_t)q * k + e] = li[e] == kEmptyIdx ? -1 : li[e];
+    }
+    if (!cert && lane == 0) uncert[atomicAdd(n_uncert, 1)] = q;
+}
+
+// Proposal list length k' (> k, <= the merge's 128) and relative error bound (derivation: score_tc.cu).
+inline int batched_kp(int k) { return 2 * k + 32 < kMaxK ? 2 * k + 32 : kMaxK; }
+inline float batched_c_rel(int E, bool bf16_catalog) {
+    const double P = bf16_catalog ? 2 : 3;
+    const double c = ldexp(1.0, -14) + (P * ((E + 15) / 16) + 8) * ldexp(1.0, -21) + (E / 32.0 + 16) * ldexp(1.0, -21);
+    return (float)(c * (1 + ldexp(1.0, -10)));
+}
+constexpr int kTcTileM = 128;              // queries per tensor-core tile
+// Rows of one catalog chunk: bf16 catalogs are read in place (the chunk only bounds the row-norm buffer), fp32 chunks are split
+// into two bf16 planes of 2 * rows * pitch elements -- at most 512 MB of scratch.
+inline int64_t batched_chunk_rows(bool bf16_catalog, int64_t pitch) {
+    if (bf16_catalog) return (int64_t)1 << 24;
+    const int64_t r = (((int64_t)1 << 27) / pitch) & ~(int64_t)255;
+    return r < 256 ? 256 : r;
+}
+struct BatchedLayout {         // workspace of codae_score_topk_batched, in this order, each part 256-byte aligned
+    int kp, W, G0, QB;
+    int64_t pitch, chunk, crow;   // crow: rows of the largest chunk (the row-norm and plane buffers hold that many)
+    size_t m_key, m_idx, ls, li, cc, qq, qplanes, cplanes, total;
+};
+inline size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
+inline BatchedLayout batched_layout(const codae_ctx* ctx, bool bf, int64_t n_rows, int E, int Q, int k) {
+    BatchedLayout L;
+    L.kp = batched_kp(k);
+    L.QB = (Q + kTcTileM - 1) / kTcTileM;
+    L.G0 = L.QB < ctx->sm_count ? L.QB : ctx->sm_count;
+    L.W = ctx->sm_count / L.G0;
+    L.pitch = (E + 7) & ~7;
+    L.chunk = batched_chunk_rows(bf, L.pitch);
+    const int64_t crow = L.crow = n_rows < L.chunk ? (n_rows > 0 ? n_rows : 1) : L.chunk;
+    const size_t lists = (size_t)L.W * Q * L.kp;
+    size_t o = 0;
+    L.m_key = o; o = al256(o + (size_t)Q * L.kp * 4);
+    L.m_idx = o; o = al256(o + (size_t)Q * L.kp * 8);
+    L.ls = o;    o = al256(o + lists * 4);
+    L.li = o;    o = al256(o + lists * 8);
+    L.cc = o;    o = al256(o + (size_t)crow * 4);
+    L.qq = o;    o = al256(o + (size_t)Q * 4);
+    L.qplanes = o; o = al256(o + (size_t)2 * Q * L.pitch * 2);
+    L.cplanes = o; if (!bf) o = al256(o + (size_t)2 * crow * L.pitch * 2);
+    L.total = o + 256;
+    return L;
 }
 
 // ---- candidate SWAPS scored by full reconstruction error --------------------------------------------------------
@@ -583,7 +714,7 @@ int codae_score_rank(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t
 int codae_row_sqnorm(codae_ctx* ctx, const float* X, int64_t ld, int64_t rows, int E, float* out, void* stream) {
     CODAE_REQUIRE(ctx, ctx && X && out && rows >= 0 && E >= 1 && ld >= E, "codae_row_sqnorm: bad argument");
     if (rows == 0) return CODAE_OK;
-    row_sqnorm_kernel<<<sweep_grid(ctx, rows), kThreads, 0, as_stream(stream)>>>(X, ld, rows, E, out);
+    row_sqnorm_kernel<float><<<sweep_grid(ctx, rows), kThreads, 0, as_stream(stream)>>>(X, ld, rows, E, out);
     return codae_check_launch(ctx, "row_sqnorm_kernel");
 }
 
@@ -599,6 +730,96 @@ int codae_rank_count(codae_ctx* ctx, const float* scores, int64_t ld, int Q, int
     if (gx > ctx->sm_count) gx = ctx->sm_count;
     rank_count_kernel<<<dim3(gx, Q), kThreads, 0, s>>>(scores, ld, Q, n, cc, qq, reinterpret_cast<unsigned long long*>(out_rank));
     return codae_check_launch(ctx, "rank_count_kernel");
+}
+
+size_t codae_score_topk_batched_workspace_bytes(const codae_ctx* ctx, int cat_dtype, int64_t n_rows, int E, int Q, int k) {
+    if (!ctx || Q < 1 || k < 1 || E < 1 || n_rows < 0 || (cat_dtype != CODAE_F32 && cat_dtype != CODAE_BF16)) return 0;
+    return batched_layout(ctx, cat_dtype == CODAE_BF16, n_rows, E, Q, k).total;
+}
+
+int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                             int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k, float* out_score,
+                             int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace, size_t ws_bytes,
+                             void* stream) {
+    CODAE_REQUIRE(ctx, ctx && catalog && query && out_score && out_idx && n_uncertified && uncertified && workspace,
+                  "codae_score_topk_batched: NULL argument");
+    CODAE_REQUIRE(ctx, k >= 1 && k <= CODAE_TOPK_BATCHED_MAX_K, "codae_score_topk_batched: k %d outside [1, %d]", k,
+                  CODAE_TOPK_BATCHED_MAX_K);
+    CODAE_REQUIRE(ctx, Q >= 1 && n_rows >= 0, "codae_score_topk_batched: bad Q / n_rows");
+    CODAE_REQUIRE(ctx, metric == CODAE_METRIC_SQERR || metric == CODAE_METRIC_COSINE, "codae_score_topk_batched: bad metric %d", metric);
+    const bool bf = cat_dtype == CODAE_BF16;
+    CODAE_REQUIRE(ctx, cat_dtype == CODAE_F32 || bf, "codae_score_topk_batched: bad cat_dtype %d", cat_dtype);
+    const int vec = bf ? 8 : 4;
+    CODAE_REQUIRE(ctx, E >= vec && E <= 4096 && E % vec == 0 && ld >= E && ld % vec == 0 &&
+                           (reinterpret_cast<uintptr_t>(catalog) & 15) == 0,
+                  "codae_score_topk_batched: E=%d ld=%lld must be multiples of %d (16-byte rows), E <= 4096", E, (long long)ld, vec);
+    const BatchedLayout L = batched_layout(ctx, bf, n_rows, E, Q, k);
+    if (ws_bytes < L.total)
+        return codae_fail(ctx, CODAE_ENOMEM, "codae_score_topk_batched: workspace %zu < %zu bytes", ws_bytes, L.total);
+    cudaStream_t s = as_stream(stream);
+    unsigned char* ws = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+    float* m_key = reinterpret_cast<float*>(ws + L.m_key);
+    int64_t* m_idx = reinterpret_cast<int64_t*>(ws + L.m_idx);
+    float* ls = reinterpret_cast<float*>(ws + L.ls);
+    int64_t* li = reinterpret_cast<int64_t*>(ws + L.li);
+    float* cc = reinterpret_cast<float*>(ws + L.cc);
+    float* qq = reinterpret_cast<float*>(ws + L.qq);
+    __nv_bfloat16* qplanes = reinterpret_cast<__nv_bfloat16*>(ws + L.qplanes);
+    __nv_bfloat16* cplanes = reinterpret_cast<__nv_bfloat16*>(ws + L.cplanes);
+    const int64_t q_plane = (int64_t)Q * L.pitch;
+    const int64_t c_plane = L.crow * L.pitch;
+
+    cudaError_t e = cudaMemsetAsync(n_uncertified, 0, sizeof(int), s);
+    if (e != cudaSuccess) return codae_fail(ctx, CODAE_ECUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
+    split_hm_kernel<<<sweep_grid(ctx, (int64_t)Q * L.pitch / 8), kThreads, 0, s>>>(query, E, Q, E, qplanes, L.pitch, q_plane);
+    row_sqnorm_kernel<float><<<sweep_grid(ctx, Q), kThreads, 0, s>>>(query, E, Q, E, qq);
+    const int64_t nl = (int64_t)L.W * Q * L.kp;
+    if (metric == CODAE_METRIC_SQERR) list_init_kernel<CODAE_METRIC_SQERR><<<sweep_grid(ctx, nl / 8), kThreads, 0, s>>>(ls, li, nl);
+    else list_init_kernel<CODAE_METRIC_COSINE><<<sweep_grid(ctx, nl / 8), kThreads, 0, s>>>(ls, li, nl);
+    int rc = codae_check_launch(ctx, "codae_score_topk_batched prologue");
+    if (rc) return rc;
+
+    ScoreTcPass p;
+    p.metric = metric;
+    p.q_planes = qplanes; p.q_ld = L.pitch; p.q_plane_stride = q_plane;
+    p.Q = Q; p.E = E; p.W = L.W; p.kp = L.kp;
+    p.cc = cc; p.qq = qq;
+    p.inv_scale = inv_scale; p.c_rel = batched_c_rel(E, bf);
+    p.ls = ls; p.li = li;
+    for (int64_t c0 = 0; c0 < n_rows; c0 += L.chunk) {
+        const int64_t rows = n_rows - c0 < L.chunk ? n_rows - c0 : L.chunk;
+        if (bf) {
+            const __nv_bfloat16* src = reinterpret_cast<const __nv_bfloat16*>(catalog) + c0 * ld;
+            row_sqnorm_kernel<__nv_bfloat16><<<sweep_grid(ctx, rows), kThreads, 0, s>>>(src, ld, rows, E, cc);
+            p.cat = src; p.cat_planes = 1; p.cat_ld = ld; p.cat_plane_stride = 0;
+        } else {
+            const float* src = reinterpret_cast<const float*>(catalog) + c0 * ld;
+            row_sqnorm_kernel<float><<<sweep_grid(ctx, rows), kThreads, 0, s>>>(src, ld, rows, E, cc);
+            split_hm_kernel<<<sweep_grid(ctx, rows * L.pitch / 8), kThreads, 0, s>>>(src, ld, rows, E, cplanes, L.pitch, c_plane);
+            p.cat = cplanes; p.cat_planes = 2; p.cat_ld = L.pitch; p.cat_plane_stride = c_plane;
+        }
+        rc = codae_check_launch(ctx, "codae_score_topk_batched chunk");
+        if (rc) return rc;
+        p.n_rows = rows; p.row0 = row_offset + c0;
+        for (int qb0 = 0; qb0 < L.QB; qb0 += L.G0) {
+            p.qb0 = qb0;
+            p.G = L.QB - qb0 < L.G0 ? L.QB - qb0 : L.G0;
+            rc = codae_score_tc_pass(ctx, p, s);
+            if (rc) return rc;
+        }
+    }
+    merge_attrs();
+    const size_t csmem = (size_t)(L.kp + k) * 12 + (size_t)E * 4 + 16;
+    if (metric == CODAE_METRIC_SQERR) {
+        topk_merge_kernel<CODAE_METRIC_SQERR><<<Q, kThreads, merge_smem(), s>>>(ls, li, L.W, Q, L.kp, m_key, m_idx, 0, 1);
+        if (bf) score_certify_kernel<CODAE_METRIC_SQERR, true><<<Q, kThreads, csmem, s>>>(catalog, n_rows, ld, E, row_offset, query, inv_scale, k, L.kp, m_key, m_idx, out_score, out_idx, n_uncertified, uncertified);
+        else score_certify_kernel<CODAE_METRIC_SQERR, false><<<Q, kThreads, csmem, s>>>(catalog, n_rows, ld, E, row_offset, query, inv_scale, k, L.kp, m_key, m_idx, out_score, out_idx, n_uncertified, uncertified);
+    } else {
+        topk_merge_kernel<CODAE_METRIC_COSINE><<<Q, kThreads, merge_smem(), s>>>(ls, li, L.W, Q, L.kp, m_key, m_idx, 0, 1);
+        if (bf) score_certify_kernel<CODAE_METRIC_COSINE, true><<<Q, kThreads, csmem, s>>>(catalog, n_rows, ld, E, row_offset, query, inv_scale, k, L.kp, m_key, m_idx, out_score, out_idx, n_uncertified, uncertified);
+        else score_certify_kernel<CODAE_METRIC_COSINE, false><<<Q, kThreads, csmem, s>>>(catalog, n_rows, ld, E, row_offset, query, inv_scale, k, L.kp, m_key, m_idx, out_score, out_idx, n_uncertified, uncertified);
+    }
+    return codae_check_launch(ctx, "score_certify_kernel");
 }
 
 }  // extern "C"

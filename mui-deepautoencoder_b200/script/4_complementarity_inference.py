@@ -74,7 +74,8 @@ if __name__ == "__main__":
     scorer = ComplementarityScorer(shard.contiguous(), E, metric=args.metric, k=args.k, inv_scale=1.0 / dataset.scale,
                                    row_offset=lo)
     p = predict_slot(model, outfits, args.slot, E)
-    scores, idx = scorer.topk(p)
+    # large query batches: one tensor-core pass over the catalog, results identical to the row sweep
+    scores, idx = scorer.topk_batched(p) if p.shape[0] >= ComplementarityScorer.TC_MIN_Q else scorer.topk(p)
     if rank == 0:
         print(json.dumps({"slot": args.slot, "metric": args.metric, "k": args.k,
                           "indices": idx.cpu().tolist(), "scores": scores.cpu().tolist()}))
