@@ -334,6 +334,31 @@ int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype,
                              int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
                              float* out_score, int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace,
                              size_t ws_bytes, void* stream);
+/* Filtered top-k: codae_score_topk / codae_score_topk_batched / codae_swap_error_topk with a say in which rows may be returned,
+ * e.g. leaving out the item the query outfit already holds, or keeping only items in stock.  Each takes its unfiltered
+ * sibling's arguments plus, before the outputs:
+ *   allow      uint8 [n_rows] indexed by LOCAL row (row j of `catalog`; swap: catalog row first_row + b), nonzero = eligible;
+ *              NULL = every row is eligible.
+ *   exclude    int64 [Q][n_exclude] GLOBAL indices (row_offset + local row) per query -- the same tensor fits every shard;
+ *              swap scoring has one outfit: [n_exclude].  Entries < 0 are padding; entries outside the shard never match.
+ *   n_exclude  0 <= n_exclude <= CODAE_TOPK_MAX_EXCLUDE; exclude is NULL exactly when n_exclude == 0.
+ * A filtered-out row behaves as if it were absent from the catalog: it never appears in the output; with fewer than k eligible
+ * rows the trailing slots are the usual empty ones (idx = -1, score = the unfiltered call's empty-slot value); ties stay
+ * (score, index).  The score of a row does not depend on which other rows are scored, so a filtered call equals, bit for bit,
+ * the unfiltered call on the catalog compacted to its eligible rows with the indices mapped back; the batched filtered call
+ * equals the filtered sweep bit for bit (its uncertified queries are recomputed with codae_score_topk_filtered, the same allow
+ * and their rows of exclude).  Workspace sizes are those of the unfiltered calls.  row_offset must be >= 0.  Bad filter
+ * arguments return CODAE_EINVAL.  No filter (allow NULL, n_exclude 0) runs exactly the unfiltered code.              */
+#define CODAE_TOPK_MAX_EXCLUDE 256
+int codae_score_topk_filtered(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                              int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
+                              const uint8_t* allow, const int64_t* exclude, int n_exclude, float* out_score, int64_t* out_idx,
+                              void* workspace, size_t ws_bytes, void* stream);
+int codae_score_topk_batched_filtered(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                                      int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
+                                      const uint8_t* allow, const int64_t* exclude, int n_exclude, float* out_score,
+                                      int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace, size_t ws_bytes,
+                                      void* stream);
 /* Deterministic merge of G per-shard lists [G, Q, k] (e.g. after an all-gather) into [Q, k]. */
 int codae_topk_merge(codae_ctx* ctx, const float* scores, const int64_t* idx, int G, int Q, int k, int metric,
                      float* out_score, int64_t* out_idx, void* stream);
@@ -367,6 +392,12 @@ int codae_swap_error_topk(codae_ctx* ctx, const float* outfit, const void* catal
                           int64_t first_row, int B, int E, int slot, int io, float inv_scale, const float* y, int64_t ld_y,
                           int64_t row_offset, int k, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes,
                           void* stream);
+/* codae_swap_error_topk with allow [rows of catalog] and exclude [n_exclude]: see the filtered top-k above. */
+int codae_swap_error_topk_filtered(codae_ctx* ctx, const float* outfit, const void* catalog, int cat_dtype, int64_t ld_cat,
+                                   int64_t first_row, int B, int E, int slot, int io, float inv_scale, const float* y,
+                                   int64_t ld_y, int64_t row_offset, int k, const uint8_t* allow, const int64_t* exclude,
+                                   int n_exclude, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes,
+                                   void* stream);
 
 #ifdef __cplusplus
 }

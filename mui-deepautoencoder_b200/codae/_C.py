@@ -68,6 +68,10 @@ SIGNATURES = {
     "codae_score_topk_batched_workspace_bytes": (_sz, [_vp, _i, _i64, _i, _i, _i]),
     "codae_score_topk_batched": (_i, [_vp, _vp, _i, _i64, _i64, _i, _i64, _vp, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz,
                                       _vp]),
+    "codae_score_topk_filtered": (_i, [_vp, _vp, _i, _i64, _i64, _i, _i64, _vp, _i, _f, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _sz,
+                                       _vp]),
+    "codae_score_topk_batched_filtered": (_i, [_vp, _vp, _i, _i64, _i64, _i, _i64, _vp, _i, _f, _i, _i, _vp, _vp, _i, _vp, _vp,
+                                               _vp, _vp, _vp, _sz, _vp]),
     "codae_topk_merge": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "codae_score_rank": (_i, [_vp, _vp, _i, _i64, _i64, _i, _vp, _i, _f, _i, _vp, _vp, _i64, _vp, _vp]),
     "codae_row_sqnorm": (_i, [_vp, _vp, _i64, _i64, _i, _vp, _vp]),
@@ -75,6 +79,8 @@ SIGNATURES = {
     "codae_swap_build": (_i, [_vp, _vp, _vp, _i, _i64, _i64, _i, _i, _i, _i, _f, _vp, _i, _i64, _vp]),
     "codae_swap_error_topk": (_i, [_vp, _vp, _vp, _i, _i64, _i64, _i, _i, _i, _i, _f, _vp, _i64, _i64, _i, _vp, _vp, _vp,
                                    _sz, _vp]),
+    "codae_swap_error_topk_filtered": (_i, [_vp, _vp, _vp, _i, _i64, _i64, _i, _i, _i, _i, _f, _vp, _i64, _i64, _i, _vp, _vp, _i,
+                                            _vp, _vp, _vp, _sz, _vp]),
 }
 
 DP_MAX_WORLD = 8
@@ -454,12 +460,29 @@ def score_topk_workspace(device, Q, k):
     return torch.empty(int(lib().codae_score_topk_workspace_bytes(c, Q, k)), dtype=torch.uint8, device=device)
 
 
-def score_topk(catalog, E, row_offset, query, inv_scale, metric, k, out_score, out_idx, ws):
-    _dev_check(catalog, query, out_score, out_idx, ws)
+TOPK_MAX_EXCLUDE = 256       # include/codae_b200.h: CODAE_TOPK_MAX_EXCLUDE
+
+
+def _n_exclude(exclude):
+    """Columns of an exclusion tensor ([Q, m] or [m]); m == 0 is passed as no list (NULL, 0)."""
+    m = 0 if exclude is None else int(exclude.shape[-1])
+    return (exclude if m else None), m
+
+
+def score_topk(catalog, E, row_offset, query, inv_scale, metric, k, out_score, out_idx, ws, allow=None, exclude=None):
+    """allow: uint8 [n_rows] or None; exclude: int64 [Q, m] global indices (-1 padding) or None.  Without either, the
+    unfiltered entry point (codae_score_topk)."""
+    _dev_check(catalog, query, out_score, out_idx, ws, allow, exclude)
     c = ctx(catalog.device)
-    check(lib().codae_score_topk(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset, p(query),
-                                 query.shape[0], inv_scale, metric, k, p(out_score), p(out_idx), p(ws), ws.numel(),
-                                 stream()), c)
+    if allow is None and exclude is None:
+        check(lib().codae_score_topk(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset, p(query),
+                                     query.shape[0], inv_scale, metric, k, p(out_score), p(out_idx), p(ws), ws.numel(),
+                                     stream()), c)
+        return
+    ex, m = _n_exclude(exclude)
+    check(lib().codae_score_topk_filtered(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset, p(query),
+                                          query.shape[0], inv_scale, metric, k, p(allow), p(ex), m, p(out_score), p(out_idx),
+                                          p(ws), ws.numel(), stream()), c)
 
 
 TOPK_BATCHED_MAX_K = 64      # include/codae_b200.h: CODAE_TOPK_BATCHED_MAX_K
@@ -471,14 +494,23 @@ def score_topk_batched_workspace(catalog, E, Q, k):
     return torch.empty(n, dtype=torch.uint8, device=catalog.device)
 
 
-def score_topk_batched(catalog, E, row_offset, query, inv_scale, metric, k, out_score, out_idx, n_uncertified, uncertified, ws):
-    """Tensor-core proposals + certification (codae_score_topk_batched).  n_uncertified: int32 [1], uncertified: int32 [Q]."""
-    _dev_check(catalog, query, out_score, out_idx, n_uncertified, uncertified, ws)
+def score_topk_batched(catalog, E, row_offset, query, inv_scale, metric, k, out_score, out_idx, n_uncertified, uncertified, ws,
+                       allow=None, exclude=None):
+    """Tensor-core proposals + certification (codae_score_topk_batched).  n_uncertified: int32 [1], uncertified: int32 [Q].
+    allow / exclude as in score_topk (codae_score_topk_batched_filtered when either is given)."""
+    _dev_check(catalog, query, out_score, out_idx, n_uncertified, uncertified, ws, allow, exclude)
     assert n_uncertified.dtype == torch.int32 and uncertified.dtype == torch.int32 and uncertified.numel() >= query.shape[0]
     c = ctx(catalog.device)
-    check(lib().codae_score_topk_batched(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset, p(query),
-                                         query.shape[0], inv_scale, metric, k, p(out_score), p(out_idx), p(n_uncertified),
-                                         p(uncertified), p(ws), ws.numel(), stream()), c)
+    if allow is None and exclude is None:
+        check(lib().codae_score_topk_batched(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset,
+                                             p(query), query.shape[0], inv_scale, metric, k, p(out_score), p(out_idx),
+                                             p(n_uncertified), p(uncertified), p(ws), ws.numel(), stream()), c)
+        return
+    ex, m = _n_exclude(exclude)
+    check(lib().codae_score_topk_batched_filtered(c, p(catalog), dt(catalog), catalog.shape[0], catalog.stride(0), E, row_offset,
+                                                  p(query), query.shape[0], inv_scale, metric, k, p(allow), p(ex), m,
+                                                  p(out_score), p(out_idx), p(n_uncertified), p(uncertified), p(ws), ws.numel(),
+                                                  stream()), c)
 
 
 def topk_merge(scores, idx, metric, out_score, out_idx):
@@ -516,12 +548,21 @@ def swap_build(outfit, catalog, first_row, B, E, slot, io, inv_scale, out_x):
                                  inv_scale, p(out_x), dt(out_x), out_x.stride(0), stream()), c)
 
 
-def swap_error_topk(outfit, catalog, first_row, B, E, slot, io, inv_scale, y, row_offset, k, out_score, out_idx, ws):
-    _dev_check(outfit, catalog, y, out_score, out_idx, ws)
+def swap_error_topk(outfit, catalog, first_row, B, E, slot, io, inv_scale, y, row_offset, k, out_score, out_idx, ws, allow=None,
+                    exclude=None):
+    """allow: uint8 [rows of catalog] or None; exclude: int64 [m] global indices or None (codae_swap_error_topk_filtered when
+    either is given)."""
+    _dev_check(outfit, catalog, y, out_score, out_idx, ws, allow, exclude)
     c = ctx(catalog.device)
-    check(lib().codae_swap_error_topk(c, p(outfit), p(catalog), dt(catalog), catalog.stride(0), first_row, B, E, slot, io,
-                                      inv_scale, p(y), y.stride(0), row_offset, k, p(out_score), p(out_idx), p(ws),
-                                      ws.numel(), stream()), c)
+    if allow is None and exclude is None:
+        check(lib().codae_swap_error_topk(c, p(outfit), p(catalog), dt(catalog), catalog.stride(0), first_row, B, E, slot, io,
+                                          inv_scale, p(y), y.stride(0), row_offset, k, p(out_score), p(out_idx), p(ws),
+                                          ws.numel(), stream()), c)
+        return
+    ex, m = _n_exclude(exclude)
+    check(lib().codae_swap_error_topk_filtered(c, p(outfit), p(catalog), dt(catalog), catalog.stride(0), first_row, B, E, slot,
+                                               io, inv_scale, p(y), y.stride(0), row_offset, k, p(allow), p(ex), m, p(out_score),
+                                               p(out_idx), p(ws), ws.numel(), stream()), c)
 
 
 def linear_engine(device, dtype, M, N, K):

@@ -6,6 +6,10 @@ item of category c (squared error against p, or cosine similarity) -> top-k.  Th
 across ranks; each rank sweeps its shard (codae_score_topk) and the per-rank lists are all-gathered and merged
 deterministically (codae_topk_merge).
 
+Both scorers take an optional filter: `allowed`, a per-shard mask of the rows that may be returned (items in stock, in the
+right region), and per call `exclude`, global row indices a query must not get back (the item the outfit already holds).  A
+filtered-out row is treated as absent from the catalog, inside the kernels (include/codae_b200.h: filtered top-k).
+
 SwapScorer is the other reading of "scores candidate item swaps by reconstruction error": every candidate is
 substituted into the slot, the whole swapped outfit goes through the DAE (tensor-core GEMMs batched over the
 candidates) and the swap is scored by the reconstruction error of the swapped outfit.
@@ -15,6 +19,35 @@ import torch
 from codae import _C
 
 METRICS = {"sqerr": _C.METRIC_SQERR, "cosine": _C.METRIC_COSINE}
+
+
+def _allowed_mask(allowed, n_local, device):
+    """bool / uint8 [n_local] CUDA tensor on the catalog's device -> contiguous uint8 (None: every row)."""
+    if allowed is None:
+        return None
+    if not isinstance(allowed, torch.Tensor) or allowed.dtype not in (torch.bool, torch.uint8):
+        raise RuntimeError("codae: allowed must be a bool or uint8 tensor")
+    if allowed.dim() != 1 or allowed.shape[0] != n_local:
+        raise RuntimeError("codae: allowed must have shape [%d] (rows of this shard), got %s" % (n_local, tuple(allowed.shape)))
+    if not allowed.is_cuda or allowed.device != device:
+        raise RuntimeError("codae: allowed must be on the catalog's device %s" % device)
+    return allowed.to(torch.uint8).contiguous()
+
+
+def _exclusions(exclude, shape0, device):
+    """int64 CUDA tensor of global row indices, [Q, m] (shape0 = Q) or [m] (shape0 = None), -1 padding; m <= 256."""
+    if exclude is None:
+        return None
+    if not isinstance(exclude, torch.Tensor) or exclude.dtype != torch.int64:
+        raise RuntimeError("codae: exclude must be an int64 tensor")
+    want = "[m]" if shape0 is None else "[%d, m]" % shape0
+    if (exclude.dim() != (1 if shape0 is None else 2) or (shape0 is not None and exclude.shape[0] != shape0)
+            or exclude.shape[-1] > _C.TOPK_MAX_EXCLUDE):
+        raise RuntimeError("codae: exclude must have shape %s with m <= %d, got %s" % (want, _C.TOPK_MAX_EXCLUDE,
+                                                                                   tuple(exclude.shape)))
+    if not exclude.is_cuda or exclude.device != device:
+        raise RuntimeError("codae: exclude must be on the catalog's device %s" % device)
+    return exclude.contiguous()
 
 
 def shard_rows(n_rows, world_size, rank):
@@ -29,10 +62,12 @@ class ComplementarityScorer:
     # the measured crossover against the row sweep on a 10 M x 512 catalog (DESIGN.md section 6).
     TC_MIN_Q = 64
 
-    def __init__(self, catalog, embedding_size, metric="sqerr", k=10, inv_scale=1.0, row_offset=0, process_group=None):
+    def __init__(self, catalog, embedding_size, metric="sqerr", k=10, inv_scale=1.0, row_offset=0, process_group=None,
+                 allowed=None):
         """catalog: [n_local, E] fp32 or bf16 CUDA tensor -- this rank's shard (rows row_offset.. of the global
         catalog).  inv_scale multiplies catalog values before the squared error (1/dataset.scale when the
-        catalog is un-scaled like dataset.data_per_category)."""
+        catalog is un-scaled like dataset.data_per_category).  allowed: bool / uint8 [n_local] CUDA tensor, the rows of this
+        shard that may be returned (None: all)."""
         if metric not in METRICS:
             raise Exception("Unknown metric.")
         if not catalog.is_cuda:
@@ -44,6 +79,7 @@ class ComplementarityScorer:
         self.inv_scale = float(inv_scale)
         self.row_offset = int(row_offset)
         self.pg = process_group
+        self.allowed = _allowed_mask(allowed, catalog.shape[0], catalog.device)
         self._ws = {}
         self._ws_batched = {}
         self.last_fallbacks = 0     # queries of the last batched call that were answered by the row sweep
@@ -57,11 +93,14 @@ class ComplementarityScorer:
             self._ws[Q] = ws
         return ws
 
-    def topk_local(self, query):
-        """(scores [Q,k] f32, global indices [Q,k] i64) of this shard; asynchronous, reuses its buffers."""
+    def topk_local(self, query, exclude=None):
+        """(scores [Q,k] f32, global indices [Q,k] i64) of this shard; asynchronous, reuses its buffers.  exclude: int64
+        [Q, m] CUDA tensor of global row indices query q must not get back (-1 padding, m <= 256)."""
         q = query.to(torch.float32).contiguous()
+        ex = _exclusions(exclude, q.shape[0], self.catalog.device)
         ws, s, i = self._workspace(q.shape[0])
-        _C.score_topk(self.catalog, self.E, self.row_offset, q, self.inv_scale, self.metric, self.k, s, i, ws)
+        _C.score_topk(self.catalog, self.E, self.row_offset, q, self.inv_scale, self.metric, self.k, s, i, ws,
+                      allow=self.allowed, exclude=ex)
         return s, i
 
     def _workspace_batched(self, Q):
@@ -74,35 +113,38 @@ class ComplementarityScorer:
             self._ws_batched[Q] = ws
         return ws
 
-    def topk_local_batched(self, query):
+    def topk_local_batched(self, query, exclude=None):
         """Same inputs and results as topk_local -- the same scores bit for bit and the same indices -- for many queries in
         about one pass over the shard: the tensor cores propose candidates, they are re-scored with the sweep's arithmetic,
         and the queries whose result cannot be certified (last_fallbacks of them) are answered by the sweep.  Synchronises
         once (one 4-byte device-to-host read of that count); reuses its buffers.  k > 64 is the sweep alone."""
         q = query.to(torch.float32).contiguous()
         Q = q.shape[0]
+        ex = _exclusions(exclude, Q, self.catalog.device)
         if self.k > _C.TOPK_BATCHED_MAX_K:
             self.last_fallbacks = Q
-            return self.topk_local(q)
+            return self.topk_local(q, ex)
         ws, s, i, n_unc, unc = self._workspace_batched(Q)
-        _C.score_topk_batched(self.catalog, self.E, self.row_offset, q, self.inv_scale, self.metric, self.k, s, i, n_unc, unc, ws)
+        _C.score_topk_batched(self.catalog, self.E, self.row_offset, q, self.inv_scale, self.metric, self.k, s, i, n_unc, unc, ws,
+                              allow=self.allowed, exclude=ex)
         nf = int(n_unc.item())
         self.last_fallbacks = nf
         if nf:
             rows = unc[:nf].long()
-            fs, fi = self.topk_local(q.index_select(0, rows))
+            fs, fi = self.topk_local(q.index_select(0, rows), None if ex is None else ex.index_select(0, rows))
             s.index_copy_(0, rows, fs)
             i.index_copy_(0, rows, fi)
         return s, i
 
-    def topk_batched(self, query):
+    def topk_batched(self, query, exclude=None):
         """Global top-k of a query batch: topk_local_batched on this rank's shard (certification and fallback are per rank),
-        then the same all-gather + merge as topk -- every rank reaches it exactly once, whatever its fallback count."""
-        return self._gather_merge(*self.topk_local_batched(query))
+        then the same all-gather + merge as topk -- every rank reaches it exactly once, whatever its fallback count.
+        exclude holds global indices, so every rank is given the same tensor."""
+        return self._gather_merge(*self.topk_local_batched(query, exclude))
 
-    def topk(self, query):
+    def topk(self, query, exclude=None):
         """Global top-k: local sweep, all-gather of k x 12 bytes per query, deterministic merge."""
-        return self._gather_merge(*self.topk_local(query))
+        return self._gather_merge(*self.topk_local(query, exclude))
 
     def _gather_merge(self, s, i):
         import torch.distributed as dist
@@ -134,7 +176,9 @@ class SwapScorer:
     writes the swapped outfits straight into the first activation buffer, the model's Linear layers run on them,
     codae_swap_error_topk reduces each chunk to k candidates and codae_topk_merge combines chunks (and ranks)."""
 
-    def __init__(self, model, catalog, embedding_size, k=10, inv_scale=1.0, row_offset=0, chunk=8192, process_group=None):
+    def __init__(self, model, catalog, embedding_size, k=10, inv_scale=1.0, row_offset=0, chunk=8192, process_group=None,
+                 allowed=None):
+        """allowed: bool / uint8 [n_local] CUDA tensor, the candidates of this shard that may be returned (None: all)."""
         if not catalog.is_cuda:
             raise RuntimeError("codae: catalog is not on a CUDA device; the B200 path has no CPU fallback")
         model._require_cuda()
@@ -144,6 +188,7 @@ class SwapScorer:
         if self.io % self.E != 0 or catalog.shape[1] < self.E:
             raise Exception("Catalog width or embedding size does not fit the model input.")
         dev = catalog.device
+        self.allowed = _allowed_mask(allowed, catalog.shape[0], dev)
         self._ws = _C.score_topk_workspace(dev, 1, k)
         self._acts = None
 
@@ -160,11 +205,13 @@ class SwapScorer:
             self._acts = (eng, acts, stage)
         return self._acts
 
-    def topk_local(self, outfit, slot):
-        """outfit: [io] scaled fp32 row.  Returns (errors [k], global candidate indices [k]) of this shard."""
+    def topk_local(self, outfit, slot, exclude=None):
+        """outfit: [io] scaled fp32 row.  Returns (errors [k], global candidate indices [k]) of this shard.  exclude: int64
+        [m] CUDA tensor of global candidate indices not to return (-1 padding, m <= 256), e.g. the item already in the slot."""
         m, dev = self.model, self.catalog.device
         if not 0 <= slot < self.io // self.E:
             raise Exception("Slot out of range.")
+        ex = _exclusions(exclude, None, dev)
         outfit = outfit.to(torch.float32).contiguous().view(-1)
         m.sync_weights()          # a sharded data-parallel trainer gathers the master weights first (collective)
         eng, acts, stage = self._buffers()
@@ -186,14 +233,14 @@ class SwapScorer:
                 _C.linear_fwd(acts[l], m.aug_view(wflat, l), None, acts[l + 1], B, o, (i + 7) // 8 * 8 + 1,
                               _C.ACT_RELU if m.relu[l] else _C.ACT_NONE, eng)
             _C.swap_error_topk(outfit, self.catalog, first, B, self.E, slot, self.io, self.inv_scale, acts[-1],
-                               self.row_offset, self.k, ls[c, 0], li[c, 0], self._ws)
+                               self.row_offset, self.k, ls[c, 0], li[c, 0], self._ws, allow=self.allowed, exclude=ex)
         out_s = torch.empty((1, self.k), dtype=torch.float32, device=dev)
         out_i = torch.empty((1, self.k), dtype=torch.int64, device=dev)
         _C.topk_merge(ls, li, _C.METRIC_SQERR, out_s, out_i)
         return out_s[0], out_i[0]
 
-    def topk(self, outfit, slot):
-        s, i = self.topk_local(outfit, slot)
+    def topk(self, outfit, slot, exclude=None):
+        s, i = self.topk_local(outfit, slot, exclude)
         import torch.distributed as dist
         if self.pg is None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
             return s, i

@@ -55,5 +55,7 @@ struct ScoreTcPass {
     const float* qq;                          // [Q] query norms
     float inv_scale, c_rel;                   // c_rel: relative error bound (score_tc.cu)
     float* ls; int64_t* li;
+    const uint8_t* allow;                     // [n_rows] eligibility of the chunk's rows, or NULL (every row)
+    const int64_t* exclude; int n_exclude;    // [Q][n_exclude] excluded global indices per query (entries < 0: padding)
 };
 int codae_score_tc_pass(codae_ctx* ctx, const ScoreTcPass& p, cudaStream_t s);

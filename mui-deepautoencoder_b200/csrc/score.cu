@@ -51,6 +51,25 @@ __device__ __forceinline__ bool list_insert(float* ls, int64_t* li, int k, float
     return true;
 }
 
+// Filtered instantiations (kFilter): may local row r, global index gi, enter the list of a query with exclusion list
+// ex[n_ex]?  Asked only after the candidate has beaten the list's worst entry -- the rare path -- so the mask byte and the
+// exclusion list are read from global memory there.  Warp-cooperative: all lanes must call with identical arguments.
+__device__ __forceinline__ bool eligible(const uint8_t* __restrict__ allow, int64_t r, const int64_t* __restrict__ ex, int n_ex,
+                                         int64_t gi, int lane) {
+    if (allow && !allow[r]) return false;
+    bool hit = false;
+    for (int e = lane; e < n_ex; e += 32) hit |= ex[e] == gi;      // padding (< 0) never equals gi >= 0
+    return !__any_sync(0xffffffffu, hit);
+}
+
+// The filtered instantiations' insertion: list_insert of an eligible row.  Kept out of line so that the sweep loop around it is
+// allocated as in the unfiltered kernels (inlined, the rare path raised the loop's register count and cost up to 1.6x).
+template <int METRIC>
+__device__ __noinline__ void filtered_insert(float* ls, int64_t* li, int k, float s, int64_t gi, const uint8_t* __restrict__ allow,
+                                             int64_t r, const int64_t* __restrict__ ex, int n_ex, int lane) {
+    if (eligible(allow, r, ex, n_ex, gi, lane)) list_insert<METRIC>(ls, li, k, s, gi, lane);
+}
+
 // R candidate rows against QC queries (smem), partial sums per lane.  All loads of a 256-element (bf16) / 128-element (f32)
 // column block of the R rows are issued before the first use: R x 16 bytes (bf16) or R x 16 bytes x 1 (f32, four column blocks
 // per unrolled pass) in flight per lane -- a 1 KB bf16 row alone leaves a warp with 2 loads in flight and the sweep at half of
@@ -130,11 +149,14 @@ __device__ __forceinline__ float finish_score(float acc, float cc, float qq) {
 }
 
 // Workspace layout: [grid][QC][k] entries per launch (scores then indices).
-template <int METRIC, int QC, bool kBf16>
+// kFilter: allow [n_rows] (NULL: every row) and exclude [QC][n_exclude] global indices of the CTA's queries; a row that fails
+// them is treated as absent.  The unfiltered instantiation ignores both.
+template <int METRIC, int QC, bool kBf16, bool kFilter>
 __global__ void __launch_bounds__(kThreads) score_topk_kernel(const void* __restrict__ catalog, int64_t n_rows, int64_t ld,
                                                               int E, int64_t row_offset, const float* __restrict__ query,
                                                               float inv_scale, int k, float* __restrict__ ws_score,
-                                                              int64_t* __restrict__ ws_idx) {
+                                                              int64_t* __restrict__ ws_idx, const uint8_t* __restrict__ allow,
+                                                              const int64_t* __restrict__ exclude, int n_exclude) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float* qs = reinterpret_cast<float*>(smem_raw);                        // [QC][E]
     float* qq = qs + QC * E;                                               // [QC] |q|^2
@@ -180,7 +202,12 @@ __global__ void __launch_bounds__(kThreads) score_topk_kernel(const void* __rest
 #pragma unroll
             for (int q = 0; q < QC; ++q) {
                 const float s = finish_score<METRIC>(acc[j][q], cc[j], qq[q]);
-                if (s == s) list_insert<METRIC>(my_s + q * k, my_i + q * k, k, s, row_offset + rj, lane);  // NaN never ranks
+                if constexpr (!kFilter) {
+                    if (s == s) list_insert<METRIC>(my_s + q * k, my_i + q * k, k, s, row_offset + rj, lane);  // NaN never ranks
+                } else if (s == s && better<METRIC>(s, row_offset + rj, my_s[q * k + k - 1], my_i[q * k + k - 1])) {
+                    filtered_insert<METRIC>(my_s + q * k, my_i + q * k, k, s, row_offset + rj, allow, rj,
+                                            exclude + (int64_t)q * n_exclude, n_exclude, lane);
+                }
             }
         }
     }
@@ -384,6 +411,10 @@ __global__ void __launch_bounds__(kThreads) list_init_kernel(float* __restrict__
 // finish_score, NaN never ranks), keep the best k under (score, index), and CERTIFY the query when the exact k-th score is
 // strictly better than b_w -- then no outside row can enter -- or when the list holds every row of the shard.  Uncertified
 // queries are appended to uncert[] (count in *n_uncert); their outputs are written but unspecified.
+// Filtered calls need nothing here: the candidate pass proposes eligible rows only, so every proposal is eligible.  A row outside
+// the merged list is either ineligible, or had a key no better than its worker's threshold when it was seen -- and thresholds
+// only improve -- so the b_w test still bounds every eligible row left out.  A list with an empty slot (iw < 0) or a shard of at
+// most kp rows still means that every eligible row was proposed.
 template <int METRIC, bool kBf16>
 __global__ void __launch_bounds__(kThreads) score_certify_kernel(const void* __restrict__ catalog, int64_t n_rows, int64_t ld, int E,
                                                                  int64_t row_offset, const float* __restrict__ query, float inv_scale,
@@ -508,12 +539,14 @@ __global__ void __launch_bounds__(256) swap_build_kernel(const float* __restrict
     }
 }
 
-template <bool kBf16Cat>
+// kFilter: allow indexed by catalog row (first_row + b), exclude [n_exclude] global indices, as in score_topk_kernel.
+template <bool kBf16Cat, bool kFilter>
 __global__ void __launch_bounds__(kThreads) swap_error_topk_kernel(const float* __restrict__ outfit, const void* __restrict__ catalog,
                                                                    int64_t ld_cat, int64_t first_row, int B, int E, int slot, int io,
                                                                    float inv_scale, const float* __restrict__ y, int64_t ld_y,
                                                                    int64_t row_offset, int k, float* __restrict__ ws_score,
-                                                                   int64_t* __restrict__ ws_idx) {
+                                                                   int64_t* __restrict__ ws_idx, const uint8_t* __restrict__ allow,
+                                                                   const int64_t* __restrict__ exclude, int n_exclude) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     int64_t* li = reinterpret_cast<int64_t*>(smem_raw);                    // [kWarps][k]
     float* ls = reinterpret_cast<float*>(li + kWarps * k);                 // [kWarps][k]
@@ -536,7 +569,14 @@ __global__ void __launch_bounds__(kThreads) swap_error_topk_kernel(const float* 
             acc = fmaf(df, df, acc);
         }
         acc = warp_sum(acc);
-        if (acc == acc) list_insert<CODAE_METRIC_SQERR>(ls + warp * k, li + warp * k, k, acc, row_offset + first_row + b, lane);
+        if constexpr (!kFilter) {
+            if (acc == acc) list_insert<CODAE_METRIC_SQERR>(ls + warp * k, li + warp * k, k, acc, row_offset + first_row + b, lane);
+        } else {
+            const int64_t gi = row_offset + first_row + b;
+            if (acc == acc && better<CODAE_METRIC_SQERR>(acc, gi, ls[warp * k + k - 1], li[warp * k + k - 1]))
+                filtered_insert<CODAE_METRIC_SQERR>(ls + warp * k, li + warp * k, k, acc, gi, allow, first_row + b, exclude, n_exclude,
+                                                    lane);
+        }
     }
     __syncthreads();
     if (warp == 0) {
@@ -564,6 +604,15 @@ inline size_t topk_smem(int QC, int E, int k) {
     return (size_t)QC * E * 4 + (size_t)((QC + 3) & ~3) * 4 + (size_t)kWarps * QC * k * 12;
 }
 
+// Arguments of the *_filtered entry points (include/codae_b200.h).  Global indices must be >= 0 so that padding never matches.
+inline int check_filter(codae_ctx* ctx, const char* fn, int64_t row_offset, const int64_t* exclude, int n_exclude) {
+    CODAE_REQUIRE(ctx, n_exclude >= 0 && n_exclude <= CODAE_TOPK_MAX_EXCLUDE, "%s: n_exclude %d outside [0, %d]", fn, n_exclude,
+                  CODAE_TOPK_MAX_EXCLUDE);
+    CODAE_REQUIRE(ctx, (exclude != nullptr) == (n_exclude > 0), "%s: exclude must be non-NULL exactly when n_exclude > 0", fn);
+    CODAE_REQUIRE(ctx, row_offset >= 0, "%s: row_offset %lld < 0", fn, (long long)row_offset);
+    return CODAE_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -573,9 +622,10 @@ size_t codae_score_topk_workspace_bytes(const codae_ctx* ctx, int Q, int k) {
     return (size_t)ctx->sm_count * 4 * 4 /*QC max*/ * (size_t)k * 12 + 256;
 }
 
-int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
-                     int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k, float* out_score,
-                     int64_t* out_idx, void* workspace, size_t ws_bytes, void* stream) {
+// codae_score_topk and codae_score_topk_filtered; no filter (allow NULL, n_exclude 0) runs the unfiltered instantiations.
+static int score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E, int64_t row_offset,
+                      const float* query, int Q, float inv_scale, int metric, int k, const uint8_t* allow, const int64_t* exclude,
+                      int n_exclude, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes, void* stream) {
     CODAE_REQUIRE(ctx, ctx && catalog && query && out_score && out_idx && workspace, "codae_score_topk: NULL argument");
     CODAE_REQUIRE(ctx, k >= 1 && k <= kMaxK, "codae_score_topk: k %d outside [1, %d]", k, kMaxK);
     CODAE_REQUIRE(ctx, Q >= 1 && n_rows >= 0, "codae_score_topk: bad Q / n_rows");
@@ -591,6 +641,7 @@ int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t
                           codae_score_topk_workspace_bytes(ctx, Q, k));
     cudaStream_t s = as_stream(stream);
     merge_attrs();
+    const bool filtered = allow || n_exclude > 0;
     const int grid0 = sweep_grid(ctx, n_rows);
     int64_t* ws_idx = reinterpret_cast<int64_t*>(workspace);
     float* ws_score = reinterpret_cast<float*>(ws_idx + (size_t)grid0 * 4 * k);
@@ -600,16 +651,18 @@ int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t
         const int reps = (Q - q0 >= 4) ? 1 : (Q - q0);  // leftover queries one at a time
         for (int rpt = 0; rpt < reps; ++rpt) {
             const float* qptr = query + (int64_t)(q0 + rpt) * E;
+            const int64_t* xptr = exclude ? exclude + (int64_t)(q0 + rpt) * n_exclude : nullptr;
             const size_t smem = topk_smem(qc, E, k);
-#define LAUNCH(MET, QC, BF)                                                                                       \
-    do {                                                                                                          \
-        cudaFuncSetAttribute(score_topk_kernel<MET, QC, BF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        /* one resident wave: the grid-stride sweep balances itself only if every CTA runs from the start */          \
-        const int occ = resident_ctas_per_sm(score_topk_kernel<MET, QC, BF>, kThreads, smem);                          \
-        if (grid > ctx->sm_count * occ) grid = ctx->sm_count * occ;                                                  \
-        score_topk_kernel<MET, QC, BF><<<grid, kThreads, smem, s>>>(catalog, n_rows, ld, E, row_offset, qptr, inv_scale, k, \
-                                                                    ws_score, ws_idx);                           \
+#define LAUNCH_F(MET, QC, BF, F)                                                                                     \
+    do {                                                                                                             \
+        cudaFuncSetAttribute(score_topk_kernel<MET, QC, BF, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        /* one resident wave: the grid-stride sweep balances itself only if every CTA runs from the start */             \
+        const int occ = resident_ctas_per_sm(score_topk_kernel<MET, QC, BF, F>, kThreads, smem);                          \
+        if (grid > ctx->sm_count * occ) grid = ctx->sm_count * occ;                                                     \
+        score_topk_kernel<MET, QC, BF, F><<<grid, kThreads, smem, s>>>(catalog, n_rows, ld, E, row_offset, qptr, inv_scale, k, \
+                                                                       ws_score, ws_idx, allow, xptr, n_exclude);   \
     } while (0)
+#define LAUNCH(MET, QC, BF) do { if (filtered) LAUNCH_F(MET, QC, BF, true); else LAUNCH_F(MET, QC, BF, false); } while (0)
             if (metric == CODAE_METRIC_SQERR) {
                 if (qc == 4) { if (bf) LAUNCH(CODAE_METRIC_SQERR, 4, true); else LAUNCH(CODAE_METRIC_SQERR, 4, false); }
                 else { if (bf) LAUNCH(CODAE_METRIC_SQERR, 1, true); else LAUNCH(CODAE_METRIC_SQERR, 1, false); }
@@ -618,6 +671,7 @@ int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t
                 else { if (bf) LAUNCH(CODAE_METRIC_COSINE, 1, true); else LAUNCH(CODAE_METRIC_COSINE, 1, false); }
             }
 #undef LAUNCH
+#undef LAUNCH_F
             int rc = codae_check_launch(ctx, "score_topk_kernel");
             if (rc) return rc;
             if (metric == CODAE_METRIC_SQERR)
@@ -629,6 +683,23 @@ int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t
         }
     }
     return CODAE_OK;
+}
+
+int codae_score_topk(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                     int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k, float* out_score,
+                     int64_t* out_idx, void* workspace, size_t ws_bytes, void* stream) {
+    return score_topk(ctx, catalog, cat_dtype, n_rows, ld, E, row_offset, query, Q, inv_scale, metric, k, nullptr, nullptr, 0,
+                      out_score, out_idx, workspace, ws_bytes, stream);
+}
+
+int codae_score_topk_filtered(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                              int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
+                              const uint8_t* allow, const int64_t* exclude, int n_exclude, float* out_score, int64_t* out_idx,
+                              void* workspace, size_t ws_bytes, void* stream) {
+    const int rc = check_filter(ctx, "codae_score_topk_filtered", row_offset, exclude, n_exclude);
+    if (rc) return rc;
+    return score_topk(ctx, catalog, cat_dtype, n_rows, ld, E, row_offset, query, Q, inv_scale, metric, k, allow, exclude,
+                      n_exclude, out_score, out_idx, workspace, ws_bytes, stream);
 }
 
 int codae_topk_merge(codae_ctx* ctx, const float* scores, const int64_t* idx, int G, int Q, int k, int metric,
@@ -660,10 +731,10 @@ int codae_swap_build(codae_ctx* ctx, const float* outfit, const void* catalog, i
     return codae_check_launch(ctx, "swap_build_kernel");
 }
 
-int codae_swap_error_topk(codae_ctx* ctx, const float* outfit, const void* catalog, int cat_dtype, int64_t ld_cat,
-                          int64_t first_row, int B, int E, int slot, int io, float inv_scale, const float* y, int64_t ld_y,
-                          int64_t row_offset, int k, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes,
-                          void* stream) {
+static int swap_error_topk(codae_ctx* ctx, const float* outfit, const void* catalog, int cat_dtype, int64_t ld_cat,
+                           int64_t first_row, int B, int E, int slot, int io, float inv_scale, const float* y, int64_t ld_y,
+                           int64_t row_offset, int k, const uint8_t* allow, const int64_t* exclude, int n_exclude,
+                           float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes, void* stream) {
     CODAE_REQUIRE(ctx, ctx && outfit && catalog && y && out_score && out_idx && workspace, "codae_swap_error_topk: NULL argument");
     CODAE_REQUIRE(ctx, B >= 1 && E >= 1 && slot >= 0 && (slot + 1) * E <= io && ld_y >= io && ld_cat >= E && k >= 1 && k <= kMaxK,
                   "codae_swap_error_topk: bad shape");
@@ -675,15 +746,34 @@ int codae_swap_error_topk(codae_ctx* ctx, const float* outfit, const void* catal
     int64_t* ws_idx = reinterpret_cast<int64_t*>(workspace);
     float* ws_score = reinterpret_cast<float*>(ws_idx + (size_t)grid * k);
     const size_t smem = (size_t)kWarps * k * 12;
-    if (cat_dtype == CODAE_BF16)
-        swap_error_topk_kernel<true><<<grid, kThreads, smem, s>>>(outfit, catalog, ld_cat, first_row, B, E, slot, io, inv_scale, y, ld_y, row_offset, k, ws_score, ws_idx);
-    else
-        swap_error_topk_kernel<false><<<grid, kThreads, smem, s>>>(outfit, catalog, ld_cat, first_row, B, E, slot, io, inv_scale, y, ld_y, row_offset, k, ws_score, ws_idx);
+    const bool bc = cat_dtype == CODAE_BF16, filtered = allow || n_exclude > 0;
+#define LAUNCH(BC, F) swap_error_topk_kernel<BC, F><<<grid, kThreads, smem, s>>>(outfit, catalog, ld_cat, first_row, B, E, slot, io, inv_scale, y, ld_y, row_offset, k, ws_score, ws_idx, allow, exclude, n_exclude)
+    if (bc && filtered) LAUNCH(true, true); else if (bc) LAUNCH(true, false); else if (filtered) LAUNCH(false, true); else LAUNCH(false, false);
+#undef LAUNCH
     int rc = codae_check_launch(ctx, "swap_error_topk_kernel");
     if (rc) return rc;
     merge_attrs();
     topk_merge_kernel<CODAE_METRIC_SQERR><<<1, kThreads, merge_smem(), s>>>(ws_score, ws_idx, grid, 1, k, out_score, out_idx, 0, 1);
     return codae_check_launch(ctx, "topk_merge_kernel");
+}
+
+int codae_swap_error_topk(codae_ctx* ctx, const float* outfit, const void* catalog, int cat_dtype, int64_t ld_cat,
+                          int64_t first_row, int B, int E, int slot, int io, float inv_scale, const float* y, int64_t ld_y,
+                          int64_t row_offset, int k, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes,
+                          void* stream) {
+    return swap_error_topk(ctx, outfit, catalog, cat_dtype, ld_cat, first_row, B, E, slot, io, inv_scale, y, ld_y, row_offset, k,
+                           nullptr, nullptr, 0, out_score, out_idx, workspace, ws_bytes, stream);
+}
+
+int codae_swap_error_topk_filtered(codae_ctx* ctx, const float* outfit, const void* catalog, int cat_dtype, int64_t ld_cat,
+                                   int64_t first_row, int B, int E, int slot, int io, float inv_scale, const float* y,
+                                   int64_t ld_y, int64_t row_offset, int k, const uint8_t* allow, const int64_t* exclude,
+                                   int n_exclude, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes,
+                                   void* stream) {
+    const int rc = check_filter(ctx, "codae_swap_error_topk_filtered", row_offset, exclude, n_exclude);
+    if (rc) return rc;
+    return swap_error_topk(ctx, outfit, catalog, cat_dtype, ld_cat, first_row, B, E, slot, io, inv_scale, y, ld_y, row_offset, k,
+                           allow, exclude, n_exclude, out_score, out_idx, workspace, ws_bytes, stream);
 }
 
 int codae_score_rank(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
@@ -737,10 +827,10 @@ size_t codae_score_topk_batched_workspace_bytes(const codae_ctx* ctx, int cat_dt
     return batched_layout(ctx, cat_dtype == CODAE_BF16, n_rows, E, Q, k).total;
 }
 
-int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
-                             int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k, float* out_score,
-                             int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace, size_t ws_bytes,
-                             void* stream) {
+static int score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                              int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
+                              const uint8_t* allow, const int64_t* exclude, int n_exclude, float* out_score, int64_t* out_idx,
+                              int* n_uncertified, int* uncertified, void* workspace, size_t ws_bytes, void* stream) {
     CODAE_REQUIRE(ctx, ctx && catalog && query && out_score && out_idx && n_uncertified && uncertified && workspace,
                   "codae_score_topk_batched: NULL argument");
     CODAE_REQUIRE(ctx, k >= 1 && k <= CODAE_TOPK_BATCHED_MAX_K, "codae_score_topk_batched: k %d outside [1, %d]", k,
@@ -786,6 +876,7 @@ int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype,
     p.cc = cc; p.qq = qq;
     p.inv_scale = inv_scale; p.c_rel = batched_c_rel(E, bf);
     p.ls = ls; p.li = li;
+    p.exclude = exclude; p.n_exclude = n_exclude;
     for (int64_t c0 = 0; c0 < n_rows; c0 += L.chunk) {
         const int64_t rows = n_rows - c0 < L.chunk ? n_rows - c0 : L.chunk;
         if (bf) {
@@ -801,6 +892,7 @@ int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype,
         rc = codae_check_launch(ctx, "codae_score_topk_batched chunk");
         if (rc) return rc;
         p.n_rows = rows; p.row0 = row_offset + c0;
+        p.allow = allow ? allow + c0 : nullptr;
         for (int qb0 = 0; qb0 < L.QB; qb0 += L.G0) {
             p.qb0 = qb0;
             p.G = L.QB - qb0 < L.G0 ? L.QB - qb0 : L.G0;
@@ -820,6 +912,25 @@ int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype,
         else score_certify_kernel<CODAE_METRIC_COSINE, false><<<Q, kThreads, csmem, s>>>(catalog, n_rows, ld, E, row_offset, query, inv_scale, k, L.kp, m_key, m_idx, out_score, out_idx, n_uncertified, uncertified);
     }
     return codae_check_launch(ctx, "score_certify_kernel");
+}
+
+int codae_score_topk_batched(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                             int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k, float* out_score,
+                             int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace, size_t ws_bytes,
+                             void* stream) {
+    return score_topk_batched(ctx, catalog, cat_dtype, n_rows, ld, E, row_offset, query, Q, inv_scale, metric, k, nullptr,
+                              nullptr, 0, out_score, out_idx, n_uncertified, uncertified, workspace, ws_bytes, stream);
+}
+
+int codae_score_topk_batched_filtered(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,
+                                      int64_t row_offset, const float* query, int Q, float inv_scale, int metric, int k,
+                                      const uint8_t* allow, const int64_t* exclude, int n_exclude, float* out_score,
+                                      int64_t* out_idx, int* n_uncertified, int* uncertified, void* workspace, size_t ws_bytes,
+                                      void* stream) {
+    const int rc = check_filter(ctx, "codae_score_topk_batched_filtered", row_offset, exclude, n_exclude);
+    if (rc) return rc;
+    return score_topk_batched(ctx, catalog, cat_dtype, n_rows, ld, E, row_offset, query, Q, inv_scale, metric, k, allow, exclude,
+                              n_exclude, out_score, out_idx, n_uncertified, uncertified, workspace, ws_bytes, stream);
 }
 
 }  // extern "C"

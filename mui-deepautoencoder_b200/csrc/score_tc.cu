@@ -39,6 +39,8 @@
 //   always reach the re-scoring, which applies the sweep's NaN / inf rules exactly.)
 // A key is compared with the thread's threshold -- the worst entry of its list, in registers -- and inserted into the sorted list
 // (global memory, [W][Q][kp]) only when it beats it: after the first few tiles almost every column is one compare.
+// Filtered calls (kFilter) test the row's mask byte and the query's exclusion list only behind that compare, and an ineligible
+// row is skipped as if it were absent: the lists hold eligible rows only (the certification argument: score.cu).
 #include <float.h>
 
 #include "common.cuh"
@@ -65,7 +67,7 @@ __device__ __forceinline__ bool key_better(float sa, int64_t ia, float sb, int64
     return sa > sb || (sa == sb && ia < ib);
 }
 
-template <int METRIC, int NPB>
+template <int METRIC, int NPB, bool kFilter>
 __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(const __grid_constant__ CUtensorMap tma_q,
                                                                const __grid_constant__ CUtensorMap tma_c, const ScoreTcPass p) {
     using C = SCfg<NPB>;
@@ -160,6 +162,7 @@ __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(const __grid_cons
         float thr_s = live ? Ls[p.kp - 1] : 0.f;
         int64_t thr_i = live ? Li[p.kp - 1] : 0;
         const float qq = live ? p.qq[qrow] : 0.f;
+        const int64_t* ex = kFilter && live ? p.exclude + (size_t)qrow * p.n_exclude : nullptr;
         const float sc = p.inv_scale, s2 = sc * sc, m2s = -2.f * sc, c_rel = p.c_rel;
         int it = 0;
         for (int t = worker; t < tiles; t += p.W, ++it) {
@@ -197,6 +200,12 @@ __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(const __grid_cons
                     }
                     const int64_t gi = p.row0 + rc + j;
                     if (key_better<METRIC>(key, gi, thr_s, thr_i)) {
+                        if constexpr (kFilter) {
+                            if (p.allow && !p.allow[rc + j]) continue;
+                            int e = 0;
+                            while (e < p.n_exclude && ex[e] != gi) ++e;
+                            if (e < p.n_exclude) continue;
+                        }
                         int pos = p.kp - 1;
                         while (pos > 0) {
                             const float ps = Ls[pos - 1];
@@ -223,18 +232,18 @@ __global__ void __launch_bounds__(kThreads, 1) score_tc_kernel(const __grid_cons
     }
 }
 
-template <int METRIC, int NPB>
+template <int METRIC, int NPB, bool kFilter>
 int launch_pass(codae_ctx* ctx, const ScoreTcPass& p, cudaStream_t s) {
     using C = SCfg<NPB>;
     static const cudaError_t attr =
-        cudaFuncSetAttribute(score_tc_kernel<METRIC, NPB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmemBytes);
+        cudaFuncSetAttribute(score_tc_kernel<METRIC, NPB, kFilter>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmemBytes);
     if (attr != cudaSuccess) return codae_fail(ctx, CODAE_ECUDA, "score_tc_kernel: cudaFuncSetAttribute: %s", cudaGetErrorString(attr));
     CUtensorMap mq, mc;
     int rc = codae_tc05_make_map(ctx, &mq, p.q_planes, p.Q, p.E, p.q_ld, BK, BM, 2, p.q_plane_stride);
     if (rc) return rc;
     rc = codae_tc05_make_map(ctx, &mc, p.cat, p.n_rows, p.E, p.cat_ld, BK, kTileN, NPB, p.cat_plane_stride);
     if (rc) return rc;
-    score_tc_kernel<METRIC, NPB><<<p.G * p.W, kThreads, C::kSmemBytes, s>>>(mq, mc, p);
+    score_tc_kernel<METRIC, NPB, kFilter><<<p.G * p.W, kThreads, C::kSmemBytes, s>>>(mq, mc, p);
     return codae_check_launch(ctx, "score_tc_kernel");
 }
 
@@ -244,6 +253,10 @@ int codae_score_tc_pass(codae_ctx* ctx, const ScoreTcPass& p, cudaStream_t s) {
     if (!ctx->encode_tiled) return codae_fail(ctx, CODAE_EARCH, "score_tc_kernel: no tensor-map encoder (driver too old)");
     if (p.n_rows < 1) return CODAE_OK;
     const bool two = p.cat_planes == 2;
-    if (p.metric == CODAE_METRIC_SQERR) return two ? launch_pass<CODAE_METRIC_SQERR, 2>(ctx, p, s) : launch_pass<CODAE_METRIC_SQERR, 1>(ctx, p, s);
-    return two ? launch_pass<CODAE_METRIC_COSINE, 2>(ctx, p, s) : launch_pass<CODAE_METRIC_COSINE, 1>(ctx, p, s);
+    if (p.allow || p.n_exclude > 0) {
+        if (p.metric == CODAE_METRIC_SQERR) return two ? launch_pass<CODAE_METRIC_SQERR, 2, true>(ctx, p, s) : launch_pass<CODAE_METRIC_SQERR, 1, true>(ctx, p, s);
+        return two ? launch_pass<CODAE_METRIC_COSINE, 2, true>(ctx, p, s) : launch_pass<CODAE_METRIC_COSINE, 1, true>(ctx, p, s);
+    }
+    if (p.metric == CODAE_METRIC_SQERR) return two ? launch_pass<CODAE_METRIC_SQERR, 2, false>(ctx, p, s) : launch_pass<CODAE_METRIC_SQERR, 1, false>(ctx, p, s);
+    return two ? launch_pass<CODAE_METRIC_COSINE, 2, false>(ctx, p, s) : launch_pass<CODAE_METRIC_COSINE, 1, false>(ctx, p, s);
 }

@@ -7,10 +7,15 @@ top-k.  The catalog is sharded by rows across ranks (torchrun), merged with an a
 
 --mode swap scores every candidate SWAP by the reconstruction error of the whole swapped outfit instead
 (candidate substituted into the slot, DAE forward per candidate; codae.tool.SwapScorer).
+
+--exclude_own_item leaves out, for query q, catalog row q (the item outfit q already holds in the slot: a trained DAE
+reconstructs it closely, and swapping it in is the identity swap); --allowed_rows PATH.npy restricts the results to the
+global row ids stored there (int64).  Both filter inside the kernels, so k results come back whenever k rows are eligible.
 """
 import argparse
 import json
 
+import numpy as np
 import torch
 import yaml
 
@@ -35,7 +40,20 @@ def parse():
     parser.add_argument('--queries', type=int, default=4)
     parser.add_argument('--synthetic', type=int, default=0)
     parser.add_argument('--catalog_dtype', type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
+    parser.add_argument('--exclude_own_item', action='store_true', help="query q never gets catalog row q back")
+    parser.add_argument('--allowed_rows', type=str, default=None, help=".npy of int64 global row ids that may be returned")
     return parser.parse_args()
+
+
+def local_allowed(path, lo, n_local, device):
+    """Mask of this rank's rows [lo, lo + n_local) from a file of global row ids (None without a file)."""
+    if path is None:
+        return None
+    rows = torch.from_numpy(np.load(path).astype(np.int64).reshape(-1))
+    rows = rows[(rows >= lo) & (rows < lo + n_local)] - lo
+    mask = torch.zeros(n_local, dtype=torch.bool)
+    mask[rows] = True
+    return mask.to(device)
 
 
 if __name__ == "__main__":
@@ -62,20 +80,22 @@ if __name__ == "__main__":
     if args.catalog_dtype == "bf16":
         shard = shard.to(torch.bfloat16)
     outfits = dataset.data[:args.queries].to(device)
+    allowed = local_allowed(args.allowed_rows, lo, n_local, device)
+    own = torch.arange(outfits.shape[0], dtype=torch.int64, device=device).view(-1, 1) if args.exclude_own_item else None
     if args.mode == "swap":
         if args.metric != "sqerr":
             raise Exception("Swap mode scores by squared reconstruction error.")
-        scorer = SwapScorer(model, shard.contiguous(), E, k=args.k, inv_scale=1.0 / dataset.scale, row_offset=lo)
-        res = [scorer.topk(outfits[q], args.slot) for q in range(outfits.shape[0])]
+        scorer = SwapScorer(model, shard.contiguous(), E, k=args.k, inv_scale=1.0 / dataset.scale, row_offset=lo, allowed=allowed)
+        res = [scorer.topk(outfits[q], args.slot, None if own is None else own[q]) for q in range(outfits.shape[0])]
         if rank == 0:
             print(json.dumps({"slot": args.slot, "mode": "swap", "metric": "sqerr", "k": args.k,
                               "indices": [i.cpu().tolist() for _, i in res], "scores": [s.cpu().tolist() for s, _ in res]}))
         raise SystemExit(0)
     scorer = ComplementarityScorer(shard.contiguous(), E, metric=args.metric, k=args.k, inv_scale=1.0 / dataset.scale,
-                                   row_offset=lo)
+                                   row_offset=lo, allowed=allowed)
     p = predict_slot(model, outfits, args.slot, E)
     # large query batches: one tensor-core pass over the catalog, results identical to the row sweep
-    scores, idx = scorer.topk_batched(p) if p.shape[0] >= ComplementarityScorer.TC_MIN_Q else scorer.topk(p)
+    scores, idx = scorer.topk_batched(p, own) if p.shape[0] >= ComplementarityScorer.TC_MIN_Q else scorer.topk(p, own)
     if rank == 0:
         print(json.dumps({"slot": args.slot, "metric": args.metric, "k": args.k,
                           "indices": idx.cpu().tolist(), "scores": scores.cpu().tolist()}))
