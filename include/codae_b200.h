@@ -398,6 +398,37 @@ int codae_swap_error_topk_filtered(codae_ctx* ctx, const float* outfit, const vo
                                    int64_t ld_y, int64_t row_offset, int k, const uint8_t* allow, const int64_t* exclude,
                                    int n_exclude, float* out_score, int64_t* out_idx, void* workspace, size_t ws_bytes,
                                    void* stream);
+/* Swaps over per-outfit candidate lists (re-ranking: retrieve M rows per outfit cheaply, score those M by swap error).  Any set of
+ * (outfit, candidate) pairs goes through the same GEMM chain in chunks of B rows, however the pairs are spread over outfits:
+ *   outfits    [Q, ld_outfit] f32, scaled rows (io columns used); one slot for every outfit.
+ *   candidates int64 [Q][m] GLOBAL catalog row ids (row_offset + local row), entries < 0 are padding; the same list fits every
+ *              shard.  Pairs are numbered p = q * m + j (0 <= p < Q m <= INT32_MAX).
+ *   pos        int64 [B]: built row b holds pair pos[b].  Its outfit is q = pos[b] / m, its local catalog row
+ *              candidates[pos[b]] - row_offset.
+ * A pos outside [0, Q m) or a local row outside [0, n_rows) is never dereferenced: the row is built as zeros and no error is written
+ * for it (pos and candidates are device data; the host cannot check them without a synchronisation).
+ *   codae_swap_build_pairs  x'[b, :] = outfit q with the slot columns replaced by catalog row * inv_scale, f32|bf16, pitch ld_x --
+ *                           codae_swap_build's values for that outfit and row.
+ *   codae_swap_error_pairs  err[pos[b]] = the swap error of built row b from y [B, ld_y] f32; err is [Q m] f32, set to NaN by the
+ *                           caller, so pairs that are not built stay NaN.
+ *   codae_swap_pairs_topk   per outfit, the best k (1 <= k <= 128) pairs by (error, candidate id): out_score / out_idx [Q][k],
+ *                           best first, NaN errors and ids < 0 skipped, unused slots (+inf, -1); a duplicated id is returned once
+ *                           per listing.  Lists of several ranks are combined with codae_topk_merge (CODAE_METRIC_SQERR).
+ * Numerics: a pair's error is computed exactly as codae_swap_error_topk computes a candidate's -- the same build values, the same
+ * codae_linear_fwd chain, the same per-lane fmaf order and warp_sum over io.  A GEMM row's result depends only on that row and on
+ * the launch's shape (the tensor-core plan follows the row count through its 128-row tile count), so (a) pairs in chunks of
+ * the same tile counts get the same bits
+ * wherever they sit and whatever the other rows of the chunk are, and in particular one outfit listing rows row_offset ..
+ * row_offset + n_rows - 1 in order gives the sweep's errors and ids bit for bit; (b) otherwise errors agree with the fp64
+ * reference to the engine's tolerance.  Bad shapes, k, NULL arguments return CODAE_EINVAL.                          */
+int codae_swap_build_pairs(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, const void* catalog, int cat_dtype,
+                           int64_t ld_cat, int64_t n_rows, int64_t row_offset, const int64_t* candidates, int m, const int64_t* pos,
+                           int B, int E, int slot, int io, float inv_scale, void* out_x, int x_dtype, int64_t ld_x, void* stream);
+int codae_swap_error_pairs(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, const void* catalog, int cat_dtype,
+                           int64_t ld_cat, int64_t n_rows, int64_t row_offset, const int64_t* candidates, int m, const int64_t* pos,
+                           int B, int E, int slot, int io, float inv_scale, const float* y, int64_t ld_y, float* err, void* stream);
+int codae_swap_pairs_topk(codae_ctx* ctx, const float* err, const int64_t* candidates, int Q, int m, int k, float* out_score,
+                          int64_t* out_idx, void* stream);
 
 #ifdef __cplusplus
 }

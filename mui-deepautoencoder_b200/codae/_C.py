@@ -81,6 +81,11 @@ SIGNATURES = {
                                    _sz, _vp]),
     "codae_swap_error_topk_filtered": (_i, [_vp, _vp, _vp, _i, _i64, _i64, _i, _i, _i, _i, _f, _vp, _i64, _i64, _i, _vp, _vp, _i,
                                             _vp, _vp, _vp, _sz, _vp]),
+    "codae_swap_build_pairs": (_i, [_vp, _vp, _i64, _i, _vp, _i, _i64, _i64, _i64, _vp, _i, _vp, _i, _i, _i, _i, _f, _vp, _i, _i64,
+                                    _vp]),
+    "codae_swap_error_pairs": (_i, [_vp, _vp, _i64, _i, _vp, _i, _i64, _i64, _i64, _vp, _i, _vp, _i, _i, _i, _i, _f, _vp, _i64, _vp,
+                                    _vp]),
+    "codae_swap_pairs_topk": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
 }
 
 DP_MAX_WORLD = 8
@@ -563,6 +568,35 @@ def swap_error_topk(outfit, catalog, first_row, B, E, slot, io, inv_scale, y, ro
     check(lib().codae_swap_error_topk_filtered(c, p(outfit), p(catalog), dt(catalog), catalog.stride(0), first_row, B, E, slot,
                                                io, inv_scale, p(y), y.stride(0), row_offset, k, p(allow), p(ex), m, p(out_score),
                                                p(out_idx), p(ws), ws.numel(), stream()), c)
+
+
+def swap_build_pairs(outfits, catalog, row_offset, candidates, pos, E, slot, io, inv_scale, out_x):
+    """Rows of out_x: the pairs pos [B] (int64 indices into candidates [Q, m], global row ids) swapped into `slot` of their
+    outfit (outfits [Q, io] f32)."""
+    _dev_check(outfits, catalog, candidates, pos, out_x)
+    c = ctx(catalog.device)
+    Q, m = candidates.shape
+    check(lib().codae_swap_build_pairs(c, p(outfits), outfits.stride(0), Q, p(catalog), dt(catalog), catalog.stride(0),
+                                       catalog.shape[0], row_offset, p(candidates), m, p(pos), pos.numel(), E, slot, io, inv_scale,
+                                       p(out_x), dt(out_x), out_x.stride(0), stream()), c)
+
+
+def swap_error_pairs(outfits, catalog, row_offset, candidates, pos, E, slot, io, inv_scale, y, err):
+    """err [Q m] f32: err[pos[b]] = swap error of reconstruction row b of y."""
+    _dev_check(outfits, catalog, candidates, pos, y, err)
+    c = ctx(catalog.device)
+    Q, m = candidates.shape
+    check(lib().codae_swap_error_pairs(c, p(outfits), outfits.stride(0), Q, p(catalog), dt(catalog), catalog.stride(0),
+                                       catalog.shape[0], row_offset, p(candidates), m, p(pos), pos.numel(), E, slot, io, inv_scale,
+                                       p(y), y.stride(0), p(err), stream()), c)
+
+
+def swap_pairs_topk(err, candidates, k, out_score, out_idx):
+    """Best k pairs per outfit by (error, candidate id): out_score [Q, k] f32, out_idx [Q, k] int64."""
+    _dev_check(err, candidates, out_score, out_idx)
+    c = ctx(err.device)
+    Q, m = candidates.shape
+    check(lib().codae_swap_pairs_topk(c, p(err), p(candidates), Q, m, k, p(out_score), p(out_idx), stream()), c)
 
 
 def linear_engine(device, dtype, M, N, K):

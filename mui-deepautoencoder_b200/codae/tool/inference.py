@@ -50,6 +50,41 @@ def _exclusions(exclude, shape0, device):
     return exclude.contiguous()
 
 
+def _pair_lists(outfits, candidates, io, device):
+    """SwapScorer.rerank_local's inputs: outfits fp32 [Q, io] and candidates int64 [Q, m] (Q m <= 2**31 - 1), both on the
+    catalog's device; contiguous copies."""
+    if not isinstance(outfits, torch.Tensor) or outfits.dtype != torch.float32:
+        raise RuntimeError("codae: outfits must be a float32 tensor")
+    if outfits.dim() != 2 or outfits.shape[1] != io or outfits.shape[0] < 1:
+        raise RuntimeError("codae: outfits must have shape [Q, %d] with Q >= 1, got %s" % (io, tuple(outfits.shape)))
+    if not isinstance(candidates, torch.Tensor) or candidates.dtype != torch.int64:
+        raise RuntimeError("codae: candidates must be an int64 tensor")
+    if candidates.dim() != 2 or candidates.shape[0] != outfits.shape[0] or candidates.shape[1] < 1:
+        raise RuntimeError("codae: candidates must have shape [%d, m] with m >= 1, got %s" % (outfits.shape[0],
+                                                                                           tuple(candidates.shape)))
+    if candidates.numel() > 2 ** 31 - 1:
+        raise RuntimeError("codae: candidates has %d entries, more than 2**31 - 1" % candidates.numel())
+    for name, t in (("outfits", outfits), ("candidates", candidates)):
+        if not t.is_cuda or t.device != device:
+            raise RuntimeError("codae: %s must be on the catalog's device %s" % (name, device))
+    return outfits.contiguous(), candidates.contiguous()
+
+
+def _gather_merge(pg, s, i, metric):
+    """All-gather of every rank's [Q, k] lists and the deterministic merge (codae_topk_merge); one process: (s, i)."""
+    import torch.distributed as dist
+    if pg is None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
+        return s, i
+    G = dist.get_world_size(pg)
+    gs = torch.empty((G,) + tuple(s.shape), dtype=s.dtype, device=s.device)
+    gi = torch.empty((G,) + tuple(i.shape), dtype=i.dtype, device=i.device)
+    dist.all_gather_into_tensor(gs, s.contiguous(), group=pg)
+    dist.all_gather_into_tensor(gi, i.contiguous(), group=pg)
+    out_s, out_i = torch.empty_like(s), torch.empty_like(i)
+    _C.topk_merge(gs, gi, metric, out_s, out_i)
+    return out_s, out_i
+
+
 def shard_rows(n_rows, world_size, rank):
     """Contiguous ceil(N/G)-row shards: (row_offset, n_local)."""
     per = (n_rows + world_size - 1) // world_size
@@ -140,24 +175,11 @@ class ComplementarityScorer:
         """Global top-k of a query batch: topk_local_batched on this rank's shard (certification and fallback are per rank),
         then the same all-gather + merge as topk -- every rank reaches it exactly once, whatever its fallback count.
         exclude holds global indices, so every rank is given the same tensor."""
-        return self._gather_merge(*self.topk_local_batched(query, exclude))
+        return _gather_merge(self.pg, *self.topk_local_batched(query, exclude), self.metric)
 
     def topk(self, query, exclude=None):
         """Global top-k: local sweep, all-gather of k x 12 bytes per query, deterministic merge."""
-        return self._gather_merge(*self.topk_local(query, exclude))
-
-    def _gather_merge(self, s, i):
-        import torch.distributed as dist
-        if self.pg is None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
-            return s, i
-        G = dist.get_world_size(self.pg)
-        gs = torch.empty((G,) + tuple(s.shape), dtype=s.dtype, device=s.device)
-        gi = torch.empty((G,) + tuple(i.shape), dtype=i.dtype, device=i.device)
-        dist.all_gather_into_tensor(gs, s.contiguous(), group=self.pg)
-        dist.all_gather_into_tensor(gi, i.contiguous(), group=self.pg)
-        out_s, out_i = torch.empty_like(s), torch.empty_like(i)
-        _C.topk_merge(gs, gi, self.metric, out_s, out_i)
-        return out_s, out_i
+        return _gather_merge(self.pg, *self.topk_local(query, exclude), self.metric)
 
 
 def predict_slot(model, outfits, slot, embedding_size):
@@ -205,18 +227,30 @@ class SwapScorer:
             self._acts = (eng, acts, stage)
         return self._acts
 
+    def _prepare(self):
+        """Weights and activation buffers of one scoring call: (engine, activations, fp32 stage or None, GEMM weights)."""
+        m = self.model
+        m.sync_weights()          # a sharded data-parallel trainer gathers the master weights first (collective)
+        eng, acts, stage = self._buffers()
+        m.refresh_shadow()
+        return eng, acts, stage, m.gemm_weights(eng)
+
+    def _forward(self, eng, acts, wflat, B):
+        """The DAE's Linear layers on the B swapped outfits in acts[0]; the reconstructions land in acts[-1]."""
+        m = self.model
+        for l, (i, o) in enumerate(m.dims):
+            _C.linear_fwd(acts[l], m.aug_view(wflat, l), None, acts[l + 1], B, o, (i + 7) // 8 * 8 + 1,
+                          _C.ACT_RELU if m.relu[l] else _C.ACT_NONE, eng)
+
     def topk_local(self, outfit, slot, exclude=None):
         """outfit: [io] scaled fp32 row.  Returns (errors [k], global candidate indices [k]) of this shard.  exclude: int64
         [m] CUDA tensor of global candidate indices not to return (-1 padding, m <= 256), e.g. the item already in the slot."""
-        m, dev = self.model, self.catalog.device
+        dev = self.catalog.device
         if not 0 <= slot < self.io // self.E:
             raise Exception("Slot out of range.")
         ex = _exclusions(exclude, None, dev)
         outfit = outfit.to(torch.float32).contiguous().view(-1)
-        m.sync_weights()          # a sharded data-parallel trainer gathers the master weights first (collective)
-        eng, acts, stage = self._buffers()
-        m.refresh_shadow()
-        wflat = m.gemm_weights(eng)
+        eng, acts, stage, wflat = self._prepare()
         n = self.catalog.shape[0]
         n_chunks = max(1, (n + self.chunk - 1) // self.chunk)
         ls = torch.full((n_chunks, 1, self.k), float("inf"), dtype=torch.float32, device=dev)
@@ -229,9 +263,7 @@ class SwapScorer:
             else:
                 _C.swap_build(outfit, self.catalog, first, B, self.E, slot, self.io, self.inv_scale, stage)
                 _C.split_x3(stage, acts[0])
-            for l, (i, o) in enumerate(m.dims):
-                _C.linear_fwd(acts[l], m.aug_view(wflat, l), None, acts[l + 1], B, o, (i + 7) // 8 * 8 + 1,
-                              _C.ACT_RELU if m.relu[l] else _C.ACT_NONE, eng)
+            self._forward(eng, acts, wflat, B)
             _C.swap_error_topk(outfit, self.catalog, first, B, self.E, slot, self.io, self.inv_scale, acts[-1],
                                self.row_offset, self.k, ls[c, 0], li[c, 0], self._ws, allow=self.allowed, exclude=ex)
         out_s = torch.empty((1, self.k), dtype=torch.float32, device=dev)
@@ -241,14 +273,51 @@ class SwapScorer:
 
     def topk(self, outfit, slot, exclude=None):
         s, i = self.topk_local(outfit, slot, exclude)
-        import torch.distributed as dist
-        if self.pg is None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
-            return s, i
-        G = dist.get_world_size(self.pg)
-        gs = torch.empty((G, 1, self.k), dtype=s.dtype, device=s.device)
-        gi = torch.empty((G, 1, self.k), dtype=i.dtype, device=i.device)
-        dist.all_gather_into_tensor(gs, s.view(1, 1, -1).contiguous(), group=self.pg)
-        dist.all_gather_into_tensor(gi, i.view(1, 1, -1).contiguous(), group=self.pg)
-        out_s, out_i = torch.empty_like(gs[0]), torch.empty_like(gi[0])
-        _C.topk_merge(gs, gi, _C.METRIC_SQERR, out_s, out_i)
-        return out_s[0], out_i[0]
+        s, i = _gather_merge(self.pg, s.view(1, -1), i.view(1, -1), _C.METRIC_SQERR)
+        return s[0], i[0]
+
+    def _owned_positions(self, candidates):
+        """Positions (ascending, int64) in the flattened [Q, m] list of the entries this shard scores: not padding, inside
+        [row_offset, row_offset + n_local), allowed.  nonzero() reads the count back: one host synchronisation."""
+        n = self.catalog.shape[0]
+        flat = candidates.reshape(-1)
+        r = flat - self.row_offset
+        own = (flat >= 0) & (r >= 0) & (r < n)
+        if self.allowed is not None and n > 0:
+            own &= self.allowed[r.clamp(0, n - 1)].bool()
+        return torch.nonzero(own).view(-1)
+
+    def rerank_local(self, outfits, slot, candidates):
+        """Re-rank per-outfit candidate lists by swap error.  outfits: [Q, io] scaled fp32 rows on the catalog's device;
+        candidates: int64 [Q, m] CUDA tensor of GLOBAL catalog row ids (< 0: padding; every rank gets the same tensor).
+        Returns (errors [Q, k] f32, global ids [Q, k] i64) of the listed pairs this shard holds, best first, ties -> lower id,
+        unused slots (+inf, -1); rows outside the shard, padding and rows `allowed` forbids are not scored, NaN errors never
+        rank, a duplicated id is returned once per listing.  The owned pairs go through the DAE in chunks of `chunk` rows,
+        whatever outfits they belong to; a pair's error is computed as topk_local computes it (bit for bit when the chunk
+        shapes coincide).  Synchronises once (_owned_positions)."""
+        dev = self.catalog.device
+        if not 0 <= slot < self.io // self.E:
+            raise Exception("Slot out of range.")
+        outfits, cand = _pair_lists(outfits, candidates, self.io, dev)
+        Q, mm = cand.shape
+        pos = self._owned_positions(cand)
+        err = torch.full((Q * mm,), float("nan"), dtype=torch.float32, device=dev)
+        eng, acts, stage, wflat = self._prepare()      # on every rank, pairs or not: sync_weights may be a collective
+        for c0 in range(0, pos.numel(), self.chunk):
+            pc = pos[c0:c0 + self.chunk]
+            _C.swap_build_pairs(outfits, self.catalog, self.row_offset, cand, pc, self.E, slot, self.io, self.inv_scale,
+                                acts[0] if stage is None else stage)
+            if stage is not None:
+                _C.split_x3(stage, acts[0])
+            self._forward(eng, acts, wflat, pc.numel())
+            _C.swap_error_pairs(outfits, self.catalog, self.row_offset, cand, pc, self.E, slot, self.io, self.inv_scale, acts[-1],
+                                err)
+        out_s = torch.empty((Q, self.k), dtype=torch.float32, device=dev)
+        out_i = torch.empty((Q, self.k), dtype=torch.int64, device=dev)
+        _C.swap_pairs_topk(err, cand, self.k, out_s, out_i)
+        return out_s, out_i
+
+    def rerank(self, outfits, slot, candidates):
+        """Global rerank_local: every rank scores the listed rows it holds, then all-gather of k entries per outfit and the
+        deterministic merge (codae_topk_merge)."""
+        return _gather_merge(self.pg, *self.rerank_local(outfits, slot, candidates), _C.METRIC_SQERR)

@@ -539,6 +539,31 @@ __global__ void __launch_bounds__(256) swap_build_kernel(const float* __restrict
     }
 }
 
+// Swap error of built row b: sum_d (y[b, d] - x'_d)^2 with x' recomputed in fp32 from the outfit and catalog row first_row + b
+// (lane-strided fmaf over io, then the warp_sum tree).  The one definition of a swap's error: codae_swap_error_topk and
+// codae_swap_error_pairs both call it, so a pair's error equals the row sweep's bit for bit whenever the GEMM chain computed the
+// same y row.  The row is passed as (first_row, b) because that is how swap_error_topk_kernel indexed it before this helper existed:
+// written so, the kernel keeps its SASS opcode sequence (profiles/r05_sass_swap_error.jsonl).
+template <bool kBf16Cat>
+__device__ __forceinline__ float swap_row_error(const float* __restrict__ outfit, const void* __restrict__ catalog, int64_t ld_cat,
+                                                int64_t first_row, int lo, int hi, int io, float inv_scale, const float* __restrict__ y,
+                                                int64_t ld_y, int b, int lane) {
+    float acc = 0.f;
+    for (int d = lane; d < io; d += 32) {
+        float t;
+        if (d >= lo && d < hi) {
+            const int64_t off = (first_row + b) * ld_cat + (d - lo);
+            t = (kBf16Cat ? __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(catalog)[off])
+                          : reinterpret_cast<const float*>(catalog)[off]) * inv_scale;
+        } else {
+            t = outfit[d];
+        }
+        const float df = y[(int64_t)b * ld_y + d] - t;
+        acc = fmaf(df, df, acc);
+    }
+    return warp_sum(acc);
+}
+
 // kFilter: allow indexed by catalog row (first_row + b), exclude [n_exclude] global indices, as in score_topk_kernel.
 template <bool kBf16Cat, bool kFilter>
 __global__ void __launch_bounds__(kThreads) swap_error_topk_kernel(const float* __restrict__ outfit, const void* __restrict__ catalog,
@@ -555,20 +580,7 @@ __global__ void __launch_bounds__(kThreads) swap_error_topk_kernel(const float* 
     __syncthreads();
     const int lo = slot * E, hi = lo + E;
     for (int b = blockIdx.x * kWarps + warp; b < B; b += gridDim.x * kWarps) {
-        float acc = 0.f;
-        for (int d = lane; d < io; d += 32) {
-            float t;
-            if (d >= lo && d < hi) {
-                const int64_t off = (first_row + b) * ld_cat + (d - lo);
-                t = (kBf16Cat ? __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(catalog)[off])
-                              : reinterpret_cast<const float*>(catalog)[off]) * inv_scale;
-            } else {
-                t = outfit[d];
-            }
-            const float df = y[(int64_t)b * ld_y + d] - t;
-            acc = fmaf(df, df, acc);
-        }
-        acc = warp_sum(acc);
+        const float acc = swap_row_error<kBf16Cat>(outfit, catalog, ld_cat, first_row, lo, hi, io, inv_scale, y, ld_y, b, lane);
         if constexpr (!kFilter) {
             if (acc == acc) list_insert<CODAE_METRIC_SQERR>(ls + warp * k, li + warp * k, k, acc, row_offset + first_row + b, lane);
         } else {
@@ -589,6 +601,111 @@ __global__ void __launch_bounds__(kThreads) swap_error_topk_kernel(const float* 
             ws_score[(int64_t)blockIdx.x * k + e] = ls[e];
             ws_idx[(int64_t)blockIdx.x * k + e] = li[e];
         }
+    }
+}
+
+// ---- swaps over per-outfit candidate lists (re-ranking) -------------------------------------------------------------------
+// The list is candidates [Q][m] (global row ids, < 0 padding), flattened to pairs p = q * m + j.  A chunk of B built rows takes
+// its pairs from pos [B] (indices into the flattened list).  Row b is valid when 0 <= pos[b] < Q m and its local catalog row
+// candidates[pos[b]] - row_offset lies in [0, n_rows); an invalid row is built as zeros and gets no error, so device-side ids and
+// positions are never dereferenced out of range.
+__device__ __forceinline__ bool pair_row(const int64_t* __restrict__ pos, const int64_t* __restrict__ candidates, int64_t n_pairs,
+                                         int m, int64_t n_rows, int64_t row_offset, int b, int64_t& p, int64_t& q, int64_t& r) {
+    p = pos[b];
+    if (p < 0 || p >= n_pairs) return false;
+    q = p / m;
+    r = candidates[p] - row_offset;
+    return r >= 0 && r < n_rows;
+}
+
+//   swap_build_pairs_kernel   x'[b, :] = outfit q with columns [slot*E, (slot+1)*E) replaced by catalog row r * inv_scale --
+//                             swap_build_kernel's values, gathered per pair.  V = 4: four columns per thread, the outfit read with
+//                             one 16-byte load (io, E, ld_outfit multiples of 4 and a 16-byte aligned outfit base).
+template <bool kBf16Cat, bool kBf16Out, int V>
+__global__ void __launch_bounds__(256) swap_build_pairs_kernel(const float* __restrict__ outfits, int64_t ld_outfit, int64_t n_pairs,
+                                                               const void* __restrict__ catalog, int64_t ld_cat, int64_t n_rows,
+                                                               int64_t row_offset, const int64_t* __restrict__ candidates, int m,
+                                                               const int64_t* __restrict__ pos, int B, int E, int slot, int io,
+                                                               float inv_scale, void* __restrict__ out, int64_t ld_out) {
+    const int per_row = io / V;
+    const int64_t total = (int64_t)B * per_row;
+    const int lo = slot * E, hi = lo + E;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+        const int b = (int)(e / per_row), d0 = (int)(e - (int64_t)b * per_row) * V;
+        int64_t p, q, r;
+        float v[V];
+        if (!pair_row(pos, candidates, n_pairs, m, n_rows, row_offset, b, p, q, r)) {
+#pragma unroll
+            for (int j = 0; j < V; ++j) v[j] = 0.f;
+        } else if (d0 >= lo && d0 < hi) {           // V divides E: the V columns are all inside the slot or all outside
+            const int64_t off = r * ld_cat + (d0 - lo);
+#pragma unroll
+            for (int j = 0; j < V; ++j)
+                v[j] = (kBf16Cat ? __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(catalog)[off + j])
+                                 : reinterpret_cast<const float*>(catalog)[off + j]) * inv_scale;
+        } else if constexpr (V == 4) {
+            const float4 o = *reinterpret_cast<const float4*>(outfits + q * ld_outfit + d0);
+            v[0] = o.x; v[1] = o.y; v[2] = o.z; v[3] = o.w;
+        } else {
+            v[0] = outfits[q * ld_outfit + d0];
+        }
+#pragma unroll
+        for (int j = 0; j < V; ++j) {
+            if (kBf16Out) reinterpret_cast<__nv_bfloat16*>(out)[(int64_t)b * ld_out + d0 + j] = __float2bfloat16_rn(v[j]);
+            else reinterpret_cast<float*>(out)[(int64_t)b * ld_out + d0 + j] = v[j];
+        }
+    }
+}
+
+//   swap_error_pairs_kernel   err[p] = swap_row_error of built row b (one warp per row, as swap_error_topk_kernel)
+template <bool kBf16Cat>
+__global__ void __launch_bounds__(kThreads) swap_error_pairs_kernel(const float* __restrict__ outfits, int64_t ld_outfit,
+                                                                    int64_t n_pairs, const void* __restrict__ catalog, int64_t ld_cat,
+                                                                    int64_t n_rows, int64_t row_offset,
+                                                                    const int64_t* __restrict__ candidates, int m,
+                                                                    const int64_t* __restrict__ pos, int B, int E, int slot, int io,
+                                                                    float inv_scale, const float* __restrict__ y, int64_t ld_y,
+                                                                    float* __restrict__ err) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lo = slot * E, hi = lo + E;
+    for (int b = blockIdx.x * kWarps + warp; b < B; b += gridDim.x * kWarps) {
+        int64_t p, q, r;
+        if (!pair_row(pos, candidates, n_pairs, m, n_rows, row_offset, b, p, q, r)) continue;
+        const float acc = swap_row_error<kBf16Cat>(outfits + q * ld_outfit, catalog, ld_cat, r - b /* row r */, lo, hi, io, inv_scale,
+                                                   y, ld_y, b, lane);
+        if (lane == 0) err[p] = acc;
+    }
+}
+
+//   swap_pairs_topk_kernel    one warp per outfit: the best k of err[q][0..m) by (error, candidate id) in a shared-memory list
+//                             (list_insert of the sweep: the same ties; NaN -- unscored -- entries and ids < 0 never rank)
+__global__ void __launch_bounds__(kThreads) swap_pairs_topk_kernel(const float* __restrict__ err, const int64_t* __restrict__ candidates,
+                                                                   int Q, int m, int k, float* __restrict__ out_score,
+                                                                   int64_t* __restrict__ out_idx) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int64_t* li = reinterpret_cast<int64_t*>(smem_raw) + warp * k;                       // [kWarps][k]
+    float* ls = reinterpret_cast<float*>(reinterpret_cast<int64_t*>(smem_raw) + kWarps * k) + warp * k;
+    const int q = blockIdx.x * kWarps + warp;
+    if (q >= Q) return;
+    for (int e = lane; e < k; e += 32) { ls[e] = INFINITY; li[e] = kEmptyIdx; }
+    __syncwarp();
+    const float* es = err + (int64_t)q * m;
+    const int64_t* ci = candidates + (int64_t)q * m;
+    for (int j0 = 0; j0 < m; j0 += 32) {
+        const int n = m - j0 < 32 ? m - j0 : 32;
+        float s_l = NAN;
+        int64_t i_l = -1;
+        if (lane < n) { s_l = es[j0 + lane]; i_l = ci[j0 + lane]; }
+        for (int j = 0; j < n; ++j) {
+            const float s = __shfl_sync(0xffffffffu, s_l, j);
+            const int64_t i = __shfl_sync(0xffffffffu, i_l, j);
+            if (s == s && i >= 0) list_insert<CODAE_METRIC_SQERR>(ls, li, k, s, i, lane);
+        }
+    }
+    for (int e = lane; e < k; e += 32) {
+        out_score[(int64_t)q * k + e] = ls[e];
+        out_idx[(int64_t)q * k + e] = li[e] == kEmptyIdx ? -1 : li[e];
     }
 }
 
@@ -774,6 +891,68 @@ int codae_swap_error_topk_filtered(codae_ctx* ctx, const float* outfit, const vo
     if (rc) return rc;
     return swap_error_topk(ctx, outfit, catalog, cat_dtype, ld_cat, first_row, B, E, slot, io, inv_scale, y, ld_y, row_offset, k,
                            allow, exclude, n_exclude, out_score, out_idx, workspace, ws_bytes, stream);
+}
+
+// Arguments shared by codae_swap_build_pairs and codae_swap_error_pairs.
+static int check_pairs(codae_ctx* ctx, const char* fn, const float* outfits, int64_t ld_outfit, int Q, const void* catalog,
+                       int cat_dtype, int64_t ld_cat, int64_t n_rows, int64_t row_offset, const int64_t* candidates, int m,
+                       const int64_t* pos, int B, int E, int slot, int io) {
+    CODAE_REQUIRE(ctx, ctx && outfits && catalog && candidates && pos, "%s: NULL argument", fn);
+    CODAE_REQUIRE(ctx, Q >= 1 && m >= 1 && (int64_t)Q * m <= INT32_MAX, "%s: bad list shape Q=%d m=%d", fn, Q, m);
+    CODAE_REQUIRE(ctx, B >= 1 && E >= 1 && slot >= 0 && (int64_t)(slot + 1) * E <= io && ld_outfit >= io && ld_cat >= E &&
+                           n_rows >= 0 && row_offset >= 0,
+                  "%s: bad shape (B=%d E=%d slot=%d io=%d)", fn, B, E, slot, io);
+    CODAE_REQUIRE(ctx, cat_dtype == CODAE_F32 || cat_dtype == CODAE_BF16, "%s: bad cat_dtype %d", fn, cat_dtype);
+    return CODAE_OK;
+}
+
+int codae_swap_build_pairs(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, const void* catalog, int cat_dtype,
+                           int64_t ld_cat, int64_t n_rows, int64_t row_offset, const int64_t* candidates, int m, const int64_t* pos,
+                           int B, int E, int slot, int io, float inv_scale, void* out_x, int x_dtype, int64_t ld_x, void* stream) {
+    int rc = check_pairs(ctx, "codae_swap_build_pairs", outfits, ld_outfit, Q, catalog, cat_dtype, ld_cat, n_rows, row_offset,
+                         candidates, m, pos, B, E, slot, io);
+    if (rc) return rc;
+    CODAE_REQUIRE(ctx, out_x && ld_x >= io && (x_dtype == CODAE_F32 || x_dtype == CODAE_BF16),
+                  "codae_swap_build_pairs: bad output (ld_x=%lld x_dtype=%d)", (long long)ld_x, x_dtype);
+    const bool bc = cat_dtype == CODAE_BF16, bo = x_dtype == CODAE_BF16;
+    const bool v4 = io % 4 == 0 && E % 4 == 0 && ld_outfit % 4 == 0 && (reinterpret_cast<uintptr_t>(outfits) & 15) == 0;
+    const int V = v4 ? 4 : 1;
+    int64_t blocks = ((int64_t)B * (io / V) + 256 * 4 - 1) / (256 * 4);
+    if (blocks > (int64_t)ctx->sm_count * 8) blocks = (int64_t)ctx->sm_count * 8;
+    const int64_t n_pairs = (int64_t)Q * m;
+    cudaStream_t s = as_stream(stream);
+#define LAUNCH(BC, BO, VV) swap_build_pairs_kernel<BC, BO, VV><<<(unsigned)blocks, 256, 0, s>>>(outfits, ld_outfit, n_pairs, catalog, ld_cat, n_rows, row_offset, candidates, m, pos, B, E, slot, io, inv_scale, out_x, ld_x)
+#define LAUNCH_V(BC, BO) do { if (v4) LAUNCH(BC, BO, 4); else LAUNCH(BC, BO, 1); } while (0)
+    if (bc && bo) LAUNCH_V(true, true); else if (bc) LAUNCH_V(true, false); else if (bo) LAUNCH_V(false, true); else LAUNCH_V(false, false);
+#undef LAUNCH_V
+#undef LAUNCH
+    return codae_check_launch(ctx, "swap_build_pairs_kernel");
+}
+
+int codae_swap_error_pairs(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, const void* catalog, int cat_dtype,
+                           int64_t ld_cat, int64_t n_rows, int64_t row_offset, const int64_t* candidates, int m, const int64_t* pos,
+                           int B, int E, int slot, int io, float inv_scale, const float* y, int64_t ld_y, float* err, void* stream) {
+    int rc = check_pairs(ctx, "codae_swap_error_pairs", outfits, ld_outfit, Q, catalog, cat_dtype, ld_cat, n_rows, row_offset,
+                         candidates, m, pos, B, E, slot, io);
+    if (rc) return rc;
+    CODAE_REQUIRE(ctx, y && err && ld_y >= io, "codae_swap_error_pairs: bad output (ld_y=%lld)", (long long)ld_y);
+    const int64_t n_pairs = (int64_t)Q * m;
+    cudaStream_t s = as_stream(stream);
+    if (cat_dtype == CODAE_BF16)
+        swap_error_pairs_kernel<true><<<sweep_grid(ctx, B), kThreads, 0, s>>>(outfits, ld_outfit, n_pairs, catalog, ld_cat, n_rows, row_offset, candidates, m, pos, B, E, slot, io, inv_scale, y, ld_y, err);
+    else
+        swap_error_pairs_kernel<false><<<sweep_grid(ctx, B), kThreads, 0, s>>>(outfits, ld_outfit, n_pairs, catalog, ld_cat, n_rows, row_offset, candidates, m, pos, B, E, slot, io, inv_scale, y, ld_y, err);
+    return codae_check_launch(ctx, "swap_error_pairs_kernel");
+}
+
+int codae_swap_pairs_topk(codae_ctx* ctx, const float* err, const int64_t* candidates, int Q, int m, int k, float* out_score,
+                          int64_t* out_idx, void* stream) {
+    CODAE_REQUIRE(ctx, ctx && err && candidates && out_score && out_idx, "codae_swap_pairs_topk: NULL argument");
+    CODAE_REQUIRE(ctx, Q >= 1 && m >= 1 && (int64_t)Q * m <= INT32_MAX, "codae_swap_pairs_topk: bad list shape Q=%d m=%d", Q, m);
+    CODAE_REQUIRE(ctx, k >= 1 && k <= kMaxK, "codae_swap_pairs_topk: k %d outside [1, %d]", k, kMaxK);
+    const int grid = (Q + kWarps - 1) / kWarps;
+    swap_pairs_topk_kernel<<<grid, kThreads, (size_t)kWarps * k * 12, as_stream(stream)>>>(err, candidates, Q, m, k, out_score, out_idx);
+    return codae_check_launch(ctx, "swap_pairs_topk_kernel");
 }
 
 int codae_score_rank(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,

@@ -8,6 +8,9 @@ top-k.  The catalog is sharded by rows across ranks (torchrun), merged with an a
 --mode swap scores every candidate SWAP by the reconstruction error of the whole swapped outfit instead
 (candidate substituted into the slot, DAE forward per candidate; codae.tool.SwapScorer).
 
+--mode rerank retrieves, then re-ranks: the top --rerank_depth M rows of the slot reading (--metric) for every outfit, then
+those M candidates scored by swap error in one batched pass (SwapScorer.rerank); it prints the final k with their swap errors.
+
 --exclude_own_item leaves out, for query q, catalog row q (the item outfit q already holds in the slot: a trained DAE
 reconstructs it closely, and swapping it in is the identity swap); --allowed_rows PATH.npy restricts the results to the
 global row ids stored there (int64).  Both filter inside the kernels, so k results come back whenever k rows are eligible.
@@ -35,7 +38,8 @@ def parse():
     parser.add_argument('--slot', type=int, default=0)
     parser.add_argument('--k', type=int, default=10)
     parser.add_argument('--metric', type=str, default="sqerr", choices=["sqerr", "cosine"])
-    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap"])
+    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank"])
+    parser.add_argument('--rerank_depth', type=int, default=50, help="rerank mode: stage-1 candidates per outfit (1..128)")
     parser.add_argument('--compute_dtype', '--dtype', dest="compute_dtype", type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
     parser.add_argument('--queries', type=int, default=4)
     parser.add_argument('--synthetic', type=int, default=0)
@@ -58,6 +62,8 @@ def local_allowed(path, lo, n_local, device):
 
 if __name__ == "__main__":
     args = parse()
+    if args.mode == "rerank" and not 1 <= args.rerank_depth <= 128:
+        raise SystemExit("--rerank_depth must lie in [1, 128]")
     rank, world, device = init_distributed()
     with open(args.config, 'r') as stream:
         config = yaml.safe_load(stream)
@@ -91,11 +97,19 @@ if __name__ == "__main__":
             print(json.dumps({"slot": args.slot, "mode": "swap", "metric": "sqerr", "k": args.k,
                               "indices": [i.cpu().tolist() for _, i in res], "scores": [s.cpu().tolist() for s, _ in res]}))
         raise SystemExit(0)
-    scorer = ComplementarityScorer(shard.contiguous(), E, metric=args.metric, k=args.k, inv_scale=1.0 / dataset.scale,
-                                   row_offset=lo, allowed=allowed)
+    rerank = args.mode == "rerank"
+    scorer = ComplementarityScorer(shard.contiguous(), E, metric=args.metric, k=args.rerank_depth if rerank else args.k,
+                                   inv_scale=1.0 / dataset.scale, row_offset=lo, allowed=allowed)
     p = predict_slot(model, outfits, args.slot, E)
     # large query batches: one tensor-core pass over the catalog, results identical to the row sweep
     scores, idx = scorer.topk_batched(p, own) if p.shape[0] >= ComplementarityScorer.TC_MIN_Q else scorer.topk(p, own)
+    if rerank:
+        swap = SwapScorer(model, shard.contiguous(), E, k=args.k, inv_scale=1.0 / dataset.scale, row_offset=lo, allowed=allowed)
+        scores, idx = swap.rerank(outfits.float().contiguous(), args.slot, idx.contiguous())
+        if rank == 0:
+            print(json.dumps({"slot": args.slot, "mode": "rerank", "depth": args.rerank_depth, "k": args.k,
+                              "indices": idx.cpu().tolist(), "scores": scores.cpu().tolist()}))
+        raise SystemExit(0)
     if rank == 0:
         print(json.dumps({"slot": args.slot, "metric": args.metric, "k": args.k,
                           "indices": idx.cpu().tolist(), "scores": scores.cpu().tolist()}))
