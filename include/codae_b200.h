@@ -430,6 +430,27 @@ int codae_swap_error_pairs(codae_ctx* ctx, const float* outfits, int64_t ld_outf
 int codae_swap_pairs_topk(codae_ctx* ctx, const float* err, const int64_t* candidates, int Q, int m, int k, float* out_score,
                           int64_t* out_idx, void* stream);
 
+/* Outfit COMPATIBILITY by leave-one-slot-out reconstruction: how well do the S items of a complete outfit go together, and which
+ * one fits least?  Slot s of the outfit is hidden (multiplied by 0), the DAE reconstructs the outfit, and the distance of the
+ * reconstructed slot s from the item that was there is that slot's error; a compatible outfit has small errors.  The input rows
+ * come from codae_corrupt_fwd: with mask_table int16 [Q, S] (every row 0 .. S-1), mask_bits [S] = 1 << s and col_var [io] = c / E,
+ * launch s (data = the Q outfit rows, batch_idx NULL, run s) writes rows [s Q, (s+1) Q) of the GEMM chain's input -- bit for bit
+ * what predict_slot(model, outfits, s, E) feeds the model (the same multiply: -0.0, NaN and inf propagate alike).
+ *   outfits [Q, ld_outfit] f32   the scaled outfit rows (S E columns used)
+ *   y       [S Q, ld_y] f32      the reconstructions, slot-major: row s Q + i is outfit i with slot s hidden
+ *   err     [Q, S] f32           err[i, s] = sum_{d < E} (y[s Q + i, s E + d] - outfits[i, s E + d])^2 (lane-strided fmaf, warp tree)
+ *   score   [Q] f32              err[i, 0] + err[i, 1] + ... + err[i, S-1], summed in slot order in fp32 (lower: more compatible)
+ *   odd     [Q] int64            argmax_s err[i, s], ties -> the lower slot (the odd item out)
+ * A NaN error makes that outfit's score NaN and its odd -1.  An outfit holding a NaN or inf in its S E columns gets NaN for every
+ * err (score NaN, odd -1): the GEMM chain's ReLU (fmaxf) maps NaN to 0, so its reconstructions may be finite but say nothing.  Q >= 1, 1 <= S <= 64 (the corruption kernel's variable limit),
+ * E % 4 == 0, ld_outfit and ld_y >= S E, buffers naturally aligned; CODAE_EINVAL otherwise.
+ * Numerics: a GEMM row depends only on that row and on the launch's 128-row tile count, so for a fixed chunk layout an outfit's
+ * err / score / odd do not depend on the other outfits of its launch or their order, and repeat bit for bit run to run; err
+ * agrees with an fp64 restatement to the engine's tolerance (1e-5 relative for the fp32-parity and FFMA engines, 1e-2 for bf16);
+ * score and odd follow from the returned err bit for bit. */
+int codae_outfit_loo_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const float* y, int64_t ld_y,
+                           float* err, float* score, int64_t* odd, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

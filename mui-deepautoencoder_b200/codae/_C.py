@@ -86,6 +86,7 @@ SIGNATURES = {
     "codae_swap_error_pairs": (_i, [_vp, _vp, _i64, _i, _vp, _i, _i64, _i64, _i64, _vp, _i, _vp, _i, _i, _i, _i, _f, _vp, _i64, _vp,
                                     _vp]),
     "codae_swap_pairs_topk": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "codae_outfit_loo_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _i64, _vp, _vp, _vp, _vp]),
 }
 
 DP_MAX_WORLD = 8
@@ -597,6 +598,15 @@ def swap_pairs_topk(err, candidates, k, out_score, out_idx):
     c = ctx(err.device)
     Q, m = candidates.shape
     check(lib().codae_swap_pairs_topk(c, p(err), p(candidates), Q, m, k, p(out_score), p(out_idx), stream()), c)
+
+
+def outfit_loo_error(outfits, S, E, y, err, score, odd):
+    """Leave-one-slot-out errors of outfits [Q, >= S E] f32 from the slot-major reconstructions y [S Q, >= S E] f32: err [Q, S] f32
+    (contiguous), score [Q] f32, odd [Q] int64."""
+    _dev_check(outfits, y, err, score, odd)
+    c = ctx(outfits.device)
+    check(lib().codae_outfit_loo_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(y), y.stride(0), p(err), p(score),
+                                       p(odd), stream()), c)
 
 
 def linear_engine(device, dtype, M, N, K):

@@ -13,6 +13,10 @@ filtered-out row is treated as absent from the catalog, inside the kernels (incl
 SwapScorer is the other reading of "scores candidate item swaps by reconstruction error": every candidate is
 substituted into the slot, the whole swapped outfit goes through the DAE (tensor-core GEMMs batched over the
 candidates) and the swap is scored by the reconstruction error of the swapped outfit.
+
+CompatibilityScorer answers the question asked of a complete outfit: how well do its items go together, and which one fits least?
+Each slot is hidden in turn and reconstructed; the per-slot errors, their sum and the slot of largest error come back, and
+compatibility_auc scores real outfits against shuffled ones.
 """
 import torch
 
@@ -192,6 +196,45 @@ def predict_slot(model, outfits, slot, embedding_size):
     return y[:, slot * E:(slot + 1) * E].contiguous()
 
 
+class _DaeChunks:
+    """The DAE's Linear layers over chunks of up to `rows` outfit rows, the forward pass of SwapScorer and CompatibilityScorer:
+    the caller writes a chunk's input rows into acts[0] (or, on the fp32-parity engine, into the fp32 stage and splits it into
+    acts[0]'s three bf16 planes), forward() leaves the reconstructions in acts[-1] (fp32)."""
+
+    def __init__(self, model, rows, io, device):
+        self.model, self.rows, self.io, self.device = model, int(rows), io, device
+        self._acts = None
+
+    def buffers(self):
+        """(engine, activations, fp32 stage or None), allocated once."""
+        if self._acts is None:
+            m, dev = self.model, self.device
+            eng = m.engine_dtype()
+            adt = m.act_dtype(eng)
+            acts = [m.new_activation(self.rows, self.io, adt, dev)]
+            for l, (i, o) in enumerate(m.dims):
+                acts.append(m.new_activation(self.rows, o, torch.float32 if l == len(m.dims) - 1 else adt, dev))
+            # fp32-parity engine: the rows are built in fp32 and split into the engine's three bf16 planes
+            stage = m.new_activation(self.rows, self.io, torch.float32, dev) if eng == _C.F32X3 else None
+            self._acts = (eng, acts, stage)
+        return self._acts
+
+    def prepare(self):
+        """Weights and activation buffers of one scoring call: (engine, activations, fp32 stage or None, GEMM weights)."""
+        m = self.model
+        m.sync_weights()          # a sharded data-parallel trainer gathers the master weights first (collective)
+        eng, acts, stage = self.buffers()
+        m.refresh_shadow()
+        return eng, acts, stage, m.gemm_weights(eng)
+
+    def forward(self, eng, acts, wflat, B):
+        """The DAE's Linear layers on the B rows in acts[0]; the reconstructions land in acts[-1]."""
+        m = self.model
+        for l, (i, o) in enumerate(m.dims):
+            _C.linear_fwd(acts[l], m.aug_view(wflat, l), None, acts[l + 1], B, o, (i + 7) // 8 * 8 + 1,
+                          _C.ACT_RELU if m.relu[l] else _C.ACT_NONE, eng)
+
+
 class SwapScorer:
     """Scores the swap "candidate j into slot c" by || DAE(outfit_j) - outfit_j ||^2 over all io dimensions (lower
     is better) and returns the best k swaps.  Candidates are processed in chunks of `chunk` rows: codae_swap_build
@@ -212,35 +255,11 @@ class SwapScorer:
         dev = catalog.device
         self.allowed = _allowed_mask(allowed, catalog.shape[0], dev)
         self._ws = _C.score_topk_workspace(dev, 1, k)
-        self._acts = None
+        self._dae = _DaeChunks(model, self.chunk, self.io, dev)
 
     def _buffers(self):
-        if self._acts is None:
-            m, dev = self.model, self.catalog.device
-            eng = m.engine_dtype()
-            adt = m.act_dtype(eng)
-            acts = [m.new_activation(self.chunk, self.io, adt, dev)]
-            for l, (i, o) in enumerate(m.dims):
-                acts.append(m.new_activation(self.chunk, o, torch.float32 if l == len(m.dims) - 1 else adt, dev))
-            # fp32-parity engine: the swap rows are built in fp32 and split into the engine's three bf16 planes
-            stage = m.new_activation(self.chunk, self.io, torch.float32, dev) if eng == _C.F32X3 else None
-            self._acts = (eng, acts, stage)
-        return self._acts
-
-    def _prepare(self):
-        """Weights and activation buffers of one scoring call: (engine, activations, fp32 stage or None, GEMM weights)."""
-        m = self.model
-        m.sync_weights()          # a sharded data-parallel trainer gathers the master weights first (collective)
-        eng, acts, stage = self._buffers()
-        m.refresh_shadow()
-        return eng, acts, stage, m.gemm_weights(eng)
-
-    def _forward(self, eng, acts, wflat, B):
-        """The DAE's Linear layers on the B swapped outfits in acts[0]; the reconstructions land in acts[-1]."""
-        m = self.model
-        for l, (i, o) in enumerate(m.dims):
-            _C.linear_fwd(acts[l], m.aug_view(wflat, l), None, acts[l + 1], B, o, (i + 7) // 8 * 8 + 1,
-                          _C.ACT_RELU if m.relu[l] else _C.ACT_NONE, eng)
+        """(engine, activations, fp32 stage or None) of the swapped-outfit chunks."""
+        return self._dae.buffers()
 
     def topk_local(self, outfit, slot, exclude=None):
         """outfit: [io] scaled fp32 row.  Returns (errors [k], global candidate indices [k]) of this shard.  exclude: int64
@@ -250,7 +269,7 @@ class SwapScorer:
             raise Exception("Slot out of range.")
         ex = _exclusions(exclude, None, dev)
         outfit = outfit.to(torch.float32).contiguous().view(-1)
-        eng, acts, stage, wflat = self._prepare()
+        eng, acts, stage, wflat = self._dae.prepare()
         n = self.catalog.shape[0]
         n_chunks = max(1, (n + self.chunk - 1) // self.chunk)
         ls = torch.full((n_chunks, 1, self.k), float("inf"), dtype=torch.float32, device=dev)
@@ -263,7 +282,7 @@ class SwapScorer:
             else:
                 _C.swap_build(outfit, self.catalog, first, B, self.E, slot, self.io, self.inv_scale, stage)
                 _C.split_x3(stage, acts[0])
-            self._forward(eng, acts, wflat, B)
+            self._dae.forward(eng, acts, wflat, B)
             _C.swap_error_topk(outfit, self.catalog, first, B, self.E, slot, self.io, self.inv_scale, acts[-1],
                                self.row_offset, self.k, ls[c, 0], li[c, 0], self._ws, allow=self.allowed, exclude=ex)
         out_s = torch.empty((1, self.k), dtype=torch.float32, device=dev)
@@ -302,14 +321,14 @@ class SwapScorer:
         Q, mm = cand.shape
         pos = self._owned_positions(cand)
         err = torch.full((Q * mm,), float("nan"), dtype=torch.float32, device=dev)
-        eng, acts, stage, wflat = self._prepare()      # on every rank, pairs or not: sync_weights may be a collective
+        eng, acts, stage, wflat = self._dae.prepare()      # on every rank, pairs or not: sync_weights may be a collective
         for c0 in range(0, pos.numel(), self.chunk):
             pc = pos[c0:c0 + self.chunk]
             _C.swap_build_pairs(outfits, self.catalog, self.row_offset, cand, pc, self.E, slot, self.io, self.inv_scale,
                                 acts[0] if stage is None else stage)
             if stage is not None:
                 _C.split_x3(stage, acts[0])
-            self._forward(eng, acts, wflat, pc.numel())
+            self._dae.forward(eng, acts, wflat, pc.numel())
             _C.swap_error_pairs(outfits, self.catalog, self.row_offset, cand, pc, self.E, slot, self.io, self.inv_scale, acts[-1],
                                 err)
         out_s = torch.empty((Q, self.k), dtype=torch.float32, device=dev)
@@ -321,3 +340,117 @@ class SwapScorer:
         """Global rerank_local: every rank scores the listed rows it holds, then all-gather of k entries per outfit and the
         deterministic merge (codae_topk_merge)."""
         return _gather_merge(self.pg, *self.rerank_local(outfits, slot, candidates), _C.METRIC_SQERR)
+
+
+def _outfit_rows(outfits, io, device):
+    """CompatibilityScorer's input: outfits fp32 [Q, io], Q >= 1, on the model's device; a contiguous copy."""
+    if not isinstance(outfits, torch.Tensor) or outfits.dtype != torch.float32:
+        raise RuntimeError("codae: outfits must be a float32 tensor")
+    if outfits.dim() != 2 or outfits.shape[1] != io or outfits.shape[0] < 1:
+        raise RuntimeError("codae: outfits must have shape [Q, %d] with Q >= 1, got %s" % (io, tuple(outfits.shape)))
+    if not outfits.is_cuda or outfits.device != device:
+        raise RuntimeError("codae: outfits must be on the model's device %s" % device)
+    return outfits.contiguous()
+
+
+class CompatibilityScorer:
+    """Outfit compatibility by leave-one-slot-out reconstruction: for every slot s of a complete outfit, slot s is hidden
+    (multiplied by 0, as model.corrupt does), the DAE reconstructs the outfit and the squared distance of the reconstructed slot s
+    from the item that was there is slot_err[s].  A compatible outfit has small errors (score = their sum); the slot of the largest
+    error holds the odd item out.  Every (outfit, slot) row is an independent DAE forward: a chunk of chunk // S whole outfits is
+    S codae_corrupt_fwd launches into the first activation buffer (rows slot-major), the model's Linear layers, then
+    codae_outfit_loo_error (include/codae_b200.h)."""
+
+    def __init__(self, model, embedding_size, chunk=8192, process_group=None):
+        model._require_cuda()
+        self.model, self.E, self.pg = model, int(embedding_size), process_group
+        self.io = model.dims[0][0]
+        if self.io % self.E != 0:
+            raise Exception("Embedding size does not divide the model input.")
+        self.S = self.io // self.E
+        if chunk < self.S:
+            raise Exception("chunk %d holds no whole outfit of %d slots." % (chunk, self.S))
+        self.chunk_outfits = int(chunk) // self.S
+        dev = self.device = model.flat.device
+        S = self.S
+        # codae_corrupt_fwd's tables: observation i gets mask s in run s, mask s zeroes variable s, column c is variable c / E
+        self._mask_table = torch.arange(S, dtype=torch.int16, device=dev).repeat(self.chunk_outfits, 1)
+        self._mask_bits = torch.bitwise_left_shift(torch.ones(S, dtype=torch.int64, device=dev), torch.arange(S, device=dev))
+        self._col_var = torch.div(torch.arange(self.io, device=dev), self.E, rounding_mode="floor").to(torch.uint8)
+        self._dae = _DaeChunks(model, self.chunk_outfits * S, self.io, dev)
+        self._out = None
+
+    def _outputs(self, Q):
+        if self._out is None or self._out[0].shape[0] != Q:
+            dev = self.device
+            self._out = (torch.empty((Q, self.S), dtype=torch.float32, device=dev), torch.empty(Q, dtype=torch.float32, device=dev),
+                         torch.empty(Q, dtype=torch.int64, device=dev))
+        return self._out
+
+    def score_local(self, outfits):
+        """outfits: [Q, io] scaled fp32 rows on the model's device.  Returns (slot_err [Q, S] f32, score [Q] f32, odd [Q] int64):
+        lower score = more compatible; odd = the slot of largest error (ties -> lower slot); an outfit with a NaN error gets a NaN
+        score and odd -1.  Asynchronous (no host synchronisation); the returned tensors are reused by the next call."""
+        x = _outfit_rows(outfits, self.io, self.device)
+        Q, S = x.shape[0], self.S
+        err, score, odd = self._outputs(Q)
+        eng, acts, stage, wflat = self._dae.prepare()
+        for c0 in range(0, Q, self.chunk_outfits):
+            Bq = min(self.chunk_outfits, Q - c0)
+            rows = x[c0:c0 + Bq]
+            dst = acts[0] if stage is None else stage
+            for s in range(S):
+                _C.corrupt_fwd(rows, None, Bq, self._mask_table, s, self._mask_bits, self._col_var, self.io, dst[s * Bq:(s + 1) * Bq])
+            if stage is not None:
+                _C.split_x3(stage, acts[0])
+            self._dae.forward(eng, acts, wflat, S * Bq)
+            _C.outfit_loo_error(rows, S, self.E, acts[-1], err[c0:c0 + Bq], score[c0:c0 + Bq], odd[c0:c0 + Bq])
+        return err, score, odd
+
+    def score(self, outfits):
+        """score_local over the ranks of the process group: every rank is given the same outfits, rank r scores its
+        shard_rows(Q, G, r) slice, and the slices are all-gathered (padded to ceil(Q / G) rows) into the full results."""
+        import torch.distributed as dist
+        pg = self.pg
+        if pg is None and not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
+            return self.score_local(outfits)
+        x = _outfit_rows(outfits, self.io, self.device)
+        Q, S, dev = x.shape[0], self.S, self.device
+        G, r = dist.get_world_size(pg), dist.get_rank(pg)
+        lo, n = shard_rows(Q, G, r)
+        per = (Q + G - 1) // G
+        err = torch.full((per, S), float("nan"), dtype=torch.float32, device=dev)
+        score = torch.full((per,), float("nan"), dtype=torch.float32, device=dev)
+        odd = torch.full((per,), -1, dtype=torch.int64, device=dev)
+        if n:
+            e, s, o = self.score_local(x[lo:lo + n])
+            err[:n], score[:n], odd[:n] = e, s, o
+        else:
+            self.model.sync_weights()      # a collective under a sharded data-parallel trainer: every rank takes part
+        out = []
+        for t in (err, score, odd):
+            g = torch.empty((G * per,) + tuple(t.shape[1:]), dtype=t.dtype, device=dev)
+            dist.all_gather_into_tensor(g, t, group=pg)
+            out.append(g[:Q])
+        return tuple(out)
+
+
+def compatibility_auc(pos_score, neg_score):
+    """Outfit compatibility AUC: the probability that a real outfit (pos_score) scores lower -- more compatible -- than a negative
+    one (neg_score), ties counting 1/2; the rank-sum (Mann-Whitney) form with average ranks for ties.  NaN scores are dropped.
+    Returns a Python float (NaN when either side is empty after dropping)."""
+    pos = pos_score.reshape(-1).double()
+    neg = neg_score.reshape(-1).double()
+    pos, neg = pos[~torch.isnan(pos)], neg[~torch.isnan(neg)]
+    n_p, n_n = pos.numel(), neg.numel()
+    if n_p == 0 or n_n == 0:
+        return float("nan")
+    # rank of every value among both sets by DESCENDING score (1 = highest), ties averaged: a real outfit below a negative one
+    # gets the larger rank; U = sum of the real outfits' ranks - n_p (n_p + 1) / 2 counts the pairs (real < negative) + ties / 2
+    allv = torch.cat([pos, neg])
+    vals, inv, counts = torch.unique(-allv, sorted=True, return_inverse=True, return_counts=True)
+    last = torch.cumsum(counts, 0).double()
+    avg = last - (counts.double() - 1) / 2
+    rank_pos = avg[inv[:n_p]].sum()
+    u = rank_pos - n_p * (n_p + 1) / 2
+    return float(u / (n_p * n_n))

@@ -709,6 +709,49 @@ __global__ void __launch_bounds__(kThreads) swap_pairs_topk_kernel(const float* 
     }
 }
 
+// ---- outfit compatibility: leave-one-slot-out reconstruction errors ------------------------------------------------------
+// The reconstructions y come slot-major: row s * Q + i is outfit i with slot s multiplied by 0 (codae_corrupt_fwd, run s).
+//   outfit_loo_error_kernel  one warp per outfit: err[i, s] = sum_{d < E} (y[s Q + i, s E + d] - outfits[i, s E + d])^2 (lane-strided
+//                            fmaf, then the warp_sum tree), score[i] = err[i, 0] + err[i, 1] + ... in slot order, odd[i] = the first
+//                            slot of largest error; a NaN error makes score NaN and odd -1.  An outfit holding a NaN or inf gets NaN
+//                            errors throughout: the GEMM epilogue's ReLU (fmaxf) turns NaN into 0, so its reconstructions can be finite
+//                            and meaningless.
+__global__ void __launch_bounds__(kThreads) outfit_loo_error_kernel(const float* __restrict__ outfits, int64_t ld_outfit, int Q, int S,
+                                                                    int E, const float* __restrict__ y, int64_t ld_y,
+                                                                    float* __restrict__ err, float* __restrict__ score,
+                                                                    int64_t* __restrict__ odd) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int i = blockIdx.x * kWarps + warp; i < Q; i += gridDim.x * kWarps) {
+        const float* x = outfits + (int64_t)i * ld_outfit;
+        float sum = 0.f, best = -INFINITY;
+        int arg = 0;
+        bool nan = false, nonfinite = false;
+        for (int s = 0; s < S; ++s) {
+            const float* yr = y + ((int64_t)s * Q + i) * ld_y + (int64_t)s * E;
+            const float* xr = x + (int64_t)s * E;
+            float acc = 0.f;
+            for (int d = lane; d < E; d += 32) {
+                const float xv = xr[d];
+                nonfinite |= !isfinite(xv);
+                const float df = yr[d] - xv;
+                acc = fmaf(df, df, acc);
+            }
+            acc = warp_sum(acc);
+            if (lane == 0) err[(int64_t)i * S + s] = acc;
+            sum += acc;
+            if (acc != acc) nan = true;
+            else if (acc > best) { best = acc; arg = s; }
+        }
+        nonfinite = __any_sync(0xffffffffu, nonfinite);
+        if (lane == 0) {
+            if (nonfinite)
+                for (int s = 0; s < S; ++s) err[(int64_t)i * S + s] = NAN;
+            score[i] = nan || nonfinite ? NAN : sum;
+            odd[i] = nan || nonfinite ? -1 : arg;
+        }
+    }
+}
+
 inline int sweep_grid(const codae_ctx* ctx, int64_t n_rows) {
     int64_t g = (n_rows + kWarps - 1) / kWarps;
     const int64_t cap = (int64_t)ctx->sm_count * 4;
@@ -953,6 +996,22 @@ int codae_swap_pairs_topk(codae_ctx* ctx, const float* err, const int64_t* candi
     const int grid = (Q + kWarps - 1) / kWarps;
     swap_pairs_topk_kernel<<<grid, kThreads, (size_t)kWarps * k * 12, as_stream(stream)>>>(err, candidates, Q, m, k, out_score, out_idx);
     return codae_check_launch(ctx, "swap_pairs_topk_kernel");
+}
+
+int codae_outfit_loo_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const float* y, int64_t ld_y,
+                           float* err, float* score, int64_t* odd, void* stream) {
+    CODAE_REQUIRE(ctx, ctx && outfits && y && err && score && odd, "codae_outfit_loo_error: NULL argument");
+    CODAE_REQUIRE(ctx, Q >= 1 && S >= 1 && S <= 64 && E >= 4 && E % 4 == 0,
+                  "codae_outfit_loo_error: bad shape Q=%d S=%d E=%d (Q >= 1, 1 <= S <= 64, E a positive multiple of 4)", Q, S, E);
+    CODAE_REQUIRE(ctx, ld_outfit >= (int64_t)S * E && ld_y >= (int64_t)S * E,
+                  "codae_outfit_loo_error: pitches ld_outfit=%lld ld_y=%lld shorter than S E = %lld", (long long)ld_outfit,
+                  (long long)ld_y, (long long)S * E);
+    const auto al = [](const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; };
+    CODAE_REQUIRE(ctx, al(outfits, 4) && al(y, 4) && al(err, 4) && al(score, 4) && al(odd, 8),
+                  "codae_outfit_loo_error: misaligned buffer");
+    outfit_loo_error_kernel<<<sweep_grid(ctx, Q), kThreads, 0, as_stream(stream)>>>(outfits, ld_outfit, Q, S, E, y, ld_y, err, score,
+                                                                                     odd);
+    return codae_check_launch(ctx, "outfit_loo_error_kernel");
 }
 
 int codae_score_rank(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,

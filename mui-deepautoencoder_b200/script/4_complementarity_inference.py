@@ -14,6 +14,11 @@ those M candidates scored by swap error in one batched pass (SwapScorer.rerank);
 --exclude_own_item leaves out, for query q, catalog row q (the item outfit q already holds in the slot: a trained DAE
 reconstructs it closely, and swapping it in is the identity swap); --allowed_rows PATH.npy restricts the results to the
 global row ids stored there (int64).  Both filter inside the kernels, so k results come back whenever k rows are eligible.
+
+--mode compat scores how well the items of the first --queries outfits go together (codae.tool.CompatibilityScorer): every slot
+is hidden in turn and reconstructed; it prints each outfit's per-slot errors, their sum (lower: more compatible) and the slot of
+largest error (the odd item out).  No catalog is built.  --compat_negatives also scores one shuffled outfit per query -- slot s
+taken from a seeded permutation of all observations -- and adds the compatibility AUC of the real outfits against them.
 """
 import argparse
 import json
@@ -27,7 +32,8 @@ from _common import init_distributed, synthetic_categories
 from codae.dataset import ConcatenatedEmbeddingDataset
 from codae.model import EmbeddingDenoisingAutoencoder
 from codae.tool import load_dataset_of_embeddings
-from codae.tool.inference import ComplementarityScorer, SwapScorer, predict_slot, shard_rows
+from codae.tool.inference import (CompatibilityScorer, ComplementarityScorer, SwapScorer, compatibility_auc, predict_slot,
+                                  shard_rows)
 
 
 def parse():
@@ -38,13 +44,15 @@ def parse():
     parser.add_argument('--slot', type=int, default=0)
     parser.add_argument('--k', type=int, default=10)
     parser.add_argument('--metric', type=str, default="sqerr", choices=["sqerr", "cosine"])
-    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank"])
+    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank", "compat"])
     parser.add_argument('--rerank_depth', type=int, default=50, help="rerank mode: stage-1 candidates per outfit (1..128)")
     parser.add_argument('--compute_dtype', '--dtype', dest="compute_dtype", type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
     parser.add_argument('--queries', type=int, default=4)
     parser.add_argument('--synthetic', type=int, default=0)
     parser.add_argument('--catalog_dtype', type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
     parser.add_argument('--exclude_own_item', action='store_true', help="query q never gets catalog row q back")
+    parser.add_argument('--compat_negatives', action='store_true',
+                        help="compat mode: also score one shuffled outfit per query and report the AUC")
     parser.add_argument('--allowed_rows', type=str, default=None, help=".npy of int64 global row ids that may be returned")
     return parser.parse_args()
 
@@ -81,6 +89,24 @@ if __name__ == "__main__":
     if args.model_path:
         model.load_state_dict(torch.load(args.model_path, map_location="cpu"))
     model.to(device).set_compute_dtype(args.compute_dtype)
+    if args.mode == "compat":
+        compat = CompatibilityScorer(model, E)
+        outfits = dataset.data[:args.queries].float().to(device).contiguous()
+        err, score, odd = (t.clone() for t in compat.score(outfits))
+        res = {"mode": "compat", "slots": compat.S, "score": score.cpu().tolist(), "slot_errors": err.cpu().tolist(),
+               "odd_slot": odd.cpu().tolist()}
+        if args.compat_negatives:
+            # one negative per query: slot s of negative q is slot s of observation perm_s[q] (a seeded permutation per slot)
+            g = torch.Generator().manual_seed(config["SEED"])
+            neg = torch.empty_like(outfits)
+            for s in range(compat.S):
+                perm = torch.randperm(dataset.nb_observation, generator=g)[:outfits.shape[0]]
+                neg[:, s * E:(s + 1) * E] = dataset.data[perm, s * E:(s + 1) * E].to(device)
+            _, neg_score, _ = compat.score(neg)
+            res["auc"] = compatibility_auc(score, neg_score)
+        if rank == 0:
+            print(json.dumps(res))
+        raise SystemExit(0)
     lo, n_local = shard_rows(dataset.nb_observation, world, rank)
     shard = dataset.data_per_category[args.slot][lo:lo + n_local].to(device)
     if args.catalog_dtype == "bf16":
