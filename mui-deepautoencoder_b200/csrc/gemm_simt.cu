@@ -5,6 +5,9 @@
 //   fwd   : A = X  (k contiguous)   B(k,n) = W[n,k]  (k contiguous)   epilogue bias + ReLU
 //   dgrad : A = dY (k contiguous)   B(k,n) = W[k,n]  (n contiguous)   epilogue ReLU mask of the layer input
 //   wgrad : A(m,k) = dY[k,m] (m contiguous)   B(k,n) = X[k,n] (n contiguous)
+#include <stdio.h>
+#include <stdlib.h>
+
 #include "common.cuh"
 #include "gemm.h"
 
@@ -204,7 +207,9 @@ template <bool A_KC, bool B_KC, int EPI>
 int launch(codae_ctx* ctx, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int M, int N,
            int K, const float* bias, int act, const float* mask_src, int64_t ldm, cudaStream_t s) {
     const long ctas64 = (long)((M + 63) / 64) * ((N + 63) / 64);
+    static const bool debug_plan = getenv("CODAE_DEBUG_PLAN") != nullptr;
     if (ctas64 >= 2L * ctx->sm_count) {
+        if (debug_plan) fprintf(stderr, "codae plan: simt M=%d N=%d K=%d EPI=%d tile 64 split 1\n", M, N, K, EPI);
         dim3 grid((N + 63) / 64, (M + 63) / 64);
         simt_gemm_kernel<64, 64, 16, A_KC, B_KC, EPI><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, bias, act, mask_src, ldm);
     } else if (ctx->splitk && K >= 256 && M * (long)N >= 64 * 64) {
@@ -213,6 +218,7 @@ int launch(codae_ctx* ctx, const float* A, int64_t lda, const float* B, int64_t 
         if (nsplit > 8) nsplit = 8;
         if (nsplit > K / 128) nsplit = K / 128;
         if (nsplit < 1) nsplit = 1;
+        if (debug_plan) fprintf(stderr, "codae plan: simt M=%d N=%d K=%d EPI=%d tile 64 split %d\n", M, N, K, EPI, nsplit);
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((N + 63) / 64, (M + 63) / 64, nsplit);
         cfg.blockDim = dim3(256);
@@ -231,6 +237,7 @@ int launch(codae_ctx* ctx, const float* A, int64_t lda, const float* B, int64_t 
             return codae_fail(ctx, CODAE_ECUDA, "simt_gemm_splitk_kernel launch (split %d): %s", nsplit, cudaGetErrorString(le));
         }
     } else {
+        if (debug_plan) fprintf(stderr, "codae plan: simt M=%d N=%d K=%d EPI=%d tile 32 split 1\n", M, N, K, EPI);
         dim3 grid((N + 31) / 32, (M + 31) / 32);
         simt_gemm_kernel<32, 32, 32, A_KC, B_KC, EPI><<<grid, 64, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, bias, act, mask_src, ldm);
     }
