@@ -451,6 +451,34 @@ int codae_swap_pairs_topk(codae_ctx* ctx, const float* err, const int64_t* candi
 int codae_outfit_loo_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const float* y, int64_t ld_y,
                            float* err, float* score, int64_t* odd, void* stream);
 
+/* Outfit COMPLETION: every empty slot of a partial outfit filled together, each combination of candidates scored by the swap error
+ * of the completed outfit.  Outfit q misses the slots s with slot_base[q, s] >= 0 (m_q of them, counted in ascending slot order);
+ * combination c in [0, depth^m_q) takes candidate b_j = (c / depth^j) % depth for its j-th missing slot, which is pool row
+ * slot_base[q, s] + b_j.  m_q = 0 has one combination, the outfit as given.
+ *   outfits   [Q, ld_outfit] f32   scaled outfit rows (io = S E columns used; the missing slots' columns are not read)
+ *   slot_base int64 [Q, S]         pool row of candidate 0 of each missing slot, < 0 for a given slot
+ *   pool      [n_pool, ld_pool] f32  candidate rows, un-scaled (E columns used); a bf16 catalog row converts to it exactly
+ *   pool_id   int64 [n_pool]       the global catalog id of each pool row, < 0 for padding
+ *   pos       int64 [B]            built row b holds combination p = pos[b] of the flattened [Q, C] grid: q = p / C, c = p % C
+ * Combination p is valid when 0 <= p < Q C, c < depth^m_q and every pool row it takes lies in [0, n_pool) with pool_id >= 0.  An
+ * invalid row is never dereferenced beyond slot_base: it is built as zeros and gets no error (pos, slot_base and pool_id are device
+ * data).
+ *   codae_complete_build  x'[b, :] = outfit q with each missing slot replaced by its pool row * inv_scale, f32|bf16 at pitch ld_x
+ *                         (columns >= io untouched): for one missing slot, codae_swap_build_pairs' values for that outfit and row.
+ *   codae_complete_error  err[p] = sum_d (y[b, d] - x'_d)^2 over io, x' recomputed in fp32 (lane-strided fmaf, then the warp tree:
+ *                         codae_swap_error_pairs' loop), so one missing slot gives a re-rank's error bit for bit.  err [Q C] is set to
+ *                         NaN by the caller; combinations not built stay NaN.
+ * Ranking is codae_swap_pairs_topk(err, combo [Q, C], ...) with combo[q, c] = c for valid combinations and -1 otherwise.
+ * 1 <= S <= 64, E >= 1, 1 <= depth <= 128, 1 <= C <= CODAE_COMPLETE_MAX_COMBOS, Q C <= INT32_MAX, n_pool >= 1, pitches >= their
+ * row widths, buffers naturally aligned; CODAE_EINVAL otherwise. */
+#define CODAE_COMPLETE_MAX_COMBOS 4096
+int codae_complete_build(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                         const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, int C,
+                         const int64_t* pos, int B, float inv_scale, void* out_x, int x_dtype, int64_t ld_x, void* stream);
+int codae_complete_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                         const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, int C,
+                         const int64_t* pos, int B, float inv_scale, const float* y, int64_t ld_y, float* err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

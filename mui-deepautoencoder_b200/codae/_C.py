@@ -87,6 +87,8 @@ SIGNATURES = {
                                     _vp]),
     "codae_swap_pairs_topk": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "codae_outfit_loo_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "codae_complete_build": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _i, _vp, _i, _f, _vp, _i, _i64, _vp]),
+    "codae_complete_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _i, _vp, _i, _f, _vp, _i64, _vp, _vp]),
 }
 
 DP_MAX_WORLD = 8
@@ -607,6 +609,28 @@ def outfit_loo_error(outfits, S, E, y, err, score, odd):
     c = ctx(outfits.device)
     check(lib().codae_outfit_loo_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(y), y.stride(0), p(err), p(score),
                                        p(odd), stream()), c)
+
+
+COMPLETE_MAX_COMBOS = 4096    # include/codae_b200.h: CODAE_COMPLETE_MAX_COMBOS
+
+
+def complete_build(outfits, S, E, slot_base, pool, pool_id, depth, C, pos, inv_scale, out_x):
+    """Rows of out_x: the combinations pos [B] (int64 positions in the [Q, C] grid) of outfits [Q, S E] f32 built with each missing
+    slot (slot_base [Q, S] int64 >= 0) replaced by its pool row (pool [R, E] f32, pool_id [R] int64) * inv_scale."""
+    _dev_check(outfits, slot_base, pool, pool_id, pos, out_x)
+    c = ctx(outfits.device)
+    check(lib().codae_complete_build(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool), pool.stride(0),
+                                     pool.shape[0], p(pool_id), depth, C, p(pos), pos.numel(), inv_scale, p(out_x), dt(out_x),
+                                     out_x.stride(0), stream()), c)
+
+
+def complete_error(outfits, S, E, slot_base, pool, pool_id, depth, C, pos, inv_scale, y, err):
+    """err [Q C] f32: err[pos[b]] = swap error of reconstruction row b of y for that combination."""
+    _dev_check(outfits, slot_base, pool, pool_id, pos, y, err)
+    c = ctx(outfits.device)
+    check(lib().codae_complete_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool), pool.stride(0),
+                                     pool.shape[0], p(pool_id), depth, C, p(pos), pos.numel(), inv_scale, p(y), y.stride(0), p(err),
+                                     stream()), c)
 
 
 def linear_engine(device, dtype, M, N, K):

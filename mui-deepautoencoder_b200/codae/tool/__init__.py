@@ -10,5 +10,5 @@ from .dictionnary import Dict
 from .parser import parse
 # additions
 from .fused_step import FusedStep
-from .inference import CompatibilityScorer, ComplementarityScorer, SwapScorer, compatibility_auc
+from .inference import CompatibilityScorer, ComplementarityScorer, OutfitCompleter, SwapScorer, compatibility_auc
 from .embedding_file import convert_json_to_cemb, load_cemb_dataset, read_cemb, write_cemb

@@ -17,6 +17,9 @@ candidates) and the swap is scored by the reconstruction error of the swapped ou
 CompatibilityScorer answers the question asked of a complete outfit: how well do its items go together, and which one fits least?
 Each slot is hidden in turn and reconstructed; the per-slot errors, their sum and the slot of largest error come back, and
 compatibility_auc scores real outfits against shuffled ones.
+
+OutfitCompleter fills every empty slot of a partial outfit together ("I have a top, complete the outfit"): candidates per missing
+slot from the slot readings, then every combination of them scored by the swap error of the completed outfit.
 """
 import torch
 
@@ -186,14 +189,20 @@ class ComplementarityScorer:
         return _gather_merge(self.pg, *self.topk_local(query, exclude), self.metric)
 
 
+def predict_missing(model, outfits, missing, embedding_size):
+    """Zero every missing slot (missing: bool [Q, S]) of the (scaled) outfit rows [Q, S E] through model.corrupt, run the DAE once,
+    return the reconstructions [Q, S E]."""
+    mask = (~missing).to(torch.float32).repeat_interleave(embedding_size, dim=1)
+    with torch.no_grad():
+        return model(model.corrupt(input_data=outfits, mask=mask))
+
+
 def predict_slot(model, outfits, slot, embedding_size):
     """Zero slot `slot` of the (scaled) outfit rows, run the DAE, return the reconstructed slot [Q, E]."""
     E = embedding_size
-    mask = torch.ones_like(outfits)
-    mask[:, slot * E:(slot + 1) * E] = 0
-    with torch.no_grad():
-        y = model(model.corrupt(input_data=outfits, mask=mask))
-    return y[:, slot * E:(slot + 1) * E].contiguous()
+    missing = torch.zeros((outfits.shape[0], outfits.shape[1] // E), dtype=torch.bool, device=outfits.device)
+    missing[:, slot] = True
+    return predict_missing(model, outfits, missing, E)[:, slot * E:(slot + 1) * E].contiguous()
 
 
 class _DaeChunks:
@@ -454,3 +463,247 @@ def compatibility_auc(pos_score, neg_score):
     rank_pos = avg[inv[:n_p]].sum()
     u = rank_pos - n_p * (n_p + 1) / 2
     return float(u / (n_p * n_n))
+
+
+def _is_distributed(pg):
+    import torch.distributed as dist
+    return pg is not None or (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1)
+
+
+def _exchange_pool(pool, pool_id, pg):
+    """Every rank's pool rows summed into every rank with one all_reduce(SUM) over int32 views.  Each row has exactly one owner and
+    every other rank holds zeros there, so the sum is the owner's bits (-0.0, NaN and inf included).  pool_id travels as id + 1, so
+    a row no rank owns comes back as -1."""
+    import torch.distributed as dist
+    R = pool_id.numel()
+    buf = torch.cat([torch.where(pool_id >= 0, pool_id + 1, 0).view(torch.int32), pool.reshape(-1).view(torch.int32)])
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=pg)
+    return buf[2 * R:].view(torch.float32).view(pool.shape), buf[:2 * R].view(torch.int64) - 1
+
+
+class OutfitCompleter:
+    """Outfit completion: every empty slot of a partial outfit filled together.  Stage 1 takes, for each missing slot, the best
+    `depth` catalog rows by `metric` against the DAE's reading of that slot with all missing slots hidden (predict_missing, then
+    ComplementarityScorer per slot).  Stage 2 scores every combination of those candidates -- depth^m_q of them for an outfit
+    missing m_q slots -- by the swap error of the completed outfit, || DAE(x') - x' ||^2 over all io columns, and keeps the best k.
+    The combinations of all outfits go through the model's GEMM chain in chunks of `chunk` rows (codae_complete_build, the Linear
+    layers, codae_complete_error) and are ranked by codae_swap_pairs_topk; with one missing slot this is SwapScorer.rerank's
+    arithmetic, bit for bit (include/codae_b200.h: outfit completion)."""
+
+    MAX_DEPTH = 128
+
+    def __init__(self, model, catalogs, embedding_size, depth=8, k=10, metric="sqerr", inv_scale=1.0, row_offsets=None,
+                 chunk=8192, process_group=None):
+        """catalogs: S entries, entry s this rank's shard of slot s's catalog ([n_local, >= E] fp32 or bf16 CUDA tensor, rows
+        row_offsets[s].. of the global catalog) or None when slot s cannot be completed.  inv_scale multiplies catalog values
+        (1 / dataset.scale for un-scaled catalogs such as dataset.data_per_category).  Shards of one slot must not overlap."""
+        model._require_cuda()
+        if metric not in METRICS:
+            raise Exception("Unknown metric.")
+        self.model, self.E, self.pg = model, int(embedding_size), process_group
+        self.io = model.dims[0][0]
+        if self.io % self.E != 0:
+            raise Exception("Embedding size does not divide the model input.")
+        self.S = S = self.io // self.E
+        if not 1 <= depth <= self.MAX_DEPTH:
+            raise RuntimeError("codae: depth %d outside [1, %d]" % (depth, self.MAX_DEPTH))
+        if not 1 <= k <= 128:
+            raise RuntimeError("codae: k %d outside [1, 128]" % k)
+        if chunk < 1:
+            raise RuntimeError("codae: chunk %d < 1" % chunk)
+        if len(catalogs) != S:
+            raise RuntimeError("codae: %d catalogs for %d slots" % (len(catalogs), S))
+        row_offsets = [0] * S if row_offsets is None else [int(o) for o in row_offsets]
+        if len(row_offsets) != S:
+            raise RuntimeError("codae: %d row offsets for %d slots" % (len(row_offsets), S))
+        self.device = dev = model.flat.device
+        for s, cat in enumerate(catalogs):
+            if cat is None:
+                continue
+            if not isinstance(cat, torch.Tensor) or cat.dtype not in (torch.float32, torch.bfloat16):
+                raise RuntimeError("codae: catalog %d must be a float32 or bfloat16 tensor" % s)
+            if cat.dim() != 2 or cat.shape[1] < self.E:
+                raise RuntimeError("codae: catalog %d must have shape [n, >= %d], got %s" % (s, self.E, tuple(cat.shape)))
+            if not cat.is_cuda or cat.device != dev:
+                raise RuntimeError("codae: catalog %d must be on the model's device %s" % (s, dev))
+        self.catalogs, self.row_offsets = list(catalogs), row_offsets
+        self.depth, self.k, self.inv_scale, self.chunk = int(depth), int(k), float(inv_scale), int(chunk)
+        self._scorers = [None if cat is None else
+                         ComplementarityScorer(cat, self.E, metric=metric, k=self.depth, inv_scale=inv_scale, row_offset=off,
+                                               process_group=process_group)
+                         for cat, off in zip(catalogs, row_offsets)]
+        self._dae = _DaeChunks(model, self.chunk, self.io, dev)
+
+    def _inputs(self, outfits, missing, candidates):
+        """outfits fp32 [Q, io], missing bool [Q, S] and candidates int64 [Q, S, m] (1 <= m <= 128, or None) on the model's device;
+        contiguous copies."""
+        x = _outfit_rows(outfits, self.io, self.device)
+        Q, S = x.shape[0], self.S
+        if not isinstance(missing, torch.Tensor) or missing.dtype != torch.bool:
+            raise RuntimeError("codae: missing must be a bool tensor")
+        if tuple(missing.shape) != (Q, S):
+            raise RuntimeError("codae: missing must have shape [%d, %d], got %s" % (Q, S, tuple(missing.shape)))
+        if not missing.is_cuda or missing.device != self.device:
+            raise RuntimeError("codae: missing must be on the model's device %s" % self.device)
+        if candidates is not None:
+            if not isinstance(candidates, torch.Tensor) or candidates.dtype != torch.int64:
+                raise RuntimeError("codae: candidates must be an int64 tensor")
+            if (candidates.dim() != 3 or tuple(candidates.shape[:2]) != (Q, S)
+                    or not 1 <= candidates.shape[2] <= self.MAX_DEPTH):
+                raise RuntimeError("codae: candidates must have shape [%d, %d, m] with 1 <= m <= %d, got %s"
+                                   % (Q, S, self.MAX_DEPTH, tuple(candidates.shape)))
+            if not candidates.is_cuda or candidates.device != self.device:
+                raise RuntimeError("codae: candidates must be on the model's device %s" % self.device)
+            candidates = candidates.contiguous()
+        return x, missing.contiguous(), candidates
+
+    def _limits(self, missing, depth):
+        """(outfits missing each slot [S], max m_q, C = depth^max m_q): one host synchronisation; RuntimeError past a limit."""
+        Q = missing.shape[0]
+        stats = torch.cat([missing.sum(0), missing.sum(1).max().view(1)]).tolist()
+        counts, m_max = [int(v) for v in stats[:-1]], int(stats[-1])
+        for s, n in enumerate(counts):
+            if n and self.catalogs[s] is None:
+                raise RuntimeError("codae: slot %d is missing in %d outfits but has no catalog" % (s, n))
+        C = depth ** m_max
+        if C > _C.COMPLETE_MAX_COMBOS:
+            raise RuntimeError("codae: %d combinations per outfit (depth %d ^ %d missing slots) exceed %d" % (C, depth, m_max,
+                                                                                                        _C.COMPLETE_MAX_COMBOS))
+        if Q * C > 2 ** 31 - 1:
+            raise RuntimeError("codae: Q * combinations = %d exceeds 2**31 - 1" % (Q * C))
+        return counts, m_max, C
+
+    def _candidates(self, x, missing, counts):
+        Q, S, E = x.shape[0], self.S, self.E
+        y = predict_missing(self.model, x, missing, E)
+        cand = torch.full((Q, S, self.depth), -1, dtype=torch.int64, device=self.device)
+        for s in range(S):
+            if not counts[s]:
+                continue
+            rows = torch.nonzero(missing[:, s]).view(-1)          # the slot's one host synchronisation
+            query = y.index_select(0, rows)[:, s * E:(s + 1) * E]
+            sc = self._scorers[s]
+            _, idx = sc.topk_batched(query) if rows.numel() >= ComplementarityScorer.TC_MIN_Q else sc.topk(query)
+            cand[rows, s] = idx
+        return cand
+
+    def candidates(self, outfits, missing):
+        """Stage 1 alone: int64 [Q, S, depth] global row ids, for each missing slot the best `depth` rows of its catalog against
+        predict_missing's reading of the slot (ComplementarityScorer.topk, or topk_batched from TC_MIN_Q outfits up), best first;
+        -1 for given slots and where a catalog has fewer than `depth` rows.  A collective under a process group."""
+        x, miss, _ = self._inputs(outfits, missing, None)
+        counts, _, _ = self._limits(miss, self.depth)
+        return self._candidates(x, miss, counts)
+
+    def _pool(self, missing, cand, counts, depth):
+        """The candidate rows this process holds: (slot_base [Q, S] int64, pool [R, E] f32 un-scaled, pool_id [R] int64).  The
+        missing (outfit, slot) pairs are numbered slot-major; pair i owns pool rows [i depth, (i + 1) depth), one per candidate.
+        Rows outside this process's shards, and padding, are zeros with pool_id -1."""
+        Q, S, E, dev = missing.shape[0], self.S, self.E, self.device
+        nm = sum(counts)
+        t = torch.nonzero_static(missing.t().reshape(-1), size=nm).view(-1)      # s Q + q, slot-major
+        pair_q, pair_s = t % Q, torch.div(t, Q, rounding_mode="floor")
+        slot_base = torch.full((Q, S), -1, dtype=torch.int64, device=dev)
+        slot_base[pair_q, pair_s] = torch.arange(nm, dtype=torch.int64, device=dev) * depth
+        R = max(1, nm * depth)
+        pool = torch.zeros((R, E), dtype=torch.float32, device=dev)
+        pool_id = torch.full((R,), -1, dtype=torch.int64, device=dev)
+        ids = cand[pair_q, pair_s]                                               # [nm, depth]
+        off = 0
+        for s in range(S):
+            n = counts[s]
+            if n and self.catalogs[s].shape[0]:
+                cat, n_local = self.catalogs[s], self.catalogs[s].shape[0]
+                g = ids[off:off + n].reshape(-1)
+                r = g - self.row_offsets[s]
+                own = (g >= 0) & (r >= 0) & (r < n_local)
+                rows = cat[:, :E].index_select(0, r.clamp(0, n_local - 1)).to(torch.float32)   # bf16 -> fp32 is exact
+                pool[off * depth:(off + n) * depth] = torch.where(own.view(-1, 1), rows, 0.0)
+                pool_id[off * depth:(off + n) * depth] = torch.where(own, g, -1)
+            off += n
+        return slot_base, pool, pool_id
+
+    def _stage2(self, x, missing, slot_base, pool, pool_id, depth, m_max, C):
+        """Every valid combination of every outfit through the DAE; (err [Q, k] f32, ids [Q, k, S] int64), best first."""
+        Q, S, E, dev = x.shape[0], self.S, self.E, self.device
+        R = pool_id.numel()
+        # pool row of candidate 0 of each outfit's j-th missing slot (-1 past its m_q)
+        base_j = torch.full((Q, m_max + 1), -1, dtype=torch.int64, device=dev)
+        base_j.scatter_(1, torch.where(missing, torch.cumsum(missing, 1) - 1, m_max), slot_base)
+        cidx = torch.arange(C, dtype=torch.int64, device=dev)
+        valid = torch.ones((Q, C), dtype=torch.bool, device=dev)
+        for j in range(m_max):
+            digit = torch.div(cidx, depth ** j, rounding_mode="floor") % depth
+            row = base_j[:, j:j + 1] + digit
+            held = (row < R) & (pool_id[row.clamp(0, R - 1)] >= 0)
+            valid &= torch.where(base_j[:, j:j + 1] >= 0, held, digit == 0)
+        combo = torch.where(valid, cidx, -1)
+        pos = torch.nonzero(valid.view(-1)).view(-1)                  # stage 2's one host synchronisation
+        err = torch.full((Q * C,), float("nan"), dtype=torch.float32, device=dev)
+        eng, acts, stage, wflat = self._dae.prepare()      # on every rank, combinations or not: sync_weights may be a collective
+        for c0 in range(0, pos.numel(), self.chunk):
+            pc = pos[c0:c0 + self.chunk]
+            _C.complete_build(x, S, E, slot_base, pool, pool_id, depth, C, pc, self.inv_scale, acts[0] if stage is None else stage)
+            if stage is not None:
+                _C.split_x3(stage, acts[0])
+            self._dae.forward(eng, acts, wflat, pc.numel())
+            _C.complete_error(x, S, E, slot_base, pool, pool_id, depth, C, pc, self.inv_scale, acts[-1], err)
+        out_s = torch.empty((Q, self.k), dtype=torch.float32, device=dev)
+        out_c = torch.empty((Q, self.k), dtype=torch.int64, device=dev)
+        _C.swap_pairs_topk(err, combo, self.k, out_s, out_c)
+        return out_s, _decode_combinations(out_c, slot_base, pool_id, depth)
+
+    def complete_local(self, outfits, missing, candidates):
+        """Stage 2 for a process that holds every listed row.  outfits [Q, io] scaled fp32, missing bool [Q, S], candidates int64
+        [Q, S, m] global row ids (< 0: padding; entries of given slots are ignored); depth = m.  Returns (err [Q, k] f32, ids
+        [Q, k, S] int64), best first by (error, combination index); ids are -1 in given slots, unused entries (+inf, -1...).
+        Combinations taking a padding id or a row outside this process's shards are not scored; NaN errors never rank."""
+        x, miss, cand = self._inputs(outfits, missing, candidates)
+        if cand is None:
+            raise RuntimeError("codae: candidates must be an int64 tensor")
+        depth = cand.shape[2]
+        counts, m_max, C = self._limits(miss, depth)
+        return self._stage2(x, miss, *self._pool(miss, cand, counts, depth), depth, m_max, C)
+
+    def complete(self, outfits, missing, candidates=None):
+        """Fill every missing slot: (err [Q, k] f32, ids [Q, k, S] int64) as complete_local.  Without candidates stage 1 runs first
+        (depth from the constructor).  Under a process group every rank is given the same inputs: the candidate pool is assembled
+        from every rank's shards (_exchange_pool), rank r scores its shard_rows(Q, G, r) outfits and the slices are all-gathered."""
+        if candidates is None:
+            candidates = self.candidates(outfits, missing)
+        if not _is_distributed(self.pg):
+            return self.complete_local(outfits, missing, candidates)
+        import torch.distributed as dist
+        x, miss, cand = self._inputs(outfits, missing, candidates)
+        depth = cand.shape[2]
+        counts, m_max, C = self._limits(miss, depth)
+        slot_base, pool, pool_id = self._pool(miss, cand, counts, depth)
+        pool, pool_id = _exchange_pool(pool, pool_id, self.pg)
+        Q, S, dev = x.shape[0], self.S, self.device
+        G, r = dist.get_world_size(self.pg), dist.get_rank(self.pg)
+        lo, n = shard_rows(Q, G, r)
+        per = (Q + G - 1) // G
+        err = torch.full((per, self.k), float("inf"), dtype=torch.float32, device=dev)
+        ids = torch.full((per, self.k, S), -1, dtype=torch.int64, device=dev)
+        if n:
+            e, i = self._stage2(x[lo:lo + n], miss[lo:lo + n], slot_base[lo:lo + n], pool, pool_id, depth, m_max, C)
+            err[:n], ids[:n] = e, i
+        else:
+            self.model.sync_weights()      # a collective under a sharded data-parallel trainer: every rank takes part
+        out = []
+        for t in (err, ids):
+            g = torch.empty((G * per,) + tuple(t.shape[1:]), dtype=t.dtype, device=dev)
+            dist.all_gather_into_tensor(g, t, group=self.pg)
+            out.append(g[:Q])
+        return tuple(out)
+
+
+def _decode_combinations(combo, slot_base, pool_id, depth):
+    """combo [Q, k] (combination indices, -1 unused) -> global ids [Q, k, S]: slot s of combination c is pool row slot_base[q, s] +
+    (c / depth^j) % depth for the j-th missing slot s, -1 for given slots and unused entries."""
+    R = pool_id.numel()
+    miss = slot_base >= 0
+    pw = torch.pow(depth, (torch.cumsum(miss, 1) - 1).clamp(min=0))                        # [Q, S]
+    digit = torch.div(combo.clamp(min=0).unsqueeze(2), pw.unsqueeze(1), rounding_mode="floor") % depth
+    row = (slot_base.unsqueeze(1) + digit).clamp(0, R - 1)
+    return torch.where(miss.unsqueeze(1) & (combo >= 0).unsqueeze(2), pool_id[row], -1)

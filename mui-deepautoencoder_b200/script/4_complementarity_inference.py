@@ -19,6 +19,11 @@ global row ids stored there (int64).  Both filter inside the kernels, so k resul
 is hidden in turn and reconstructed; it prints each outfit's per-slot errors, their sum (lower: more compatible) and the slot of
 largest error (the odd item out).  No catalog is built.  --compat_negatives also scores one shuffled outfit per query -- slot s
 taken from a seeded permutation of all observations -- and adds the compatibility AUC of the real outfits against them.
+
+--mode complete fills the slots listed by --missing (e.g. 1,2) of the first --queries outfits together
+(codae.tool.OutfitCompleter): the best --complete_depth B rows per missing slot by --metric, then every combination of them
+scored by the reconstruction error of the completed outfit; it prints the best k completions as ids [Q][k][S] (-1 in given slots)
+with their errors [Q][k].  --exclude_own_item and --allowed_rows do not apply to this mode.
 """
 import argparse
 import json
@@ -32,8 +37,8 @@ from _common import init_distributed, synthetic_categories
 from codae.dataset import ConcatenatedEmbeddingDataset
 from codae.model import EmbeddingDenoisingAutoencoder
 from codae.tool import load_dataset_of_embeddings
-from codae.tool.inference import (CompatibilityScorer, ComplementarityScorer, SwapScorer, compatibility_auc, predict_slot,
-                                  shard_rows)
+from codae.tool.inference import (CompatibilityScorer, ComplementarityScorer, OutfitCompleter, SwapScorer, compatibility_auc,
+                                  predict_slot, shard_rows)
 
 
 def parse():
@@ -44,8 +49,11 @@ def parse():
     parser.add_argument('--slot', type=int, default=0)
     parser.add_argument('--k', type=int, default=10)
     parser.add_argument('--metric', type=str, default="sqerr", choices=["sqerr", "cosine"])
-    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank", "compat"])
+    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank", "compat", "complete"])
     parser.add_argument('--rerank_depth', type=int, default=50, help="rerank mode: stage-1 candidates per outfit (1..128)")
+    parser.add_argument('--missing', type=str, default="1", help="complete mode: comma-separated slots to fill")
+    parser.add_argument('--complete_depth', type=int, default=8,
+                        help="complete mode: candidates per missing slot (1..128, depth^#missing <= 4096)")
     parser.add_argument('--compute_dtype', '--dtype', dest="compute_dtype", type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
     parser.add_argument('--queries', type=int, default=4)
     parser.add_argument('--synthetic', type=int, default=0)
@@ -72,6 +80,8 @@ if __name__ == "__main__":
     args = parse()
     if args.mode == "rerank" and not 1 <= args.rerank_depth <= 128:
         raise SystemExit("--rerank_depth must lie in [1, 128]")
+    if args.mode == "complete" and (args.exclude_own_item or args.allowed_rows):
+        raise SystemExit("--exclude_own_item and --allowed_rows are not supported by --mode complete (completion takes no filters)")
     rank, world, device = init_distributed()
     with open(args.config, 'r') as stream:
         config = yaml.safe_load(stream)
@@ -108,6 +118,24 @@ if __name__ == "__main__":
             print(json.dumps(res))
         raise SystemExit(0)
     lo, n_local = shard_rows(dataset.nb_observation, world, rank)
+    if args.mode == "complete":
+        slots = sorted({int(v) for v in args.missing.split(",")})
+        S = len(cats)
+        if not slots or not all(0 <= s < S for s in slots):
+            raise SystemExit("--missing must list slots in [0, %d)" % S)
+        cat_dtype = torch.bfloat16 if args.catalog_dtype == "bf16" else torch.float32
+        catalogs = [dataset.data_per_category[s][lo:lo + n_local].to(device).to(cat_dtype).contiguous() if s in slots else None
+                    for s in range(S)]
+        comp = OutfitCompleter(model, catalogs, E, depth=args.complete_depth, k=args.k, metric=args.metric,
+                               inv_scale=1.0 / dataset.scale, row_offsets=[lo] * S)
+        outfits = dataset.data[:args.queries].float().to(device).contiguous()
+        missing = torch.zeros((outfits.shape[0], S), dtype=torch.bool, device=device)
+        missing[:, slots] = True
+        err, ids = comp.complete(outfits, missing)
+        if rank == 0:
+            print(json.dumps({"mode": "complete", "missing": slots, "depth": args.complete_depth, "metric": args.metric, "k": args.k,
+                              "ids": ids.cpu().tolist(), "errors": err.cpu().tolist()}))
+        raise SystemExit(0)
     shard = dataset.data_per_category[args.slot][lo:lo + n_local].to(device)
     if args.catalog_dtype == "bf16":
         shard = shard.to(torch.bfloat16)
