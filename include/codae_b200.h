@@ -479,6 +479,35 @@ int codae_complete_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit
                          const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, int C,
                          const int64_t* pos, int B, float inv_scale, const float* y, int64_t ld_y, float* err, void* stream);
 
+/* Outfit completion by BEAM search: the missing slots s_0 < s_1 < ... of outfit q filled one level at a time, the best W partial
+ * outfits kept after each.  A partial assignment of missing slots 0 .. j is a combination index c < depth^(j+1) in the convention of
+ * codae_complete_*: digit i = (c / depth^i) % depth.  Level j expands parent t < W of outfit q, beam_c[q, t] (< 0: empty), by
+ * candidate b < depth of slot s_j into child c' = beam_c[q, t] + b depth^j, at position p = (q W + t) depth + b of the [Q, W depth]
+ * child grid.  outfits, slot_base, pool and pool_id are codae_complete_build's.
+ *   beam_c    int64 [Q, W]          the parents of this level (level 0: beam_c[q, 0] = 0, the rest -1)
+ *   pos       int64 [B]             built row b holds child pos[b]
+ * Child p is valid when 0 <= p < Q W depth, 0 <= beam_c[q, t] < depth^level, level < m_q and every pool row it takes lies in
+ * [0, n_pool) with pool_id >= 0.  An invalid row is built as zeros and gets no error (pos, beam_c, slot_base and pool_id are device
+ * data).
+ *   codae_complete_beam_build  x'[b, :] = outfit q with missing slots s_0 .. s_level replaced by their pool rows * inv_scale
+ *                              (codae_complete_build's values) and the later missing slots -- hidden -- +0.0, f32|bf16 at pitch ld_x.
+ *   codae_complete_beam_error  err[p] = sum_d (y[b, d] - x'_d)^2 over the columns of the given slots and of s_0 .. s_level only (the
+ *                              partial error), codae_complete_error's loop with the hidden columns skipped: at level m_q - 1 nothing
+ *                              is hidden and it is codae_complete_error's value for c' bit for bit.  err [Q W depth] is set to NaN by
+ *                              the caller; children not built stay NaN.
+ * Selection is codae_swap_pairs_topk(err [Q, W depth], key, k = W) with key = c' for valid children and -1 otherwise; its indices are
+ * the next level's beam_c.
+ * 1 <= S <= 64, E >= 1, 1 <= depth <= 128, 1 <= W <= 128, Q W depth <= INT32_MAX, 0 <= level < S, depth^(level+1) <= 2^62,
+ * n_pool >= 1, pitches >= their row widths, buffers naturally aligned; CODAE_EINVAL otherwise. */
+int codae_complete_beam_build(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                              const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth,
+                              const int64_t* beam_c, int W, int level, const int64_t* pos, int B, float inv_scale, void* out_x,
+                              int x_dtype, int64_t ld_x, void* stream);
+int codae_complete_beam_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                              const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth,
+                              const int64_t* beam_c, int W, int level, const int64_t* pos, int B, float inv_scale, const float* y,
+                              int64_t ld_y, float* err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

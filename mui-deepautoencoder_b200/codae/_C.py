@@ -89,6 +89,10 @@ SIGNATURES = {
     "codae_outfit_loo_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _i64, _vp, _vp, _vp, _vp]),
     "codae_complete_build": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _i, _vp, _i, _f, _vp, _i, _i64, _vp]),
     "codae_complete_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _i, _vp, _i, _f, _vp, _i64, _vp, _vp]),
+    "codae_complete_beam_build": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _vp, _i, _i, _vp, _i, _f, _vp, _i,
+                                       _i64, _vp]),
+    "codae_complete_beam_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _vp, _i, _i, _vp, _i, _f, _vp, _i64,
+                                       _vp, _vp]),
 }
 
 DP_MAX_WORLD = 8
@@ -631,6 +635,26 @@ def complete_error(outfits, S, E, slot_base, pool, pool_id, depth, C, pos, inv_s
     check(lib().codae_complete_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool), pool.stride(0),
                                      pool.shape[0], p(pool_id), depth, C, p(pos), pos.numel(), inv_scale, p(y), y.stride(0), p(err),
                                      stream()), c)
+
+
+def complete_beam_build(outfits, S, E, slot_base, pool, pool_id, depth, beam_c, level, pos, inv_scale, out_x):
+    """Rows of out_x: the children pos [B] (int64 positions in the [Q, W depth] grid) of the parents beam_c [Q, W] int64 at `level`,
+    built as complete_build builds a combination, with the missing slots past the level +0.0."""
+    _dev_check(outfits, slot_base, pool, pool_id, beam_c, pos, out_x)
+    c = ctx(outfits.device)
+    check(lib().codae_complete_beam_build(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool),
+                                          pool.stride(0), pool.shape[0], p(pool_id), depth, p(beam_c), beam_c.shape[1], level, p(pos),
+                                          pos.numel(), inv_scale, p(out_x), dt(out_x), out_x.stride(0), stream()), c)
+
+
+def complete_beam_error(outfits, S, E, slot_base, pool, pool_id, depth, beam_c, level, pos, inv_scale, y, err):
+    """err [Q W depth] f32: err[pos[b]] = partial error of reconstruction row b of y for that child (given slots and missing slots up
+    to the level)."""
+    _dev_check(outfits, slot_base, pool, pool_id, beam_c, pos, y, err)
+    c = ctx(outfits.device)
+    check(lib().codae_complete_beam_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool),
+                                          pool.stride(0), pool.shape[0], p(pool_id), depth, p(beam_c), beam_c.shape[1], level, p(pos),
+                                          pos.numel(), inv_scale, p(y), y.stride(0), p(err), stream()), c)
 
 
 def linear_engine(device, dtype, M, N, K):

@@ -19,7 +19,9 @@ Each slot is hidden in turn and reconstructed; the per-slot errors, their sum an
 compatibility_auc scores real outfits against shuffled ones.
 
 OutfitCompleter fills every empty slot of a partial outfit together ("I have a top, complete the outfit"): candidates per missing
-slot from the slot readings, then every combination of them scored by the swap error of the completed outfit.
+slot from the slot readings, then every combination of them scored by the swap error of the completed outfit -- or, where there are
+too many combinations, a beam search that fills the missing slots one at a time and keeps the best `width` partial outfits after
+each (complete_beam).
 """
 import torch
 
@@ -488,9 +490,16 @@ class OutfitCompleter:
     missing m_q slots -- by the swap error of the completed outfit, || DAE(x') - x' ||^2 over all io columns, and keeps the best k.
     The combinations of all outfits go through the model's GEMM chain in chunks of `chunk` rows (codae_complete_build, the Linear
     layers, codae_complete_error) and are ranked by codae_swap_pairs_topk; with one missing slot this is SwapScorer.rerank's
-    arithmetic, bit for bit (include/codae_b200.h: outfit completion)."""
+    arithmetic, bit for bit (include/codae_b200.h: outfit completion).
+
+    complete_beam replaces stage 2's depth^m_q combinations by a beam search of m_q W depth rows per outfit: the missing slots are
+    filled one level at a time in ascending slot order, each level scores every child of the W kept partial outfits by its partial
+    error (the swap error over the given slots and the slots filled so far, the later missing slots hidden as +0.0) and keeps the best
+    W by (error, combination index) (include/codae_b200.h: beam completion).  When the beam holds every combination it is
+    complete's search, bit for bit at chunks of <= 128 rows."""
 
     MAX_DEPTH = 128
+    MAX_WIDTH = 128
 
     def __init__(self, model, catalogs, embedding_size, depth=8, k=10, metric="sqerr", inv_scale=1.0, row_offsets=None,
                  chunk=8192, process_group=None):
@@ -557,14 +566,21 @@ class OutfitCompleter:
             candidates = candidates.contiguous()
         return x, missing.contiguous(), candidates
 
-    def _limits(self, missing, depth):
-        """(outfits missing each slot [S], max m_q, C = depth^max m_q): one host synchronisation; RuntimeError past a limit."""
-        Q = missing.shape[0]
-        stats = torch.cat([missing.sum(0), missing.sum(1).max().view(1)]).tolist()
-        counts, m_max = [int(v) for v in stats[:-1]], int(stats[-1])
+    def _counts(self, missing):
+        """(outfits missing each slot [S], max m_q, outfits missing nothing): one host synchronisation; RuntimeError for a missing slot
+        without a catalog."""
+        m_q = missing.sum(1)
+        stats = torch.cat([missing.sum(0), m_q.max().view(1), (m_q == 0).sum().view(1)]).tolist()
+        counts, m_max, n_full = [int(v) for v in stats[:-2]], int(stats[-2]), int(stats[-1])
         for s, n in enumerate(counts):
             if n and self.catalogs[s] is None:
                 raise RuntimeError("codae: slot %d is missing in %d outfits but has no catalog" % (s, n))
+        return counts, m_max, n_full
+
+    def _limits(self, missing, depth):
+        """(outfits missing each slot [S], max m_q, C = depth^max m_q): one host synchronisation; RuntimeError past a limit."""
+        Q = missing.shape[0]
+        counts, m_max, _ = self._counts(missing)
         C = depth ** m_max
         if C > _C.COMPLETE_MAX_COMBOS:
             raise RuntimeError("codae: %d combinations per outfit (depth %d ^ %d missing slots) exceed %d" % (C, depth, m_max,
@@ -595,6 +611,12 @@ class OutfitCompleter:
         counts, _, _ = self._limits(miss, self.depth)
         return self._candidates(x, miss, counts)
 
+    def _beam_candidates(self, outfits, missing):
+        """Stage 1 for complete_beam: candidates() without the exhaustive cap on depth^m_q."""
+        x, miss, _ = self._inputs(outfits, missing, None)
+        counts, _, _ = self._counts(miss)
+        return self._candidates(x, miss, counts)
+
     def _pool(self, missing, cand, counts, depth):
         """The candidate rows this process holds: (slot_base [Q, S] int64, pool [R, E] f32 un-scaled, pool_id [R] int64).  The
         missing (outfit, slot) pairs are numbered slot-major; pair i owns pool rows [i depth, (i + 1) depth), one per candidate.
@@ -623,13 +645,31 @@ class OutfitCompleter:
             off += n
         return slot_base, pool, pool_id
 
+    def _through_dae(self, prep, pos, build, error):
+        """The rows pos (int64 positions) through the DAE in chunks of `chunk`: build(pc, dst) writes a chunk's rows into dst, the
+        fp32-parity engine splits them into its planes, the Linear layers run and error(pc, y) reads the reconstructions y.  prep is
+        _DaeChunks.prepare()'s result."""
+        eng, acts, stage, wflat = prep
+        for c0 in range(0, pos.numel(), self.chunk):
+            pc = pos[c0:c0 + self.chunk]
+            build(pc, acts[0] if stage is None else stage)
+            if stage is not None:
+                _C.split_x3(stage, acts[0])
+            self._dae.forward(eng, acts, wflat, pc.numel())
+            error(pc, acts[-1])
+
+    @staticmethod
+    def _missing_bases(missing, slot_base, m_max):
+        """[Q, m_max + 1] int64: pool row of candidate 0 of each outfit's j-th missing slot (-1 past its m_q)."""
+        base_j = torch.full((missing.shape[0], m_max + 1), -1, dtype=torch.int64, device=missing.device)
+        base_j.scatter_(1, torch.where(missing, torch.cumsum(missing, 1) - 1, m_max), slot_base)
+        return base_j
+
     def _stage2(self, x, missing, slot_base, pool, pool_id, depth, m_max, C):
         """Every valid combination of every outfit through the DAE; (err [Q, k] f32, ids [Q, k, S] int64), best first."""
         Q, S, E, dev = x.shape[0], self.S, self.E, self.device
         R = pool_id.numel()
-        # pool row of candidate 0 of each outfit's j-th missing slot (-1 past its m_q)
-        base_j = torch.full((Q, m_max + 1), -1, dtype=torch.int64, device=dev)
-        base_j.scatter_(1, torch.where(missing, torch.cumsum(missing, 1) - 1, m_max), slot_base)
+        base_j = self._missing_bases(missing, slot_base, m_max)
         cidx = torch.arange(C, dtype=torch.int64, device=dev)
         valid = torch.ones((Q, C), dtype=torch.bool, device=dev)
         for j in range(m_max):
@@ -640,14 +680,10 @@ class OutfitCompleter:
         combo = torch.where(valid, cidx, -1)
         pos = torch.nonzero(valid.view(-1)).view(-1)                  # stage 2's one host synchronisation
         err = torch.full((Q * C,), float("nan"), dtype=torch.float32, device=dev)
-        eng, acts, stage, wflat = self._dae.prepare()      # on every rank, combinations or not: sync_weights may be a collective
-        for c0 in range(0, pos.numel(), self.chunk):
-            pc = pos[c0:c0 + self.chunk]
-            _C.complete_build(x, S, E, slot_base, pool, pool_id, depth, C, pc, self.inv_scale, acts[0] if stage is None else stage)
-            if stage is not None:
-                _C.split_x3(stage, acts[0])
-            self._dae.forward(eng, acts, wflat, pc.numel())
-            _C.complete_error(x, S, E, slot_base, pool, pool_id, depth, C, pc, self.inv_scale, acts[-1], err)
+        prep = self._dae.prepare()      # on every rank, combinations or not: sync_weights may be a collective
+        self._through_dae(prep, pos,
+                          lambda pc, dst: _C.complete_build(x, S, E, slot_base, pool, pool_id, depth, C, pc, self.inv_scale, dst),
+                          lambda pc, y: _C.complete_error(x, S, E, slot_base, pool, pool_id, depth, C, pc, self.inv_scale, y, err))
         out_s = torch.empty((Q, self.k), dtype=torch.float32, device=dev)
         out_c = torch.empty((Q, self.k), dtype=torch.int64, device=dev)
         _C.swap_pairs_topk(err, combo, self.k, out_s, out_c)
@@ -673,21 +709,26 @@ class OutfitCompleter:
             candidates = self.candidates(outfits, missing)
         if not _is_distributed(self.pg):
             return self.complete_local(outfits, missing, candidates)
-        import torch.distributed as dist
         x, miss, cand = self._inputs(outfits, missing, candidates)
         depth = cand.shape[2]
         counts, m_max, C = self._limits(miss, depth)
         slot_base, pool, pool_id = self._pool(miss, cand, counts, depth)
         pool, pool_id = _exchange_pool(pool, pool_id, self.pg)
-        Q, S, dev = x.shape[0], self.S, self.device
+        return self._sharded(x.shape[0], lambda lo, n: self._stage2(x[lo:lo + n], miss[lo:lo + n], slot_base[lo:lo + n], pool,
+                                                                    pool_id, depth, m_max, C))
+
+    def _sharded(self, Q, run):
+        """Under a process group: run(lo, n) -> (err [n, k], ids [n, k, S]) on this rank's shard_rows(Q, G, r) slice of the outfits,
+        then the slices all-gathered (padded to ceil(Q / G) rows) into the full results."""
+        import torch.distributed as dist
+        S, dev = self.S, self.device
         G, r = dist.get_world_size(self.pg), dist.get_rank(self.pg)
         lo, n = shard_rows(Q, G, r)
         per = (Q + G - 1) // G
         err = torch.full((per, self.k), float("inf"), dtype=torch.float32, device=dev)
         ids = torch.full((per, self.k, S), -1, dtype=torch.int64, device=dev)
         if n:
-            e, i = self._stage2(x[lo:lo + n], miss[lo:lo + n], slot_base[lo:lo + n], pool, pool_id, depth, m_max, C)
-            err[:n], ids[:n] = e, i
+            err[:n], ids[:n] = run(lo, n)
         else:
             self.model.sync_weights()      # a collective under a sharded data-parallel trainer: every rank takes part
         out = []
@@ -696,6 +737,102 @@ class OutfitCompleter:
             dist.all_gather_into_tensor(g, t, group=self.pg)
             out.append(g[:Q])
         return tuple(out)
+
+    def _check_width(self, width):
+        if not 1 <= width <= self.MAX_WIDTH:
+            raise RuntimeError("codae: beam width %d outside [1, %d]" % (width, self.MAX_WIDTH))
+        if self.k > width:
+            raise RuntimeError("codae: k %d exceeds the beam width %d" % (self.k, width))
+
+    def _beam_limits(self, missing, depth, width):
+        """complete_beam's limits: (outfits missing each slot [S], max m_q, outfits missing nothing); one host synchronisation;
+        RuntimeError past a limit."""
+        self._check_width(width)
+        Q = missing.shape[0]
+        if Q * width * depth > 2 ** 31 - 1:
+            raise RuntimeError("codae: Q * width * depth = %d exceeds 2**31 - 1" % (Q * width * depth))
+        counts, m_max, n_full = self._counts(missing)
+        if depth ** m_max > 2 ** 62:
+            raise RuntimeError("codae: depth %d ^ %d missing slots exceeds 2**62 (the beam's combination keys are int64)"
+                               % (depth, m_max))
+        return counts, m_max, n_full
+
+    def _beam(self, x, missing, slot_base, pool, pool_id, depth, m_max, n_full, width):
+        """Beam search over the missing slots of every outfit; (err [Q, k] f32, ids [Q, k, S] int64), best first.  n_full bounds the
+        outfits missing nothing (their count, or more: extra positions are padding)."""
+        Q, S, E, W, k, dev = x.shape[0], self.S, self.E, width, self.k, self.device
+        R = pool_id.numel()
+        inv = self.inv_scale
+        m_q = missing.sum(1)
+        base_j = self._missing_bases(missing, slot_base, m_max)
+        prep = self._dae.prepare()      # on every rank, rows or not: sync_weights may be a collective
+        err_f = torch.full((Q, k), float("inf"), dtype=torch.float32, device=dev)
+        c_f = torch.full((Q, k), -1, dtype=torch.int64, device=dev)
+        if n_full:
+            # outfits missing nothing: complete's answer, the outfit as given scored once (a [Q, 1] combination grid)
+            pos = torch.nonzero_static(m_q == 0, size=min(n_full, Q), fill_value=-1).view(-1)
+            e0 = torch.full((Q,), float("nan"), dtype=torch.float32, device=dev)
+            self._through_dae(prep, pos, lambda pc, dst: _C.complete_build(x, S, E, slot_base, pool, pool_id, depth, 1, pc, inv, dst),
+                              lambda pc, y: _C.complete_error(x, S, E, slot_base, pool, pool_id, depth, 1, pc, inv, y, e0))
+            scored = e0 == e0                                       # NaN never ranks
+            err_f[:, 0] = torch.where(scored, e0, float("inf"))
+            c_f[:, 0] = torch.where(scored, 0, -1)
+        beam = torch.full((Q, W), -1, dtype=torch.int64, device=dev)
+        beam[:, 0] = 0
+        b = torch.arange(depth, dtype=torch.int64, device=dev)
+        for j in range(m_max):
+            # child (q, t, b) = parent beam[q, t] + b depth^j; valid while the parent is, j < m_q and candidate b's row is held
+            row = base_j[:, j:j + 1] + b
+            held = (base_j[:, j:j + 1] >= 0) & (row < R) & (pool_id[row.clamp(0, R - 1)] >= 0)           # [Q, depth]
+            valid = (beam >= 0).unsqueeze(2) & held.unsqueeze(1)                                         # [Q, W, depth]
+            key = torch.where(valid, beam.unsqueeze(2) + b * depth ** j, -1).view(Q, W * depth)
+            pos = torch.nonzero(valid.view(-1)).view(-1)            # the level's one host synchronisation
+            err = torch.full((Q * W * depth,), float("nan"), dtype=torch.float32, device=dev)
+            parents = beam
+            self._through_dae(prep, pos,
+                              lambda pc, dst: _C.complete_beam_build(x, S, E, slot_base, pool, pool_id, depth, parents, j, pc, inv,
+                                                                     dst),
+                              lambda pc, y: _C.complete_beam_error(x, S, E, slot_base, pool, pool_id, depth, parents, j, pc, inv, y,
+                                                                   err))
+            out_s = torch.empty((Q, W), dtype=torch.float32, device=dev)
+            beam = torch.empty((Q, W), dtype=torch.int64, device=dev)
+            _C.swap_pairs_topk(err, key, W, out_s, beam)
+            done = (m_q == j + 1).view(Q, 1)                        # the outfits whose last level this is
+            err_f = torch.where(done, out_s[:, :k], err_f)
+            c_f = torch.where(done, beam[:, :k], c_f)
+        return err_f, _decode_combinations(c_f, slot_base, pool_id, depth)
+
+    def complete_beam_local(self, outfits, missing, candidates, width):
+        """complete_local by beam search of width W = `width` (1 <= k <= W <= 128): the missing slots of each outfit are filled in
+        ascending slot order, and after each the best W partial outfits are kept by (partial error, combination index).  The partial
+        error is the swap error over the columns of the given slots and the slots filled so far; the later missing slots are hidden
+        (+0.0 in the DAE input, not in the error).  Returns (err [Q, k] f32, ids [Q, k, S] int64) as complete_local: the first k of
+        the last level's selection, whose errors are complete's errors of those combinations.  With W >= depth^(m_max - 1) nothing is
+        pruned and, at chunks of <= 128 rows, the result is complete_local's bit for bit.  Synchronises once for the limits and once
+        per level."""
+        x, miss, cand = self._inputs(outfits, missing, candidates)
+        if cand is None:
+            raise RuntimeError("codae: candidates must be an int64 tensor")
+        depth = cand.shape[2]
+        counts, m_max, n_full = self._beam_limits(miss, depth, width)
+        return self._beam(x, miss, *self._pool(miss, cand, counts, depth), depth, m_max, n_full, width)
+
+    def complete_beam(self, outfits, missing, width, candidates=None):
+        """complete_beam_local for any process: without candidates stage 1 runs first (depth from the constructor).  Under a process
+        group every rank is given the same inputs, the candidate pool is assembled from every rank's shards, rank r searches its
+        shard_rows(Q, G, r) outfits and the slices are all-gathered -- as complete does."""
+        self._check_width(width)
+        if candidates is None:
+            candidates = self._beam_candidates(outfits, missing)
+        if not _is_distributed(self.pg):
+            return self.complete_beam_local(outfits, missing, candidates, width)
+        x, miss, cand = self._inputs(outfits, missing, candidates)
+        depth = cand.shape[2]
+        counts, m_max, n_full = self._beam_limits(miss, depth, width)
+        slot_base, pool, pool_id = self._pool(miss, cand, counts, depth)
+        pool, pool_id = _exchange_pool(pool, pool_id, self.pg)
+        return self._sharded(x.shape[0], lambda lo, n: self._beam(x[lo:lo + n], miss[lo:lo + n], slot_base[lo:lo + n], pool, pool_id,
+                                                                  depth, m_max, n_full, width))
 
 
 def _decode_combinations(combo, slot_base, pool_id, depth):

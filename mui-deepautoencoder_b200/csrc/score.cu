@@ -846,6 +846,125 @@ __global__ void __launch_bounds__(kThreads) complete_error_kernel(const float* _
     }
 }
 
+// ---- beam completion: the missing slots filled one level at a time, the slots not yet filled hidden -------------------------
+constexpr int64_t kHiddenSlot = -2;
+// v /= d, returning v % d, for 0 <= v and 1 <= d <= 128 in 32-bit divisions (a 64-bit division is a call, which spills here):
+// the high word, then the low word in two 16-bit steps, each dividend below 2^23.
+__device__ __forceinline__ int divmod_small(int64_t& v, int d) {
+    const uint32_t ud = (uint32_t)d, hi = (uint32_t)((uint64_t)v >> 32), lo = (uint32_t)v;
+    const uint32_t a = ((hi % ud) << 16) | (lo >> 16), b = ((a % ud) << 16) | (lo & 0xffffu);
+    v = (int64_t)(((uint64_t)(hi / ud) << 32) | ((a / ud) << 16) | (b / ud));
+    return (int)(b % ud);
+}
+// Child p of the flattened [Q, W depth] grid at `level` (include/codae_b200.h: beam completion) -- the one decode and validity rule of
+// both beam kernels.  Child (q, t, b) extends parent beam_c[q, t] by candidate b of the level-th missing slot of outfit q.  Returns
+// whether it is valid and sets q and, in row, what slot `want` holds: its pool row, -1 for a given slot, kHiddenSlot for a missing
+// slot past the level.  The parent's digits (complete_row's convention) fill missing slots 0 .. level-1; the parent is < depth^level
+// exactly when nothing of it is left after them, and the level is < m_q exactly when more than `level` missing slots were seen.  Every
+// pool row the child takes is checked before any of it is read.
+__device__ __forceinline__ bool beam_row(const int64_t* __restrict__ pos, const int64_t* __restrict__ beam_c, int W,
+                                         const int64_t* __restrict__ slot_base, const int64_t* __restrict__ pool_id, int64_t n_pool,
+                                         int Q, int S, int depth, int level, int b, int want, int64_t& p, int64_t& q, int64_t& row) {
+    p = pos[b];
+    row = -1;
+    const int wd = W * depth;
+    if (p < 0 || p >= (int64_t)Q * wd) return false;
+    const int pc = (int)p;                             // Q W depth <= INT32_MAX: 32-bit divisions from here on
+    q = pc / wd;
+    const int t = (pc - (int)q * wd) / depth;
+    const int cand = pc - (int)q * wd - t * depth;
+    int64_t parent = beam_c[q * W + t];
+    if (parent < 0) return false;
+    const int64_t* sb = slot_base + q * S;
+    int j = 0;
+    for (int s = 0; s < S; ++s) {
+        const int64_t base = sb[s];
+        if (base < 0) continue;
+        const int jj = j++;
+        if (jj > level) {
+            if (s == want) row = kHiddenSlot;
+            continue;
+        }
+        int digit = cand;
+        if (jj < level) digit = divmod_small(parent, depth);
+        if (base >= n_pool || digit >= n_pool - base) return false;
+        if (pool_id[base + digit] < 0) return false;
+        if (s == want) row = base + digit;
+    }
+    return j > level && parent == 0;
+}
+
+//   beam_build_kernel   x'[b, :] = outfit q with missing slots 0 .. level filled (pool row * inv_scale, complete_build_kernel's
+//                       values) and the later missing slots +0.0; V = 4 as in complete_build_kernel.
+template <bool kBf16Out, int V>
+__global__ void __launch_bounds__(256) beam_build_kernel(const float* __restrict__ outfits, int64_t ld_outfit, int Q, int S, int E,
+                                                         const int64_t* __restrict__ slot_base, const float* __restrict__ pool,
+                                                         int64_t ld_pool, int64_t n_pool, const int64_t* __restrict__ pool_id,
+                                                         int depth, const int64_t* __restrict__ beam_c, int W, int level,
+                                                         const int64_t* __restrict__ pos, int B, float inv_scale,
+                                                         void* __restrict__ out, int64_t ld_out) {
+    const int per_row = S * E / V;
+    const int64_t total = (int64_t)B * per_row;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+        const int b = (int)(e / per_row), d0 = (int)(e - (int64_t)b * per_row) * V;
+        const int s = d0 / E;                        // V divides E: the V columns lie in one slot
+        int64_t p, q, r;
+        float v[V];
+        if (!beam_row(pos, beam_c, W, slot_base, pool_id, n_pool, Q, S, depth, level, b, s, p, q, r) || r == kHiddenSlot) {
+#pragma unroll
+            for (int j = 0; j < V; ++j) v[j] = 0.f;
+        } else if (r >= 0) {
+            const float* src = pool + r * ld_pool + (d0 - s * E);
+#pragma unroll
+            for (int j = 0; j < V; ++j) v[j] = src[j] * inv_scale;
+        } else if constexpr (V == 4) {
+            const float4 o = *reinterpret_cast<const float4*>(outfits + q * ld_outfit + d0);
+            v[0] = o.x; v[1] = o.y; v[2] = o.z; v[3] = o.w;
+        } else {
+            v[0] = outfits[q * ld_outfit + d0];
+        }
+#pragma unroll
+        for (int j = 0; j < V; ++j) {
+            if (kBf16Out) reinterpret_cast<__nv_bfloat16*>(out)[(int64_t)b * ld_out + d0 + j] = __float2bfloat16_rn(v[j]);
+            else reinterpret_cast<float*>(out)[(int64_t)b * ld_out + d0 + j] = v[j];
+        }
+    }
+}
+
+//   beam_error_kernel   err[p] = sum_d (y[b, d] - x'_d)^2 over the columns of the given slots and of missing slots 0 .. level: the loop
+//                       of complete_error_kernel with the hidden columns skipped, so at a child's last level it is complete_error's
+//                       value bit for bit.  The minimum of one CTA per SM in the launch bounds lets ptxas use the 40 registers the
+//                       decode needs; without it ptxas held the kernel to 32 and spilled.
+__global__ void __launch_bounds__(kThreads, 1) beam_error_kernel(const float* __restrict__ outfits, int64_t ld_outfit, int Q, int S, int E,
+                                                              const int64_t* __restrict__ slot_base, const float* __restrict__ pool,
+                                                              int64_t ld_pool, int64_t n_pool, const int64_t* __restrict__ pool_id,
+                                                              int depth, const int64_t* __restrict__ beam_c, int W, int level,
+                                                              const int64_t* __restrict__ pos, int B, float inv_scale,
+                                                              const float* __restrict__ y, int64_t ld_y, float* __restrict__ err) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int io = S * E;
+    for (int b = blockIdx.x * kWarps + warp; b < B; b += gridDim.x * kWarps) {
+        int64_t p, q, r;
+        if (!beam_row(pos, beam_c, W, slot_base, pool_id, n_pool, Q, S, depth, level, b, 0, p, q, r)) continue;
+        const float* x = outfits + q * ld_outfit;
+        float acc = 0.f;
+        int lo = 0;
+        for (int d = lane; d < io; d += 32) {
+            if (d >= lo + E) {
+                const int s = d / E;
+                lo = s * E;
+                beam_row(pos, beam_c, W, slot_base, pool_id, n_pool, Q, S, depth, level, b, s, p, q, r);
+            }
+            if (r == kHiddenSlot) continue;
+            const float t = r >= 0 ? pool[r * ld_pool + (d - lo)] * inv_scale : x[d];
+            const float df = y[(int64_t)b * ld_y + d] - t;
+            acc = fmaf(df, df, acc);
+        }
+        acc = warp_sum(acc);
+        if (lane == 0) err[p] = acc;
+    }
+}
+
 inline int sweep_grid(const codae_ctx* ctx, int64_t n_rows) {
     int64_t g = (n_rows + kWarps - 1) / kWarps;
     const int64_t cap = (int64_t)ctx->sm_count * 4;
@@ -1161,6 +1280,69 @@ int codae_complete_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit
                                                                                    n_pool, pool_id, depth, C, pos, B, inv_scale, y, ld_y,
                                                                                    err);
     return codae_check_launch(ctx, "complete_error_kernel");
+}
+
+// Arguments shared by codae_complete_beam_build and codae_complete_beam_error.
+static int check_beam(codae_ctx* ctx, const char* fn, const float* outfits, int64_t ld_outfit, int Q, int S, int E,
+                      const int64_t* slot_base, const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth,
+                      const int64_t* beam_c, int W, int level, const int64_t* pos, int B) {
+    CODAE_REQUIRE(ctx, ctx && outfits && slot_base && pool && pool_id && beam_c && pos, "%s: NULL argument", fn);
+    CODAE_REQUIRE(ctx, Q >= 1 && S >= 1 && S <= 64 && E >= 1 && (int64_t)S * E <= INT32_MAX && B >= 1,
+                  "%s: bad shape Q=%d S=%d E=%d B=%d (Q, B >= 1, 1 <= S <= 64)", fn, Q, S, E, B);
+    CODAE_REQUIRE(ctx, depth >= 1 && depth <= kMaxK && W >= 1 && W <= kMaxK && (int64_t)Q * W * depth <= INT32_MAX,
+                  "%s: bad beam depth=%d W=%d (1 <= depth, W <= %d, Q W depth <= INT32_MAX)", fn, depth, W, kMaxK);
+    bool fits = level >= 0 && level < S;                 // the keys of level `level` are < depth^(level+1) <= 2^62
+    for (int64_t pw = 1, i = 0; fits && i <= level; ++i) {
+        fits = pw <= ((int64_t)1 << 62) / depth;
+        pw *= depth;
+    }
+    CODAE_REQUIRE(ctx, fits, "%s: bad level %d (0 <= level < S, depth^(level+1) <= 2^62)", fn, level);
+    CODAE_REQUIRE(ctx, n_pool >= 1 && ld_pool >= E && ld_outfit >= (int64_t)S * E,
+                  "%s: bad pool or pitch (n_pool=%lld ld_pool=%lld ld_outfit=%lld)", fn, (long long)n_pool, (long long)ld_pool,
+                  (long long)ld_outfit);
+    const auto al = [](const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; };
+    CODAE_REQUIRE(ctx, al(outfits, 4) && al(pool, 4) && al(slot_base, 8) && al(pool_id, 8) && al(beam_c, 8) && al(pos, 8),
+                  "%s: misaligned buffer", fn);
+    return CODAE_OK;
+}
+
+int codae_complete_beam_build(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                              const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth,
+                              const int64_t* beam_c, int W, int level, const int64_t* pos, int B, float inv_scale, void* out_x,
+                              int x_dtype, int64_t ld_x, void* stream) {
+    int rc = check_beam(ctx, "codae_complete_beam_build", outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool, n_pool, pool_id,
+                        depth, beam_c, W, level, pos, B);
+    if (rc) return rc;
+    const int io = S * E;
+    const bool bo = x_dtype == CODAE_BF16;
+    CODAE_REQUIRE(ctx, out_x && ld_x >= io && (x_dtype == CODAE_F32 || bo) &&
+                           (reinterpret_cast<uintptr_t>(out_x) & (bo ? 1 : 3)) == 0,
+                  "codae_complete_beam_build: bad output (ld_x=%lld x_dtype=%d)", (long long)ld_x, x_dtype);
+    const bool v4 = E % 4 == 0 && ld_outfit % 4 == 0 && (reinterpret_cast<uintptr_t>(outfits) & 15) == 0;
+    const int V = v4 ? 4 : 1;
+    int64_t blocks = ((int64_t)B * (io / V) + 256 * 4 - 1) / (256 * 4);
+    if (blocks > (int64_t)ctx->sm_count * 8) blocks = (int64_t)ctx->sm_count * 8;
+    cudaStream_t s = as_stream(stream);
+#define LAUNCH(BO, VV) beam_build_kernel<BO, VV><<<(unsigned)blocks, 256, 0, s>>>(outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool, n_pool, pool_id, depth, beam_c, W, level, pos, B, inv_scale, out_x, ld_x)
+    if (bo) { if (v4) LAUNCH(true, 4); else LAUNCH(true, 1); } else { if (v4) LAUNCH(false, 4); else LAUNCH(false, 1); }
+#undef LAUNCH
+    return codae_check_launch(ctx, "beam_build_kernel");
+}
+
+int codae_complete_beam_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                              const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth,
+                              const int64_t* beam_c, int W, int level, const int64_t* pos, int B, float inv_scale, const float* y,
+                              int64_t ld_y, float* err, void* stream) {
+    int rc = check_beam(ctx, "codae_complete_beam_error", outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool, n_pool, pool_id,
+                        depth, beam_c, W, level, pos, B);
+    if (rc) return rc;
+    CODAE_REQUIRE(ctx, y && err && ld_y >= (int64_t)S * E && (reinterpret_cast<uintptr_t>(y) & 3) == 0 &&
+                           (reinterpret_cast<uintptr_t>(err) & 3) == 0,
+                  "codae_complete_beam_error: bad output (ld_y=%lld)", (long long)ld_y);
+    beam_error_kernel<<<sweep_grid(ctx, B), kThreads, 0, as_stream(stream)>>>(outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool,
+                                                                               n_pool, pool_id, depth, beam_c, W, level, pos, B,
+                                                                               inv_scale, y, ld_y, err);
+    return codae_check_launch(ctx, "beam_error_kernel");
 }
 
 int codae_score_rank(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,

@@ -23,7 +23,9 @@ taken from a seeded permutation of all observations -- and adds the compatibilit
 --mode complete fills the slots listed by --missing (e.g. 1,2) of the first --queries outfits together
 (codae.tool.OutfitCompleter): the best --complete_depth B rows per missing slot by --metric, then every combination of them
 scored by the reconstruction error of the completed outfit; it prints the best k completions as ids [Q][k][S] (-1 in given slots)
-with their errors [Q][k].  --exclude_own_item and --allowed_rows do not apply to this mode.
+with their errors [Q][k].  --exclude_own_item and --allowed_rows do not apply to this mode.  With --beam W the combinations
+are searched by a beam of width W instead (OutfitCompleter.complete_beam: the missing slots filled one at a time, the best W
+partial outfits kept after each), which has no cap on depth^#missing; the JSON then also holds "beam": W.
 """
 import argparse
 import json
@@ -53,7 +55,9 @@ def parse():
     parser.add_argument('--rerank_depth', type=int, default=50, help="rerank mode: stage-1 candidates per outfit (1..128)")
     parser.add_argument('--missing', type=str, default="1", help="complete mode: comma-separated slots to fill")
     parser.add_argument('--complete_depth', type=int, default=8,
-                        help="complete mode: candidates per missing slot (1..128, depth^#missing <= 4096)")
+                        help="complete mode: candidates per missing slot (1..128, depth^#missing <= 4096 without --beam)")
+    parser.add_argument('--beam', type=int, default=None,
+                        help="complete mode: search by a beam of this width (k <= W <= 128) instead of every combination")
     parser.add_argument('--compute_dtype', '--dtype', dest="compute_dtype", type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
     parser.add_argument('--queries', type=int, default=4)
     parser.add_argument('--synthetic', type=int, default=0)
@@ -131,10 +135,16 @@ if __name__ == "__main__":
         outfits = dataset.data[:args.queries].float().to(device).contiguous()
         missing = torch.zeros((outfits.shape[0], S), dtype=torch.bool, device=device)
         missing[:, slots] = True
-        err, ids = comp.complete(outfits, missing)
+        if args.beam is None:
+            err, ids = comp.complete(outfits, missing)
+        else:
+            err, ids = comp.complete_beam(outfits, missing, args.beam)
         if rank == 0:
-            print(json.dumps({"mode": "complete", "missing": slots, "depth": args.complete_depth, "metric": args.metric, "k": args.k,
-                              "ids": ids.cpu().tolist(), "errors": err.cpu().tolist()}))
+            res = {"mode": "complete", "missing": slots, "depth": args.complete_depth, "metric": args.metric, "k": args.k,
+                   "ids": ids.cpu().tolist(), "errors": err.cpu().tolist()}
+            if args.beam is not None:
+                res["beam"] = args.beam
+            print(json.dumps(res))
         raise SystemExit(0)
     shard = dataset.data_per_category[args.slot][lo:lo + n_local].to(device)
     if args.catalog_dtype == "bf16":
