@@ -508,6 +508,31 @@ int codae_complete_beam_error(codae_ctx* ctx, const float* outfits, int64_t ld_o
                               const int64_t* beam_c, int W, int level, const int64_t* pos, int B, float inv_scale, const float* y,
                               int64_t ld_y, float* err, void* stream);
 
+/* Outfit REVISION: the best single-item replacements of a complete outfit.  Outfit q has a grid of 1 + S depth rows: column 0 is the
+ * outfit as given (the base row), column 1 + s depth + c is the outfit with slot s replaced by its candidate c, pool row
+ * slot_base[q, s] + c.  outfits, pool and pool_id are codae_complete_build's.
+ *   slot_base int64 [Q, S]         pool row of candidate 0 of each revised slot, < 0 for a slot not revised
+ *   pos       int64 [B]            built row b holds row p = pos[b] of the flattened [Q, 1 + S depth] grid
+ * Row p is valid when 0 <= p < Q (1 + S depth) and, for a swap, slot_base[q, s] >= 0 and its pool row lies in [0, n_pool) with
+ * pool_id >= 0.  An invalid row is never dereferenced beyond slot_base: it is built as zeros and gets no error.
+ *   codae_revise_build  x'[b, :] = outfit q with slot s replaced by its pool row * inv_scale (codae_complete_build's values), the outfit
+ *                       as given for column 0; f32|bf16 at pitch ld_x (columns >= io untouched).
+ *   codae_revise_error  err[p] = sum_d (y[b, d] - x'_d)^2 over io, x' recomputed in fp32: codae_complete_error's loop (lane-strided
+ *                       fmaf, then the warp tree), so the base row's error is codae_complete_error's for the outfit with nothing
+ *                       missing, and a swap's is codae_complete_error's for that slot missing with the same candidate, bit for bit
+ *                       given the same y row.  A swap whose x' equals the outfit value for value in the swapped slot (the held item
+ *                       proposed again) gets no error.  err [Q (1 + S depth)] is set to NaN by the caller; rows not built stay NaN.
+ * Ranking is codae_swap_pairs_topk(err, key [Q, 1 + S depth], ...) with key = s depth + c for valid swaps and -1 otherwise (the base
+ * row included), then the list is cut where the error reaches the base row's.
+ * 1 <= S <= 64, E >= 1, 1 <= depth <= 128, Q (1 + S depth) <= INT32_MAX, n_pool >= 1, pitches >= their row widths, buffers naturally
+ * aligned; CODAE_EINVAL otherwise. */
+int codae_revise_build(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                       const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, const int64_t* pos, int B,
+                       float inv_scale, void* out_x, int x_dtype, int64_t ld_x, void* stream);
+int codae_revise_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                       const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, const int64_t* pos, int B,
+                       float inv_scale, const float* y, int64_t ld_y, float* err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

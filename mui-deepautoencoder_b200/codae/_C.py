@@ -93,6 +93,8 @@ SIGNATURES = {
                                        _i64, _vp]),
     "codae_complete_beam_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _vp, _i, _i, _vp, _i, _f, _vp, _i64,
                                        _vp, _vp]),
+    "codae_revise_build": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _vp, _i, _f, _vp, _i, _i64, _vp]),
+    "codae_revise_error": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _i64, _i64, _vp, _i, _vp, _i, _f, _vp, _i64, _vp, _vp]),
 }
 
 DP_MAX_WORLD = 8
@@ -655,6 +657,26 @@ def complete_beam_error(outfits, S, E, slot_base, pool, pool_id, depth, beam_c, 
     check(lib().codae_complete_beam_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool),
                                           pool.stride(0), pool.shape[0], p(pool_id), depth, p(beam_c), beam_c.shape[1], level, p(pos),
                                           pos.numel(), inv_scale, p(y), y.stride(0), p(err), stream()), c)
+
+
+def revise_build(outfits, S, E, slot_base, pool, pool_id, depth, pos, inv_scale, out_x):
+    """Rows of out_x: the rows pos [B] (int64 positions in the [Q, 1 + S depth] grid) of outfits [Q, S E] f32, the outfit as given for
+    column 0 and slot s replaced by its candidate c (pool row slot_base[q, s] + c) * inv_scale for column 1 + s depth + c."""
+    _dev_check(outfits, slot_base, pool, pool_id, pos, out_x)
+    c = ctx(outfits.device)
+    check(lib().codae_revise_build(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool), pool.stride(0),
+                                   pool.shape[0], p(pool_id), depth, p(pos), pos.numel(), inv_scale, p(out_x), dt(out_x), out_x.stride(0),
+                                   stream()), c)
+
+
+def revise_error(outfits, S, E, slot_base, pool, pool_id, depth, pos, inv_scale, y, err):
+    """err [Q (1 + S depth)] f32: err[pos[b]] = swap error of reconstruction row b of y for that grid row (none for a swap that
+    leaves the outfit as it is)."""
+    _dev_check(outfits, slot_base, pool, pool_id, pos, y, err)
+    c = ctx(outfits.device)
+    check(lib().codae_revise_error(c, p(outfits), outfits.stride(0), outfits.shape[0], S, E, p(slot_base), p(pool), pool.stride(0),
+                                   pool.shape[0], p(pool_id), depth, p(pos), pos.numel(), inv_scale, p(y), y.stride(0), p(err), stream()),
+          c)
 
 
 def linear_engine(device, dtype, M, N, K):

@@ -21,7 +21,8 @@ compatibility_auc scores real outfits against shuffled ones.
 OutfitCompleter fills every empty slot of a partial outfit together ("I have a top, complete the outfit"): candidates per missing
 slot from the slot readings, then every combination of them scored by the swap error of the completed outfit -- or, where there are
 too many combinations, a beam search that fills the missing slots one at a time and keeps the best `width` partial outfits after
-each (complete_beam).
+each (complete_beam).  For a complete outfit it answers "which one item should I replace, and with what?" (revise): candidates for
+every slot from its leave-one-slot-out reading, then every single-item replacement scored by swap error against the outfit as given.
 """
 import torch
 
@@ -405,6 +406,14 @@ class CompatibilityScorer:
         x = _outfit_rows(outfits, self.io, self.device)
         Q, S = x.shape[0], self.S
         err, score, odd = self._outputs(Q)
+        self._loo(x, lambda c0, Bq, y: _C.outfit_loo_error(x[c0:c0 + Bq], S, self.E, y, err[c0:c0 + Bq], score[c0:c0 + Bq],
+                                                           odd[c0:c0 + Bq]))
+        return err, score, odd
+
+    def _loo(self, x, on_chunk):
+        """The leave-one-slot-out forward of the outfit rows x [Q, io] in chunks of chunk_outfits whole outfits: on_chunk(c0, Bq, y)
+        receives each chunk's reconstructions y, slot-major (row s Bq + i is outfit c0 + i with slot s hidden)."""
+        Q, S = x.shape[0], self.S
         eng, acts, stage, wflat = self._dae.prepare()
         for c0 in range(0, Q, self.chunk_outfits):
             Bq = min(self.chunk_outfits, Q - c0)
@@ -415,8 +424,7 @@ class CompatibilityScorer:
             if stage is not None:
                 _C.split_x3(stage, acts[0])
             self._dae.forward(eng, acts, wflat, S * Bq)
-            _C.outfit_loo_error(rows, S, self.E, acts[-1], err[c0:c0 + Bq], score[c0:c0 + Bq], odd[c0:c0 + Bq])
-        return err, score, odd
+            on_chunk(c0, Bq, acts[-1])
 
     def score(self, outfits):
         """score_local over the ranks of the process group: every rank is given the same outfits, rank r scores its
@@ -496,7 +504,12 @@ class OutfitCompleter:
     filled one level at a time in ascending slot order, each level scores every child of the W kept partial outfits by its partial
     error (the swap error over the given slots and the slots filled so far, the later missing slots hidden as +0.0) and keeps the best
     W by (error, combination index) (include/codae_b200.h: beam completion).  When the beam holds every combination it is
-    complete's search, bit for bit at chunks of <= 128 rows."""
+    complete's search, bit for bit at chunks of <= 128 rows.
+
+    revise takes complete outfits and returns the single-item replacements that lower the swap error: stage 1 reads every slot with
+    only that slot hidden (CompatibilityScorer's pass) and takes `depth` candidates per slot; stage 2 scores the outfit as given and
+    every (slot, candidate) swap through the GEMM chain (codae_revise_build, the Linear layers, codae_revise_error) and keeps the
+    best k swaps below the outfit's own error (include/codae_b200.h: outfit revision)."""
 
     MAX_DEPTH = 128
     MAX_WIDTH = 128
@@ -542,18 +555,30 @@ class OutfitCompleter:
                                                process_group=process_group)
                          for cat, off in zip(catalogs, row_offsets)]
         self._dae = _DaeChunks(model, self.chunk, self.io, dev)
+        self._has_catalog = torch.tensor([cat is not None for cat in catalogs], dtype=torch.bool, device=dev)
+        self._compat = None         # revise's stage 1: a CompatibilityScorer, made on first use
 
     def _inputs(self, outfits, missing, candidates):
         """outfits fp32 [Q, io], missing bool [Q, S] and candidates int64 [Q, S, m] (1 <= m <= 128, or None) on the model's device;
         contiguous copies."""
         x = _outfit_rows(outfits, self.io, self.device)
-        Q, S = x.shape[0], self.S
-        if not isinstance(missing, torch.Tensor) or missing.dtype != torch.bool:
-            raise RuntimeError("codae: missing must be a bool tensor")
-        if tuple(missing.shape) != (Q, S):
-            raise RuntimeError("codae: missing must have shape [%d, %d], got %s" % (Q, S, tuple(missing.shape)))
-        if not missing.is_cuda or missing.device != self.device:
-            raise RuntimeError("codae: missing must be on the model's device %s" % self.device)
+        Q = x.shape[0]
+        return x, self._slot_mask(missing, Q, "missing"), self._candidate_lists(candidates, Q)
+
+    def _slot_mask(self, mask, Q, name):
+        """bool [Q, S] on the model's device; a contiguous copy."""
+        S = self.S
+        if not isinstance(mask, torch.Tensor) or mask.dtype != torch.bool:
+            raise RuntimeError("codae: %s must be a bool tensor" % name)
+        if tuple(mask.shape) != (Q, S):
+            raise RuntimeError("codae: %s must have shape [%d, %d], got %s" % (name, Q, S, tuple(mask.shape)))
+        if not mask.is_cuda or mask.device != self.device:
+            raise RuntimeError("codae: %s must be on the model's device %s" % (name, self.device))
+        return mask.contiguous()
+
+    def _candidate_lists(self, candidates, Q):
+        """int64 [Q, S, m] (1 <= m <= 128) on the model's device, or None; a contiguous copy."""
+        S = self.S
         if candidates is not None:
             if not isinstance(candidates, torch.Tensor) or candidates.dtype != torch.int64:
                 raise RuntimeError("codae: candidates must be an int64 tensor")
@@ -564,7 +589,7 @@ class OutfitCompleter:
             if not candidates.is_cuda or candidates.device != self.device:
                 raise RuntimeError("codae: candidates must be on the model's device %s" % self.device)
             candidates = candidates.contiguous()
-        return x, missing.contiguous(), candidates
+        return candidates
 
     def _counts(self, missing):
         """(outfits missing each slot [S], max m_q, outfits missing nothing): one host synchronisation; RuntimeError for a missing slot
@@ -717,22 +742,25 @@ class OutfitCompleter:
         return self._sharded(x.shape[0], lambda lo, n: self._stage2(x[lo:lo + n], miss[lo:lo + n], slot_base[lo:lo + n], pool,
                                                                     pool_id, depth, m_max, C))
 
-    def _sharded(self, Q, run):
-        """Under a process group: run(lo, n) -> (err [n, k], ids [n, k, S]) on this rank's shard_rows(Q, G, r) slice of the outfits,
-        then the slices all-gathered (padded to ceil(Q / G) rows) into the full results."""
+    def _sharded(self, Q, run, results=None):
+        """Under a process group: run(lo, n) on this rank's shard_rows(Q, G, r) slice of the outfits, then the slices all-gathered
+        (padded to ceil(Q / G) rows) into the full results.  results: (per-outfit shape, dtype, fill) of each tensor run returns,
+        by default complete's (err [n, k] f32, ids [n, k, S] int64)."""
         import torch.distributed as dist
-        S, dev = self.S, self.device
+        dev = self.device
+        if results is None:
+            results = (((self.k,), torch.float32, float("inf")), ((self.k, self.S), torch.int64, -1))
         G, r = dist.get_world_size(self.pg), dist.get_rank(self.pg)
         lo, n = shard_rows(Q, G, r)
         per = (Q + G - 1) // G
-        err = torch.full((per, self.k), float("inf"), dtype=torch.float32, device=dev)
-        ids = torch.full((per, self.k, S), -1, dtype=torch.int64, device=dev)
+        outs = [torch.full((per,) + shape, fill, dtype=dtype, device=dev) for shape, dtype, fill in results]
         if n:
-            err[:n], ids[:n] = run(lo, n)
+            for t, v in zip(outs, run(lo, n)):
+                t[:n] = v
         else:
             self.model.sync_weights()      # a collective under a sharded data-parallel trainer: every rank takes part
         out = []
-        for t in (err, ids):
+        for t in outs:
             g = torch.empty((G * per,) + tuple(t.shape[1:]), dtype=t.dtype, device=dev)
             dist.all_gather_into_tensor(g, t, group=self.pg)
             out.append(g[:Q])
@@ -833,6 +861,137 @@ class OutfitCompleter:
         pool, pool_id = _exchange_pool(pool, pool_id, self.pg)
         return self._sharded(x.shape[0], lambda lo, n: self._beam(x[lo:lo + n], miss[lo:lo + n], slot_base[lo:lo + n], pool, pool_id,
                                                                   depth, m_max, n_full, width))
+
+    def _revise_inputs(self, outfits, keep, exclude, candidates):
+        """revise's inputs: outfits fp32 [Q, io], keep bool [Q, S], exclude int64 [Q, S, n] (1 <= n <= 256) and candidates int64
+        [Q, S, m] (1 <= m <= 128), the last three optional, on the model's device; contiguous copies.  RuntimeError unless
+        Q (1 + S depth) <= 2**31 - 1, depth = m or, without candidates, the constructor's."""
+        x = _outfit_rows(outfits, self.io, self.device)
+        Q, S = x.shape[0], self.S
+        keep = None if keep is None else self._slot_mask(keep, Q, "keep")
+        if exclude is not None:
+            if not isinstance(exclude, torch.Tensor) or exclude.dtype != torch.int64:
+                raise RuntimeError("codae: exclude must be an int64 tensor")
+            if exclude.dim() != 3 or tuple(exclude.shape[:2]) != (Q, S) or not 1 <= exclude.shape[2] <= _C.TOPK_MAX_EXCLUDE:
+                raise RuntimeError("codae: exclude must have shape [%d, %d, n] with 1 <= n <= %d, got %s"
+                                   % (Q, S, _C.TOPK_MAX_EXCLUDE, tuple(exclude.shape)))
+            if not exclude.is_cuda or exclude.device != self.device:
+                raise RuntimeError("codae: exclude must be on the model's device %s" % self.device)
+            exclude = exclude.contiguous()
+        cand = self._candidate_lists(candidates, Q)
+        depth = self.depth if cand is None else cand.shape[2]
+        if Q * (1 + S * depth) > 2 ** 31 - 1:
+            raise RuntimeError("codae: Q * (1 + S * depth) = %d exceeds 2**31 - 1" % (Q * (1 + S * depth)))
+        return x, keep, exclude, cand
+
+    def _revise_candidates(self, x, keep, exclude):
+        """Stage 1 of revise: for every revisable (outfit, slot), the best `depth` rows of the slot's catalog against the reconstruction
+        of that slot with only that slot hidden (CompatibilityScorer's leave-one-slot-out forward); one nonzero per slot with a
+        catalog."""
+        Q, S, E, dev = x.shape[0], self.S, self.E, self.device
+        if self._compat is None:
+            self._compat = CompatibilityScorer(self.model, E, chunk=max(self.chunk, S))
+            if self.chunk >= S:
+                self._compat._dae = self._dae       # its chunks of whole outfits fit this completer's activation buffers
+        query = torch.empty((Q, S, E), dtype=torch.float32, device=dev)
+
+        def take(c0, Bq, y):                        # y[s Bq + i, s E:(s + 1) E]: outfit c0 + i's slot s, read with slot s hidden
+            query[c0:c0 + Bq] = torch.diagonal(y[:S * Bq, :self.io].reshape(S, Bq, S, E), dim1=0, dim2=2).permute(0, 2, 1)
+        self._compat._loo(x, take)
+        cand = torch.full((Q, S, self.depth), -1, dtype=torch.int64, device=dev)
+        for s in range(S):
+            if self.catalogs[s] is None:
+                continue
+            if keep is None:
+                rows = torch.arange(Q, dtype=torch.int64, device=dev)
+            else:
+                rows = torch.nonzero(~keep[:, s]).view(-1)            # the slot's one host synchronisation
+                if rows.numel() == 0:
+                    continue
+            ex = None if exclude is None else exclude[rows, s]
+            sc = self._scorers[s]
+            qs = query[rows, s]
+            _, idx = sc.topk_batched(qs, ex) if rows.numel() >= ComplementarityScorer.TC_MIN_Q else sc.topk(qs, ex)
+            cand[rows, s] = idx
+        return cand
+
+    def revise_candidates(self, outfits, keep=None, exclude=None):
+        """Stage 1 of revise alone: int64 [Q, S, depth] global row ids.  For every slot s of outfit q that keep[q, s] does not keep and
+        whose catalog is not None, the best `depth` rows of catalog s by `metric` against the DAE's reconstruction of slot s with only
+        slot s hidden -- predict_slot(model, outfits, s, E)'s reading, computed by CompatibilityScorer's leave-one-slot-out pass --
+        never returning the global ids exclude[q, s] (< 0: padding), best first (ComplementarityScorer.topk, or topk_batched from
+        TC_MIN_Q outfits up); -1 for kept slots and padding.  A collective under a process group."""
+        x, keep, exclude, _ = self._revise_inputs(outfits, keep, exclude, None)
+        return self._revise_candidates(x, keep, exclude)
+
+    def _revise_limits(self, cand):
+        """(revised bool [Q, S], revised outfits per slot [S]): slot s of outfit q is revised when it has a catalog and its list holds
+        an id >= 0.  One host synchronisation."""
+        revised = (cand >= 0).any(2) & self._has_catalog
+        return revised, [int(v) for v in revised.sum(0).tolist()]
+
+    def _revise(self, x, slot_base, pool, pool_id, depth):
+        """Stage 2: the grid [Q, 1 + S depth] of every outfit -- column 0 the outfit as given, column 1 + s depth + c slot s replaced by
+        its candidate c -- through the DAE; (base [Q] f32, err [Q, k] f32, slot [Q, k] int64, ids [Q, k] int64)."""
+        Q, S, k, dev = x.shape[0], self.S, self.k, self.device
+        R = pool_id.numel()
+        G = 1 + S * depth
+        row = slot_base.unsqueeze(2) + torch.arange(depth, dtype=torch.int64, device=dev)                    # [Q, S, depth]
+        held = (slot_base.unsqueeze(2) >= 0) & (row < R) & (pool_id[row.clamp(0, R - 1)] >= 0)
+        valid = torch.cat([torch.ones((Q, 1), dtype=torch.bool, device=dev), held.view(Q, S * depth)], 1)
+        # key s depth + c of column 1 + s depth + c; the base row and the rows not held never rank
+        key = torch.where(held.view(Q, S * depth), torch.arange(S * depth, dtype=torch.int64, device=dev), -1)
+        key = torch.cat([torch.full((Q, 1), -1, dtype=torch.int64, device=dev), key], 1)
+        pos = torch.nonzero(valid.view(-1)).view(-1)                  # stage 2's one host synchronisation
+        err = torch.full((Q * G,), float("nan"), dtype=torch.float32, device=dev)
+        prep = self._dae.prepare()      # on every rank, rows or not: sync_weights may be a collective
+        inv = self.inv_scale
+        self._through_dae(prep, pos, lambda pc, dst: _C.revise_build(x, S, self.E, slot_base, pool, pool_id, depth, pc, inv, dst),
+                          lambda pc, y: _C.revise_error(x, S, self.E, slot_base, pool, pool_id, depth, pc, inv, y, err))
+        out_s = torch.empty((Q, k), dtype=torch.float32, device=dev)
+        out_key = torch.empty((Q, k), dtype=torch.int64, device=dev)
+        _C.swap_pairs_topk(err, key, k, out_s, out_key)
+        base = err.view(Q, G)[:, 0].contiguous()
+        better = out_s < base.unsqueeze(1)          # every improving swap ranks first: the cut is exact; a NaN base keeps nothing
+        slot = torch.div(out_key, depth, rounding_mode="floor").clamp(min=0)
+        ids = pool_id[(slot_base.gather(1, slot) + out_key - slot * depth).clamp(0, R - 1)]
+        return (base, torch.where(better, out_s, float("inf")), torch.where(better, slot, -1), torch.where(better, ids, -1))
+
+    def revise_local(self, outfits, candidates):
+        """Stage 2 of revise for a process that holds every listed row.  outfits [Q, io] scaled fp32; candidates int64 [Q, S, m] global
+        row ids (< 0: padding), depth = m; a slot whose list holds no id >= 0, or whose catalog is None, is not revised.  Every
+        outfit is scored as given (base) and with each listed candidate of each revised slot swapped in, by the swap error
+        || DAE(x') - x' ||^2 over all io columns.  Returns (base [Q] f32, err [Q, k] f32, slot [Q, k] int64, ids [Q, k] int64): the
+        swaps of error strictly below base, best first by (error, s depth + c) -- ties to the lower slot, then to the earlier
+        candidate --, unused entries (+inf, -1, -1).  A swap that leaves the outfit as it is (the held item proposed again) never
+        lists; an outfit holding a NaN has a NaN base and no swaps.  Synchronises once for the limits and once for the grid."""
+        x, _, _, cand = self._revise_inputs(outfits, None, None, candidates)
+        if cand is None:
+            raise RuntimeError("codae: candidates must be an int64 tensor")
+        depth = cand.shape[2]
+        revised, counts = self._revise_limits(cand)
+        return self._revise(x, *self._pool(revised, cand, counts, depth), depth)
+
+    def revise(self, outfits, keep=None, exclude=None, candidates=None):
+        """Revise complete outfits: (base, err, slot, ids) as revise_local.  keep bool [Q, S]: slots that are not changed; without
+        candidates stage 1 (revise_candidates, with the exclusion lists exclude) runs first, depth from the constructor.  Under a
+        process group every rank is given the same inputs: the candidate pool is assembled from every rank's shards, rank r scores its
+        shard_rows(Q, G, r) outfits and the slices are all-gathered -- as complete does."""
+        x, keep, exclude, cand = self._revise_inputs(outfits, keep, exclude, candidates)
+        if cand is None:
+            cand = self._revise_candidates(x, keep, exclude)
+        elif keep is not None:
+            cand = torch.where(keep.unsqueeze(2), -1, cand)
+        if not _is_distributed(self.pg):
+            return self.revise_local(x, cand)
+        depth = cand.shape[2]
+        revised, counts = self._revise_limits(cand)
+        slot_base, pool, pool_id = self._pool(revised, cand, counts, depth)
+        pool, pool_id = _exchange_pool(pool, pool_id, self.pg)
+        k = self.k
+        return self._sharded(x.shape[0], lambda lo, n: self._revise(x[lo:lo + n], slot_base[lo:lo + n], pool, pool_id, depth),
+                             (((), torch.float32, float("nan")), ((k,), torch.float32, float("inf")), ((k,), torch.int64, -1),
+                              ((k,), torch.int64, -1)))
 
 
 def _decode_combinations(combo, slot_base, pool_id, depth):

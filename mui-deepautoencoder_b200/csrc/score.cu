@@ -965,6 +965,100 @@ __global__ void __launch_bounds__(kThreads, 1) beam_error_kernel(const float* __
     }
 }
 
+// ---- outfit revision: the outfit as given and every single-item replacement of it, each scored by swap error --------------
+// Row p of the flattened [Q, 1 + S depth] grid (include/codae_b200.h: outfit revision) -- the one decode and validity rule of both
+// revision kernels.  Column 0 of outfit q is the outfit as given (slot = -1); column 1 + s depth + c replaces slot s by its candidate
+// c, pool row slot_base[q, s] + c.  Returns whether p is valid and sets q, slot and row (-1 for column 0).  The pool row is checked
+// before it is read; Q (1 + S depth) <= INT32_MAX, so the decode uses 32-bit divisions.
+__device__ __forceinline__ bool revise_row(const int64_t* __restrict__ pos, const int64_t* __restrict__ slot_base,
+                                           const int64_t* __restrict__ pool_id, int64_t n_pool, int Q, int S, int depth, int b,
+                                           int64_t& p, int64_t& q, int& slot, int64_t& row) {
+    p = pos[b];
+    slot = -1;
+    row = -1;
+    const int g = 1 + S * depth;
+    if (p < 0 || p >= (int64_t)Q * g) return false;
+    const int pc = (int)p;
+    q = pc / g;
+    const int col = pc - (int)q * g;
+    if (col == 0) return true;
+    slot = (col - 1) / depth;
+    const int cand = col - 1 - slot * depth;
+    const int64_t base = slot_base[q * S + slot];
+    if (base < 0 || base >= n_pool || cand >= n_pool - base) return false;
+    row = base + cand;
+    return pool_id[row] >= 0;
+}
+
+//   revise_build_kernel   x'[b, :] = outfit q with slot `slot` replaced by its pool row * inv_scale (complete_build_kernel's values),
+//                         the outfit itself for column 0.  V = 4 as in complete_build_kernel.
+template <bool kBf16Out, int V>
+__global__ void __launch_bounds__(256) revise_build_kernel(const float* __restrict__ outfits, int64_t ld_outfit, int Q, int S, int E,
+                                                           const int64_t* __restrict__ slot_base, const float* __restrict__ pool,
+                                                           int64_t ld_pool, int64_t n_pool, const int64_t* __restrict__ pool_id,
+                                                           int depth, const int64_t* __restrict__ pos, int B, float inv_scale,
+                                                           void* __restrict__ out, int64_t ld_out) {
+    const int per_row = S * E / V;
+    const int64_t total = (int64_t)B * per_row;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+        const int b = (int)(e / per_row), d0 = (int)(e - (int64_t)b * per_row) * V;
+        const int s = d0 / E;                        // V divides E: the V columns lie in one slot
+        int64_t p, q, r;
+        int slot;
+        float v[V];
+        if (!revise_row(pos, slot_base, pool_id, n_pool, Q, S, depth, b, p, q, slot, r)) {
+#pragma unroll
+            for (int j = 0; j < V; ++j) v[j] = 0.f;
+        } else if (s == slot) {
+            const float* src = pool + r * ld_pool + (d0 - s * E);
+#pragma unroll
+            for (int j = 0; j < V; ++j) v[j] = src[j] * inv_scale;
+        } else if constexpr (V == 4) {
+            const float4 o = *reinterpret_cast<const float4*>(outfits + q * ld_outfit + d0);
+            v[0] = o.x; v[1] = o.y; v[2] = o.z; v[3] = o.w;
+        } else {
+            v[0] = outfits[q * ld_outfit + d0];
+        }
+#pragma unroll
+        for (int j = 0; j < V; ++j) {
+            if (kBf16Out) reinterpret_cast<__nv_bfloat16*>(out)[(int64_t)b * ld_out + d0 + j] = __float2bfloat16_rn(v[j]);
+            else reinterpret_cast<float*>(out)[(int64_t)b * ld_out + d0 + j] = v[j];
+        }
+    }
+}
+
+//   revise_error_kernel   err[p] = sum_d (y[b, d] - x'_d)^2 over io, one warp per row: complete_error_kernel's loop (lane-strided fmaf
+//                         over io, then the warp_sum tree), x'_d recomputed in fp32, the pool read only in the swapped slot.  A swap
+//                         whose x' equals the outfit value for value (the held item proposed again) gets no error: it is not a change.
+__global__ void __launch_bounds__(kThreads) revise_error_kernel(const float* __restrict__ outfits, int64_t ld_outfit, int Q, int S,
+                                                                int E, const int64_t* __restrict__ slot_base,
+                                                                const float* __restrict__ pool, int64_t ld_pool, int64_t n_pool,
+                                                                const int64_t* __restrict__ pool_id, int depth,
+                                                                const int64_t* __restrict__ pos, int B, float inv_scale,
+                                                                const float* __restrict__ y, int64_t ld_y, float* __restrict__ err) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int io = S * E;
+    for (int b = blockIdx.x * kWarps + warp; b < B; b += gridDim.x * kWarps) {
+        int64_t p, q, r;
+        int slot;
+        if (!revise_row(pos, slot_base, pool_id, n_pool, Q, S, depth, b, p, q, slot, r)) continue;
+        const float* x = outfits + q * ld_outfit;
+        const int lo = slot < 0 ? io : slot * E, hi = lo + E;
+        float acc = 0.f;
+        bool same = true;
+        for (int d = lane; d < io; d += 32) {
+            const bool in = d >= lo && d < hi;
+            const float t = in ? pool[r * ld_pool + (d - lo)] * inv_scale : x[d];
+            same &= !in || t == x[d];
+            const float df = y[(int64_t)b * ld_y + d] - t;
+            acc = fmaf(df, df, acc);
+        }
+        acc = warp_sum(acc);
+        if (slot >= 0 && __all_sync(0xffffffffu, same)) continue;
+        if (lane == 0) err[p] = acc;
+    }
+}
+
 inline int sweep_grid(const codae_ctx* ctx, int64_t n_rows) {
     int64_t g = (n_rows + kWarps - 1) / kWarps;
     const int64_t cap = (int64_t)ctx->sm_count * 4;
@@ -1343,6 +1437,59 @@ int codae_complete_beam_error(codae_ctx* ctx, const float* outfits, int64_t ld_o
                                                                                n_pool, pool_id, depth, beam_c, W, level, pos, B,
                                                                                inv_scale, y, ld_y, err);
     return codae_check_launch(ctx, "beam_error_kernel");
+}
+
+// Arguments shared by codae_revise_build and codae_revise_error.
+static int check_revise(codae_ctx* ctx, const char* fn, const float* outfits, int64_t ld_outfit, int Q, int S, int E,
+                        const int64_t* slot_base, const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth,
+                        const int64_t* pos, int B) {
+    CODAE_REQUIRE(ctx, ctx && outfits && slot_base && pool && pool_id && pos, "%s: NULL argument", fn);
+    CODAE_REQUIRE(ctx, Q >= 1 && S >= 1 && S <= 64 && E >= 1 && (int64_t)S * E <= INT32_MAX && B >= 1,
+                  "%s: bad shape Q=%d S=%d E=%d B=%d (Q, B >= 1, 1 <= S <= 64)", fn, Q, S, E, B);
+    CODAE_REQUIRE(ctx, depth >= 1 && depth <= kMaxK && (int64_t)Q * (1 + (int64_t)S * depth) <= INT32_MAX,
+                  "%s: bad grid depth=%d (1 <= depth <= %d, Q (1 + S depth) <= INT32_MAX)", fn, depth, kMaxK);
+    CODAE_REQUIRE(ctx, n_pool >= 1 && ld_pool >= E && ld_outfit >= (int64_t)S * E,
+                  "%s: bad pool or pitch (n_pool=%lld ld_pool=%lld ld_outfit=%lld)", fn, (long long)n_pool, (long long)ld_pool,
+                  (long long)ld_outfit);
+    const auto al = [](const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; };
+    CODAE_REQUIRE(ctx, al(outfits, 4) && al(pool, 4) && al(slot_base, 8) && al(pool_id, 8) && al(pos, 8), "%s: misaligned buffer", fn);
+    return CODAE_OK;
+}
+
+int codae_revise_build(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                       const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, const int64_t* pos, int B,
+                       float inv_scale, void* out_x, int x_dtype, int64_t ld_x, void* stream) {
+    int rc = check_revise(ctx, "codae_revise_build", outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool, n_pool, pool_id, depth,
+                          pos, B);
+    if (rc) return rc;
+    const int io = S * E;
+    const bool bo = x_dtype == CODAE_BF16;
+    CODAE_REQUIRE(ctx, out_x && ld_x >= io && (x_dtype == CODAE_F32 || bo) &&
+                           (reinterpret_cast<uintptr_t>(out_x) & (bo ? 1 : 3)) == 0,
+                  "codae_revise_build: bad output (ld_x=%lld x_dtype=%d)", (long long)ld_x, x_dtype);
+    const bool v4 = E % 4 == 0 && ld_outfit % 4 == 0 && (reinterpret_cast<uintptr_t>(outfits) & 15) == 0;
+    const int V = v4 ? 4 : 1;
+    int64_t blocks = ((int64_t)B * (io / V) + 256 * 4 - 1) / (256 * 4);
+    if (blocks > (int64_t)ctx->sm_count * 8) blocks = (int64_t)ctx->sm_count * 8;
+    cudaStream_t s = as_stream(stream);
+#define LAUNCH(BO, VV) revise_build_kernel<BO, VV><<<(unsigned)blocks, 256, 0, s>>>(outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool, n_pool, pool_id, depth, pos, B, inv_scale, out_x, ld_x)
+    if (bo) { if (v4) LAUNCH(true, 4); else LAUNCH(true, 1); } else { if (v4) LAUNCH(false, 4); else LAUNCH(false, 1); }
+#undef LAUNCH
+    return codae_check_launch(ctx, "revise_build_kernel");
+}
+
+int codae_revise_error(codae_ctx* ctx, const float* outfits, int64_t ld_outfit, int Q, int S, int E, const int64_t* slot_base,
+                       const float* pool, int64_t ld_pool, int64_t n_pool, const int64_t* pool_id, int depth, const int64_t* pos, int B,
+                       float inv_scale, const float* y, int64_t ld_y, float* err, void* stream) {
+    int rc = check_revise(ctx, "codae_revise_error", outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool, n_pool, pool_id, depth,
+                          pos, B);
+    if (rc) return rc;
+    CODAE_REQUIRE(ctx, y && err && ld_y >= (int64_t)S * E && (reinterpret_cast<uintptr_t>(y) & 3) == 0 &&
+                           (reinterpret_cast<uintptr_t>(err) & 3) == 0,
+                  "codae_revise_error: bad output (ld_y=%lld)", (long long)ld_y);
+    revise_error_kernel<<<sweep_grid(ctx, B), kThreads, 0, as_stream(stream)>>>(outfits, ld_outfit, Q, S, E, slot_base, pool, ld_pool,
+                                                                                 n_pool, pool_id, depth, pos, B, inv_scale, y, ld_y, err);
+    return codae_check_launch(ctx, "revise_error_kernel");
 }
 
 int codae_score_rank(codae_ctx* ctx, const void* catalog, int cat_dtype, int64_t n_rows, int64_t ld, int E,

@@ -26,6 +26,13 @@ scored by the reconstruction error of the completed outfit; it prints the best k
 with their errors [Q][k].  --exclude_own_item and --allowed_rows do not apply to this mode.  With --beam W the combinations
 are searched by a beam of width W instead (OutfitCompleter.complete_beam: the missing slots filled one at a time, the best W
 partial outfits kept after each), which has no cap on depth^#missing; the JSON then also holds "beam": W.
+
+--mode revise asks of each of the first --queries outfits, complete as they are, which one item to replace and with what
+(codae.tool.OutfitCompleter.revise): every slot is read with only that slot hidden, its best --complete_depth B catalog rows by
+--metric are swapped in one at a time, and the swaps whose reconstruction error is below the outfit's own are ranked.  It prints
+the outfit's error as "base" [Q] and the best k swaps as "errors", "slots" and "ids" [Q][k] (+inf / -1 where fewer swaps improve).
+--exclude_own_item keeps each outfit's own items out of its candidates (outfit q holds row q of every slot's catalog);
+--allowed_rows does not apply to this mode.
 """
 import argparse
 import json
@@ -51,11 +58,13 @@ def parse():
     parser.add_argument('--slot', type=int, default=0)
     parser.add_argument('--k', type=int, default=10)
     parser.add_argument('--metric', type=str, default="sqerr", choices=["sqerr", "cosine"])
-    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank", "compat", "complete"])
+    parser.add_argument('--mode', type=str, default="slot", choices=["slot", "swap", "rerank", "compat", "complete",
+                                                                                "revise"])
     parser.add_argument('--rerank_depth', type=int, default=50, help="rerank mode: stage-1 candidates per outfit (1..128)")
     parser.add_argument('--missing', type=str, default="1", help="complete mode: comma-separated slots to fill")
     parser.add_argument('--complete_depth', type=int, default=8,
-                        help="complete mode: candidates per missing slot (1..128, depth^#missing <= 4096 without --beam)")
+                        help="complete mode: candidates per missing slot (1..128, depth^#missing <= 4096 without --beam); "
+                             "revise mode: candidates per slot (1..128)")
     parser.add_argument('--beam', type=int, default=None,
                         help="complete mode: search by a beam of this width (k <= W <= 128) instead of every combination")
     parser.add_argument('--compute_dtype', '--dtype', dest="compute_dtype", type=str, default="fp32", choices=["fp32", "bf16", "fp32_simt"])
@@ -86,6 +95,8 @@ if __name__ == "__main__":
         raise SystemExit("--rerank_depth must lie in [1, 128]")
     if args.mode == "complete" and (args.exclude_own_item or args.allowed_rows):
         raise SystemExit("--exclude_own_item and --allowed_rows are not supported by --mode complete (completion takes no filters)")
+    if args.mode == "revise" and args.allowed_rows:
+        raise SystemExit("--allowed_rows is not supported by --mode revise (revision takes no allowed-row mask)")
     rank, world, device = init_distributed()
     with open(args.config, 'r') as stream:
         config = yaml.safe_load(stream)
@@ -145,6 +156,22 @@ if __name__ == "__main__":
             if args.beam is not None:
                 res["beam"] = args.beam
             print(json.dumps(res))
+        raise SystemExit(0)
+    if args.mode == "revise":
+        S = len(cats)
+        cat_dtype = torch.bfloat16 if args.catalog_dtype == "bf16" else torch.float32
+        catalogs = [dataset.data_per_category[s][lo:lo + n_local].to(device).to(cat_dtype).contiguous() for s in range(S)]
+        comp = OutfitCompleter(model, catalogs, E, depth=args.complete_depth, k=args.k, metric=args.metric,
+                               inv_scale=1.0 / dataset.scale, row_offsets=[lo] * S)
+        outfits = dataset.data[:args.queries].float().to(device).contiguous()
+        Q = outfits.shape[0]
+        exclude = (torch.arange(Q, dtype=torch.int64, device=device).view(Q, 1, 1).expand(Q, S, 1)
+                   if args.exclude_own_item else None)
+        base, err, slot, ids = comp.revise(outfits, exclude=exclude)
+        if rank == 0:
+            print(json.dumps({"mode": "revise", "depth": args.complete_depth, "metric": args.metric, "k": args.k,
+                              "base": base.cpu().tolist(), "errors": err.cpu().tolist(), "slots": slot.cpu().tolist(),
+                              "ids": ids.cpu().tolist()}))
         raise SystemExit(0)
     shard = dataset.data_per_category[args.slot][lo:lo + n_local].to(device)
     if args.catalog_dtype == "bf16":
